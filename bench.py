@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the GenPC geometric hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload = "C2"): batched Chamfer fwd+bwd, B=32 per GPU, 2048 x 16384 points (PCN shape,
@@ -299,7 +299,7 @@ def run_gpu_arm(args, loss_fn, rank, world, dev, part, comp, tag, host_loss_fn=N
         b.grad = None
         loss = loss_fn(a, b)
         loss.backward()
-        return loss
+        return loss, a.grad, b.grad
 
     def step_e2e():
         da = ha.to(dev, non_blocking=True).requires_grad_(True)
@@ -321,7 +321,9 @@ def run_gpu_arm(args, loss_fn, rank, world, dev, part, comp, tag, host_loss_fn=N
             dist.barrier()
         torch.cuda.synchronize(dev)
 
-    def timed(step, K, W):
+    last = {}   # --dump-outputs: host copies of what the last timed step of each device-resident path returned
+
+    def timed(step, K, W, name=None):
         for _ in range(W):
             flush.zero_()
             step()
@@ -330,9 +332,13 @@ def run_gpu_arm(args, loss_fn, rank, world, dev, part, comp, tag, host_loss_fn=N
         for i in range(K):
             flush.zero_()  # L2 flush between timed iterations, outside the event bracket
             ev[i][0].record()
-            step()
+            out = step()
             ev[i][1].record()
+            if i < K - 1:
+                del out    # outputs kept alive into the next step would make the allocator hand that step other blocks (slower)
         barrier()
+        if name is not None and args.dump_outputs:
+            last[name] = [t.detach().float().cpu().numpy() for t in out]
         ms = sum(e0.elapsed_time(e1) for e0, e1 in ev)
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
@@ -341,12 +347,12 @@ def run_gpu_arm(args, loss_fn, rank, world, dev, part, comp, tag, host_loss_fn=N
 
     sampler = ClockSampler(dev.index)
     sampler.start()
-    ms_eager = timed(step_resident, args.steps, args.warmup)
+    ms_eager = timed(step_resident, args.steps, args.warmup, "eager")
     ms_res = ms_eager
     if graphed_factory is not None:
         # the same step (same kernels, same device-resident inputs) captured once into a CUDA graph: one graph launch per step
         gstep = graphed_factory(a.detach(), b.detach())
-        ms_res = timed(lambda: gstep(), args.steps, args.warmup)
+        ms_res = timed(lambda: gstep(), args.steps, args.warmup, "graphed")
     clocks = sampler.stop()
     ms_plain = timed(step_e2e, args.steps, args.warmup)
     ms_e2e = timed(step_e2e_hostfed, args.steps, args.warmup) if host_loss_fn is not None else ms_plain
@@ -375,7 +381,29 @@ def run_gpu_arm(args, loss_fn, rank, world, dev, part, comp, tag, host_loss_fn=N
         res["e2e_plain"] = {"value": pairs_per_step * args.steps / (ms_plain * 1e-3), "unit": "pairs/s",
                             "ms_per_step": ms_plain / args.steps,
                             "api": "gen.to(device); gt.to(device); get_loss; backward; loss -> host (copy, then compute)"}
+    if args.dump_outputs and rank == 0:
+        path = "eager" if graphed_factory is None or ms_eager < ms_res else "graphed"   # the path `value` reports
+        res["dumped_outputs"] = {"path": path, "files": dump_outputs(args.dump_outputs, *last[path])}
     return res, (a, b, flush)
+
+
+def dump_outputs(out_dir, loss, grad_gen, grad_gt):
+    """--dump-outputs: what the timed step hands its caller -- the loss and the gradients of both clouds -- as float32 .npy
+    files under out_dir (7.1 MB at C2's shape)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "grad_gen": grad_gen, "grad_gt": grad_gt}
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x)
+    return [name + ".npy" for name in arrays]
+
+
+def no_dump(args, line):
+    """--impl reference timed on the CPU port: no GPU step ran, so --dump-outputs writes nothing, and says so in the line and
+    on stderr (an empty DIR must not pass for a dump)."""
+    if args.dump_outputs:
+        line["dumped_outputs"] = None
+        sys.stderr.write("bench.py: --dump-outputs: nothing written (the CPU port was timed, not a GPU step)\n")
+    return line
 
 
 def time_kernels_ours(dev, a, b, flush, iters=20):
@@ -727,7 +755,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C1 / C4 / C5 legs (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (loss, grad_gen, grad_gt; rank 0's) "
+                         "as DIR/<name>.npy in float32; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank, local, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
 
@@ -736,10 +769,11 @@ def main():
             # no GPU: the reference's CUDA extension cannot run; time the CPU port instead
             part, comp = make_inputs(0)
             cb = cpu_baseline(part, comp, budget_b=4)
-            print(json.dumps({"impl": "reference", "metric": "chamfer_fwd_bwd_point_pairs_per_sec",
-                              "value": cb["value"], "unit": "pairs/s", "n_gpus": 0, "cpu_baseline": cb,
-                              "e2e": {"value": cb["value"], "unit": "pairs/s", "h2d_bytes_per_step": 0,
-                                      "d2h_bytes_per_step": 0}}))
+            out = {"impl": "reference", "metric": "chamfer_fwd_bwd_point_pairs_per_sec",
+                   "value": cb["value"], "unit": "pairs/s", "n_gpus": 0, "cpu_baseline": cb,
+                   "e2e": {"value": cb["value"], "unit": "pairs/s", "h2d_bytes_per_step": 0,
+                           "d2h_bytes_per_step": 0}}
+            print(json.dumps(no_dump(args, out)))
             return
         raise SystemExit("bench.py: no CUDA device (genpc_b200 has no CPU fallback)")
 
@@ -772,7 +806,7 @@ def main():
                              "e2e": {"value": cb["value"], "unit": "pairs/s", "h2d_bytes_per_step": 0,
                                      "d2h_bytes_per_step": 0},
                              "note": "oracle/_ref not built: timed the CPU port"})
-                print(json.dumps(line))
+                print(json.dumps(no_dump(args, line)))
             return
         api = import_reference_api()
         if api is not None:

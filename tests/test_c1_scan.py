@@ -1,8 +1,8 @@
 """BASELINE config C1 on the REAL scan: the reference's data/01184.ply (71 372 points) against the 16 384-point synthetic
 shape, batch 1.  The scan's float32 coordinates are committed (tests/golden/scan_01184_xyz.npz, made by
 tests/golden/make_c1_fixture.py with an independent PLY parser); the reference extension's answer on a B200 is
-tests/golden/c1_ref_chamfer.npz.  CPU: the product's PLY reader against the fixture (and against the original file when
-/root/reference is present), the oracle against the golden.  GPU: the kernels against both."""
+tests/golden/c1_ref_chamfer.npz.  CPU: the product's PLY reader against the fixture (also written back in the original
+file's layout), the oracle against the golden.  GPU: the kernels against both."""
 import hashlib
 import os
 
@@ -14,7 +14,6 @@ import oracle
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIX = os.path.join(HERE, "golden", "scan_01184_xyz.npz")
 GOLD = os.path.join(HERE, "golden", "c1_ref_chamfer.npz")
-ORIG = "/root/reference/data/01184.ply"
 
 
 def digest(*arrays):
@@ -38,15 +37,21 @@ def test_fixture_is_intact():
     assert np.allclose(lo, [-0.19, -0.39, -0.38], atol=0.01) and np.allclose(hi, [0.20, 0.30, 0.14], atol=0.01)
 
 
-@pytest.mark.skipif(not os.path.exists(ORIG), reason="/root/reference is not present on this box")
-def test_ply_reader_on_the_reference_scan():
+def test_ply_reader_on_the_reference_scan(tmp_path):
+    """The reference's data/01184.ply holds the scan as binary little-endian doubles x, y, z.  That file is not part of this
+    repository: the committed coordinates are written back in its layout, with a header written here (not by write_ply_xyz)."""
     from genpc_b200.utils.dataUtils import load_xyz, read_ply_xyz
 
     want = np.load(FIX)["xyz"]
-    pts, col = read_ply_xyz(ORIG)
+    orig = str(tmp_path / "01184.ply")
+    with open(orig, "wb") as f:
+        f.write(f"ply\nformat binary_little_endian 1.0\nelement vertex {len(want)}\nproperty double x\nproperty double y\n"
+                "property double z\nend_header\n".encode("ascii"))
+        f.write(want.astype("<f8").tobytes())
+    pts, col = read_ply_xyz(orig)
     assert pts.dtype == np.float32 and np.array_equal(pts, want)
     assert col is None                                   # the fixture scans carry no colour
-    pts2, col2 = load_xyz(ORIG)                          # utils/dataUtils.py:174-189: colour = min-max normalised xyz
+    pts2, col2 = load_xyz(orig)                          # utils/dataUtils.py:174-189: colour = min-max normalised xyz
     assert np.array_equal(pts2, want) and col2.shape == want.shape
     ref_col = np.clip((want - want.min(0)) / (want.max(0) - want.min(0) + 1e-8), 0, 1)
     assert np.allclose(col2, ref_col, atol=1e-6)
