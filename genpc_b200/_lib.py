@@ -33,11 +33,9 @@ _SIGNATURES = {
     "genpc_get_tunable": (ctypes.c_char_p, [ctypes.c_char_p]),
     "genpc_chamfer_workspace_bytes": (_sz, [_int, _int, _int]),
     "genpc_chamfer_forward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _vp, _sz, _vp]),
-    "genpc_chamfer_tc_stats": (_int, [_vp]),
     "genpc_chamfer_prune_stats": (_int, [_vp]),
     "genpc_chamfer_scan_kind": (_int, [_int, _int, _int]),
     "genpc_chamfer_sort_layout": (_int, [_int, _int, _int, _int, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]),
-    "genpc_tc_probe": (_int, [_vp, _vp, _vp, _vp]),
     "genpc_host_feed_create": (_int, [ctypes.POINTER(_vp)]),
     "genpc_host_feed_destroy": (_int, [_vp]),
     "genpc_host_feed_error": (_int, [_vp, _vp]),

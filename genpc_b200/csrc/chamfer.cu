@@ -19,15 +19,11 @@
 
 #include "nn_core.cuh"
 #include "nn_sym.cuh"
-#include "nn_tc.cuh"
 #include "nn_prune.cuh"
 #include "nn_grid.cuh"
 
 #ifndef GENPC_DEFAULT_SYM
 #define GENPC_DEFAULT_SYM true
-#endif
-#ifndef GENPC_DEFAULT_PERSIST
-#define GENPC_DEFAULT_PERSIST false
 #endif
 #ifndef GENPC_DEFAULT_BALANCED
 #define GENPC_DEFAULT_BALANCED true
@@ -208,19 +204,6 @@ static cudaError_t launch_scan(const NNParams &p, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
-static unsigned *g_tc_stats = nullptr;   // diagnostics counters of the filter (genpc_chamfer_tc_stats), nullptr in production
-
-// Tensor-core filter (nn_tc.cuh).  MEASURED r02 (profiles/r02c_nn_tc_*): bit-identical results, but the C2 forward takes
-// 0.438 ms against 0.272 ms of the FP32 symmetric scan -- the exact re-evaluation of the winning chunks (every point, once
-// per item) and the stalls it causes in the drain pipeline cost more than the tensor pipe saves at dim = 3 -- so it is
-// OFF by default: GENPC_CHAMFER_TC=1 selects it for any shape with at least one full row block (tests, experiments).
-static bool tc_eligible(int B, int nr, int nc) {
-    (void)B;
-    const char *k = tunable("GENPC_CHAMFER_TC");
-    if (k == nullptr || atoi(k) != 1) return false;
-    return nr >= TC_RBLK && nc >= 1;
-}
-
 // Spatially pruned exact scan (nn_prune.cuh, r02): Hilbert-ordered clouds, one warp per 32 queries, blocks visited nearest first.
 // GENPC_CHAMFER_PRUNE=1 forces it for any shape it can take (64 .. 32768 points per cloud), =0 forbids it; by default it takes
 // device-resident batches whose exhaustive scan is at least 2^30 distance evaluations with >= 2048 points per cloud -- BASELINE C2
@@ -232,8 +215,6 @@ static bool prune_eligible(int B, int nr, int nc) {
     if (!prune_shape_ok(nr, nc)) return false;
     const char *k = tunable("GENPC_CHAMFER_PRUNE");
     if (k != nullptr) return atoi(k) == 1;
-    const char *tc = tunable("GENPC_CHAMFER_TC");
-    if (tc != nullptr && atoi(tc) == 1) return false;   // an explicit request for the tensor-core filter wins over the default
     // (>= 2048 points per cloud: a thousand 1.8 K-point clouds -- the ICP scale search -- pay one sort CTA per cloud for next to
     // nothing: 72.6 vs 66.2 ms per search)
     return nr >= 2048 && nc >= 2048 && (long long)B * nr * nc >= (1LL << 30);
@@ -430,7 +411,7 @@ static int launch_prune_subbatch(const float *rows, const float *cols, int nr, i
 // Symmetric path: rows = the larger cloud (registers), cols = the smaller one (shared-memory sweep).
 // gate != nullptr: host-fed launch (nn_sym_gated_kernel), see genpc_chamfer_forward_host.
 static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist1, float *dist2, int *idx1, int *idx2,
-                               int B, int N, int M, unsigned long long *packed, int *counter, cudaStream_t stream,
+                               int B, int N, int M, unsigned long long *packed, int *ctl, cudaStream_t stream,
                                const unsigned *gate = nullptr, unsigned gate_gen = 0, int gate_pairs = 1,
                                const genpc_chamfer_fuse_t *fuse = nullptr, double *fuse_partial = nullptr,
                                unsigned *fuse_ticket = nullptr, void *prune_extra = nullptr, const int *prune_chunks = nullptr) {
@@ -444,10 +425,9 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     p.rblock_base = 0;
     p.gate = gate, p.gate_gen = gate_gen, p.gate_pairs = gate_pairs;
     p.select = nullptr;
-    // ---- tensor-core filter (nn_tc.cuh): both launches are queued, a device-side flag written by the precheck decides which
-    // one does the work (coordinates at unit scale -> nn_tc_kernel, anything else -> the FP32 kernel below) ----
-    int *ctl = counter;   // [0] persistent work counter, [1] selection flag, [2] precheck accumulator, [3] precheck ticket
-    // ---- spatially pruned scan (nn_prune.cuh): the sort doubles as the range check and sets the same selection flag ----
+    // ---- spatially pruned scan (nn_prune.cuh): both it and the exhaustive kernel below are queued; the selection flag ctl[1],
+    // written by the sort's range check or by the grid probe, decides on the device which one does the work.  ctl[2] / ctl[3]:
+    // accumulator and ticket of the range check (ctl[2] also counts the probe's block visits); ctl[0] has no user ----
     const bool use_grid = ctl != nullptr && gate == nullptr && prune_extra != nullptr && B <= 8 && grid_eligible(p.nr, p.nc);   // one sort per cloud: small batches only
     const bool use_prune = use_grid || (ctl != nullptr && gate == nullptr && prune_extra != nullptr && prune_eligible(B, p.nr, p.nc));
     if (use_grid) {
@@ -525,50 +505,18 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         }
         p.select = ctl + 1;
     }
-    const bool use_tc = !use_prune && ctl != nullptr && tc_eligible(B, p.nr, p.nc);
-    if (use_tc) {
-        static bool attr_done = false;   // opt in to 166 KB of dynamic shared memory once per process
-        if (!attr_done) {
-            cudaError_t ea = cudaFuncSetAttribute(nn_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TcSmem));
-            if (ea == cudaSuccess) ea = cudaFuncSetAttribute(nn_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TcSmem));
-            if (ea != cudaSuccess) return (int)ea;
-            attr_done = true;
-        }
-        const char *lim = tunable("GENPC_TC_LIMIT");
-        const float limit = lim != nullptr ? (float)atof(lim) : 2.0f;
-        if (gate == nullptr) {
-            nn_tc_precheck_kernel<<<2 * GENPC_NUM_SMS, 256, 0, stream>>>(p.rows, (size_t)B * p.nr * 3, p.cols, (size_t)B * p.nc * 3, limit, ctl);
-            GENPC_CHECK_LAUNCH();
-            p.select = ctl + 1;
-        }   // host-fed launches cannot look at data that has not arrived: the caller vouches for the range (get_loss_from_host)
-        TcParams t = {};
-        t.rows = p.rows, t.cols = p.cols, t.prow = p.prow, t.pcol = p.pcol, t.B = B, t.nr = p.nr, t.nc = p.nc;
-        t.rblks = (p.nr + TC_RBLK - 1) / TC_RBLK, t.total_units = B * t.rblks;
-        t.select = p.select, t.gate = gate, t.gate_gen = gate_gen, t.gate_pairs = gate_pairs, t.stats = g_tc_stats;
-        const int grid = t.total_units < GENPC_NUM_SMS ? t.total_units : GENPC_NUM_SMS;
-        if (gate != nullptr) nn_tc_kernel<true><<<grid, TC_THREADS, sizeof(TcSmem), stream>>>(t);
-        else nn_tc_kernel<false><<<grid, TC_THREADS, sizeof(TcSmem), stream>>>(t);
-        GENPC_CHECK_LAUNCH();
-    }
-    const bool fp32_needed = !use_tc || gate == nullptr;   // gated + filter: the filter is the only launch
     // measured on B200 (profiles/r01c_sym_variants.txt): QT=4 at 3 CTAs/SM is within 1 % of QT=8 at 2 CTAs/SM on
     // large clouds and clearly better when the grid is small
-    int QT = p.nr >= 1024 ? 4 : 2;
-    const char *fq = tunable("GENPC_SYM_QT");  // experiments only
-    if (gate == nullptr && fq != nullptr && (atoi(fq) == 8 || atoi(fq) == 6 || atoi(fq) == 4 || atoi(fq) == 2)) QT = atoi(fq);
+    const int QT = p.nr >= 1024 ? 4 : 2;
     p.rtiles = (p.nr + SYM_THREADS * QT - 1) / (SYM_THREADS * QT);
     // column span: the largest that still gives >= 2 waves of work items (3 CTAs x 148 SMs), at least 256 columns
     int span = SYM_SPAN_MAX;
     const long long want = 2LL * 3 * GENPC_NUM_SMS;
     while (span > 256 && (long long)B * p.rtiles * ((p.nc + span - 1) / span) < want) span >>= 1;
-    const char *fs = tunable("GENPC_SYM_SPAN");
-    if (fs != nullptr && atoi(fs) >= 32 && atoi(fs) <= SYM_SPAN_MAX && atoi(fs) % 32 == 0) span = atoi(fs);
     p.span = span;
     p.cspans = (p.nc + span - 1) / span;
     const long long items = (long long)B * p.rtiles * p.cspans;
     if (items > 0x7fffffffLL) return GENPC_ERR_RANGE;
-    const char *pm = tunable("GENPC_SYM_PERSIST");
-    const bool persist = (pm == nullptr) ? GENPC_DEFAULT_PERSIST : (atoi(pm) != 0);
     // measured on B200 (profiles/r01h_sym_balanced_vs_grid.txt): with fewer than two waves of full-span work items the
     // balanced form wins (B=1 16384^2 +5 %, 3 x 5000 x 3333 +12 %); with more, one CTA per item is 4-5 % faster (resident
     // CTAs drift out of phase, so staging / publishing of one overlaps the scan of the other)
@@ -577,12 +525,10 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     // (the pruned grid scan queues this launch only as the device-selected fall-back: a fixed-size grid returns at once,
     // one CTA per work item of a 1M x 1M pair spent 0.8 ms launching CTAs that do nothing)
     const bool balanced = (bm == nullptr) ? ((GENPC_DEFAULT_BALANCED && few_items) || use_grid) : (atoi(bm) != 0);
-    if (!fp32_needed) {
-        // nothing: nn_tc_kernel<true> does the whole scan
-    } else if (gate != nullptr) {
+    if (gate != nullptr) {
         if (QT >= 4) nn_sym_gated_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
         else nn_sym_gated_kernel<2><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
-    } else if (balanced && !persist && (QT == 4 || QT == 2)) {
+    } else if (balanced) {
         // balanced grid: 2 resident CTAs per SM, each walks an equal share of the (row tile x 32-column block) units
         const int upj = (p.nc + 31) / 32;
         const long long units = (long long)B * p.rtiles * upj;
@@ -590,22 +536,9 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         const int grid = (int)(units < 2LL * GENPC_NUM_SMS ? units : 2LL * GENPC_NUM_SMS);
         if (QT == 4) nn_sym_balanced_kernel<4><<<grid, SYM_THREADS, 0, stream>>>(p, (int)units, upj);
         else nn_sym_balanced_kernel<2><<<grid, SYM_THREADS, 0, stream>>>(p, (int)units, upj);
-#if GENPC_SYM_SPAN_MAX <= 1024
-    } else if (persist && (QT == 4 || QT == 2) && counter != nullptr) {
-        // persistent grid: 2 CTAs per SM, items handed out by an atomic counter, next span prefetched with cp.async
-        const int grid = (int)(items < 2LL * GENPC_NUM_SMS ? items : 2LL * GENPC_NUM_SMS);
-        if (QT == 4) nn_sym_persistent_kernel<4><<<grid, SYM_THREADS, 0, stream>>>(p, (int)items, counter);
-        else nn_sym_persistent_kernel<2><<<grid, SYM_THREADS, 0, stream>>>(p, (int)items, counter);
-#endif
-    } else if (QT == 4 && tunable("GENPC_SYM_TMA") != nullptr && atoi(tunable("GENPC_SYM_TMA")) == 1 && p.nc % 4 == 0 && p.span % 4 == 0 &&
-               (reinterpret_cast<size_t>(p.cols) & 15) == 0) {
-        nn_sym_tma_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);   // r02 experiment: TMA bulk staging
-    } else
-    switch (QT) {
-        case 8: nn_sym_kernel<8><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p); break;
-        case 6: nn_sym_kernel<6><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p); break;
-        case 4: nn_sym_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p); break;
-        default: nn_sym_kernel<2><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p); break;
+    } else {
+        if (QT == 4) nn_sym_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
+        else nn_sym_kernel<2><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
     }
     GENPC_CHECK_LAUNCH();
     const size_t nrw = (size_t)B * p.nr, ncw = (size_t)B * p.nc;
@@ -613,9 +546,8 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     const unsigned unpack_blocks = (unsigned)((nrw + EPI_ROWS_PER_CTA - 1) / EPI_ROWS_PER_CTA);
     EpiFuse f;
     memset(&f, 0, sizeof(f));
-    // column words are exact iff the filter did the work: ctl[1] == 0 after the precheck; a gated launch has no precheck and
-    // points at ctl[2], which is zero between launches
-    f.select = use_tc ? (gate == nullptr ? ctl + 1 : ctl + 2) : (use_prune ? ctl + 1 : nullptr);
+    // column words are exact iff the pruned scan did the work (ctl[1] == 0)
+    f.select = use_prune ? ctl + 1 : nullptr;
     if (fuse == nullptr) {
         nn_sym_epilogue_kernel<false><<<fix_blocks + unpack_blocks, 256, 0, stream>>>(
             p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT, fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
@@ -646,7 +578,7 @@ static size_t sym_epilogue_ctas(int B, int N, int M) {
 
 using namespace genpc;
 
-// packed words + work-item counter / selection words
+// packed words + 16 control bytes (selection flag, accumulator and ticket of the pruned scans; chamfer_forward_sym)
 static size_t chamfer_base_bytes(int B, int N, int M) { return ((size_t)B * N + (size_t)B * M) * sizeof(unsigned long long) + 16; }
 
 extern "C" size_t genpc_chamfer_workspace_bytes(int B, int N, int M) {
@@ -723,23 +655,18 @@ extern "C" int genpc_chamfer_forward_fused(const float *xyz1, const float *xyz2,
     const bool sym = takes_sym_path(N, M);
     if (!(sym && fuse != nullptr && fuse->workspace_armed)) {  // an armed workspace already holds all-ones words
         e = cudaMemsetAsync(packed, 0xff, (n1 + n2) * 8, stream);
-        if (e == cudaSuccess) e = cudaMemsetAsync(packed + n1 + n2, 0, 16, stream);   // control words (counter, filter flag / ticket)
+        if (e == cudaSuccess) e = cudaMemsetAsync(packed + n1 + n2, 0, 16, stream);   // control words (selection flag, accumulator, ticket)
         if (e != cudaSuccess) return (int)e;
     }
     if (sym) {
-        int *counter = (int *)(packed + n1 + n2);  // work-item counter of the persistent kernel (after the packed words)
-        const char *pm = tunable("GENPC_SYM_PERSIST");
-        if ((pm == nullptr) ? GENPC_DEFAULT_PERSIST : (atoi(pm) != 0)) {
-            e = cudaMemsetAsync(counter, 0, 16, stream);
-            if (e != cudaSuccess) return (int)e;
-        }
+        int *ctl = (int *)(packed + n1 + n2);  // control words of the pruned scans (after the packed words)
         double *partial = fuse ? (double *)fuse->loss_workspace : nullptr;
         unsigned *ticket = partial ? (unsigned *)(partial + sym_epilogue_ctas(B, N, M)) : nullptr;
         // (a workspace sized while the knob was off stays on the exhaustive kernels)
         const size_t base_bytes = chamfer_base_bytes(B, N, M);
         void *extra = (prune_extra_bytes(B, N, M) != 0 && workspace_bytes >= base_bytes + prune_extra_bytes(B, N, M))
                           ? (void *)((char *)(packed + n1 + n2) + 16) : nullptr;
-        return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, packed, counter, stream, nullptr, 0, 1, fuse,
+        return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, packed, ctl, stream, nullptr, 0, 1, fuse,
                                    partial, ticket, extra);
     }
 
@@ -789,16 +716,15 @@ extern "C" int genpc_chamfer_backward(const float *xyz1, const float *xyz2, cons
     return GENPC_OK;
 }
 
-// Diagnostics of the tensor-core filter: while `stats4` (device, 4 x u32, zeroed by the caller) is set, every filter launch
-// adds {runner-up chunk re-evaluations, whole-tile exact scans, degenerate items, items} to it.  nullptr switches it off.
-// Which scan genpc_chamfer_forward would queue for this shape with the current knobs (host logic only, no device call):
-// 0 = exhaustive (symmetric or per-direction), 1 = Hilbert-sorted pruned scan (nn_prune.cuh), 2 = two-level pruned scan for large
-// clouds (nn_grid.cuh).  The device may still hand a pruned launch back to the exhaustive kernels (range / overlap / probe).
+// The pruned scan's sort layout for B cloud pairs on a part with `sms` SMs (<= 0: 148) -- sort_layout above, host logic only.
 extern "C" int genpc_chamfer_sort_layout(int B, int N, int M, int sms, int *mixed, int *grid) {
     if (B <= 0 || N <= 0 || M <= 0 || mixed == nullptr || grid == nullptr) return GENPC_ERR_SHAPE;
     return sort_layout(B, N > M ? N : M, N > M ? M : N, sms > 0 ? sms : GENPC_NUM_SMS_B200, mixed, grid);
 }
 
+// Which scan genpc_chamfer_forward would queue for this shape with the current knobs (host logic only, no device call):
+// 0 = exhaustive (symmetric or per-direction), 1 = Hilbert-sorted pruned scan (nn_prune.cuh), 2 = two-level pruned scan for large
+// clouds (nn_grid.cuh).  The device may still hand a pruned launch back to the exhaustive kernels (range / overlap / probe).
 extern "C" int genpc_chamfer_scan_kind(int B, int N, int M) {
     if (B <= 0 || N <= 0 || M <= 0) return GENPC_ERR_SHAPE;
     if (!takes_sym_path(N, M)) return 0;
@@ -810,19 +736,6 @@ extern "C" int genpc_chamfer_scan_kind(int B, int N, int M) {
 // diagnostics of the pruned scan: stats4 = device pointer to 4 counters (blocks scanned, groups that took the tie pass, groups, -)
 extern "C" int genpc_chamfer_prune_stats(unsigned *stats4) {
     g_prune_stats = stats4;
-    return GENPC_OK;
-}
-
-extern "C" int genpc_chamfer_tc_stats(unsigned *stats4) {
-    g_tc_stats = stats4;
-    return GENPC_OK;
-}
-
-// Test probe: e(x,y) = u(x).v(y) of one 128 x 256 tile as the tensor pipe computes it (rows128 [128][3], cols256 [256][3],
-// e_out [128][256], all device memory).
-extern "C" int genpc_tc_probe(const float *rows128, const float *cols256, float *e_out, genpc_stream_t stream_) {
-    nn_tc_probe_kernel<<<1, 128, 0, (cudaStream_t)stream_>>>(rows128, cols256, e_out);
-    GENPC_CHECK_LAUNCH();
     return GENPC_OK;
 }
 

@@ -1048,16 +1048,14 @@ extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *di
     int dev = 0, sms = 0, per_sm = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const char *pmb = tunable("GENPC_EMD_PRUNE_MINB");  // experiments only
-    // three CTAs per SM (80 registers) beat four (64 registers, spills) on every shape of a same-box A/B
+    // pruned: three CTAs per SM (80 registers) beat four (64 registers, spills) on every shape of a same-box A/B
     // (profiles/r02k_emd_prune.txt)
-    const bool mb4 = pmb != nullptr && atoi(pmb) == 4;
     void *kernel = (void *)emd_auction_kernel<0, 5>;
     if (prune) {
         const int nblk = n / EMD_BLOCK;
-        if (nblk <= 128) kernel = mb4 ? (void *)emd_auction_kernel<4, 4> : (void *)emd_auction_kernel<4, 3>;
-        else if (nblk <= 256) kernel = mb4 ? (void *)emd_auction_kernel<8, 4> : (void *)emd_auction_kernel<8, 3>;
-        else kernel = mb4 ? (void *)emd_auction_kernel<16, 4> : (void *)emd_auction_kernel<16, 3>;
+        if (nblk <= 128) kernel = (void *)emd_auction_kernel<4, 3>;
+        else if (nblk <= 256) kernel = (void *)emd_auction_kernel<8, 3>;
+        else kernel = (void *)emd_auction_kernel<16, 3>;
     }
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, EMD_THREADS, 0);
     if (e != cudaSuccess) return (int)e;
@@ -1087,15 +1085,9 @@ extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *di
     // same-box sweep (ms: B1 n8192 | B32 n8192 | B1 n16384 | B20 n2048): 64: 1.10 | 2.48 | 1.24 | 0.99;  256: 1.08 | 2.47 | 1.24 | 0.91;
     // 512: 1.04 | 2.45 | 1.23 | 0.90;  1024: 1.08 | 2.48 | 1.31 | 0.90;  2048: 1.10 | 2.51 | 1.38 | 0.89;  4096: 1.12 | 2.53 | 1.43 | 0.90
     a.tail_spread_u = 512;
-    const char *tsu = tunable("GENPC_EMD_TAIL_SPREAD");  // experiments only
-    if (tsu != nullptr) a.tail_spread_u = atoi(tsu);
     a.two_level_div = 8;
     const char *gm = tunable("GENPC_EMD_GETMAX");  // "lowest": the other legitimate outcome of the reference's race
     a.getmax_lowest = (gm != nullptr && strcmp(gm, "lowest") == 0) ? 1 : 0;
-    const char *tl = tunable("GENPC_EMD_TWO_LEVEL");  // experiments only
-    if (tl != nullptr) a.two_level_div = atoi(tl);
-    const char *dp = tunable("GENPC_EMD_DIRECT_P");  // experiments only
-    if (dp != nullptr) a.direct_p = atoi(dp);
     if ((reinterpret_cast<size_t>(xyz2) & 7) != 0 || (reinterpret_cast<size_t>(price) & 7) != 0) a.direct_p = 0;  // LDG.64
     if (prune) {
         float4 *tsort = reinterpret_cast<float4 *>(static_cast<char *>(workspace) + emd_ctl_bytes(B));

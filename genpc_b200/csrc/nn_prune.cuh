@@ -20,7 +20,7 @@
 // that saw the same minimum in two chunks takes a second pass over the surviving blocks).  The box distance is scaled
 // down by 1e-5, far more than the rounding of the reference's arithmetic, and compared with <= so that ties are kept.
 // The sort kernel doubles as the range check (NaN / Inf / |x| > 1e15 -> the exhaustive kernel runs instead, selected on
-// the device through the same flag as the tensor-core filter).
+// the device through a flag in the control words that the exhaustive kernel and the epilogue read).
 #pragma once
 #include <cooperative_groups.h>
 
@@ -86,7 +86,7 @@ struct PruneSortParams {
     int n[2];
     int B;
     float limit;
-    int *ctl;              // [1] selection flag (0: pruned kernels run), [2] accumulator, [3] ticket -- as nn_tc_precheck_kernel
+    int *ctl;              // [1] selection flag (0: pruned kernels run), [2] accumulator, [3] ticket of the range check
     int hilbert;           // cell order: Hilbert curve (1) or Z-order (0)
     float *bbx;            // optional [2][B][8]: every cloud's bounding box, for the overlap test below (nullptr: none)
     int accumulate;        // 1: OR the verdict into ctl[1] (a later chunk of the same batch), 0: overwrite it

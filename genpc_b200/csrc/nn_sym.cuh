@@ -10,7 +10,7 @@
 //   row side: running minimum by FMNMX3, winning 8-column chunk id tracked, exact lowest index recovered by a
 //             re-scan of that chunk, merged across column spans by a packed 64-bit atomicMin (as nn_core.cuh);
 //   col side: per 32-column block every lane folds its QT rows into 32 accumulators (FMNMX3 over row pairs),
-//             a 31-step butterfly (SHFL + FMNMX) leaves lane l with the warp-wide minimum of column l, and ONE
+//             one warp reduction per column (REDUX.MIN) leaves lane l with the warp-wide minimum of column l, and ONE
 //             coalesced 64-bit atomicMin per lane publishes (dist_bits << 32 | row_block_id).  The exact lowest
 //             row index is recovered afterwards by nn_sym_epilogue_kernel, which re-scans only the winning
 //             32*QT-row block of each column (lowest block wins ties, first match inside it => lowest index).
@@ -20,15 +20,9 @@
 namespace genpc {
 
 constexpr int SYM_THREADS = 256;
-#ifndef GENPC_SYM_SPAN_MAX
-#define GENPC_SYM_SPAN_MAX 1024
-#endif
-constexpr int SYM_SPAN_MAX = GENPC_SYM_SPAN_MAX;  // columns staged per item (12 B of shared memory each)
+constexpr int SYM_SPAN_MAX = 1024;  // columns staged per item (12 B of shared memory each)
 #ifndef GENPC_SYM_CHUNK
 #define GENPC_SYM_CHUNK 8
-#endif
-#ifndef GENPC_SYM_REDUX
-#define GENPC_SYM_REDUX 1
 #endif
 constexpr int SYM_CHUNK = GENPC_SYM_CHUNK;  // row-side index-recovery granularity (columns)
 
@@ -44,8 +38,8 @@ struct SymParams {
     const unsigned *gate;
     unsigned gate_gen;
     int gate_pairs;
-    // tensor-core filter selection (nn_tc.cuh): when set, this FP32 launch only runs if *select != 0, i.e. the precheck
-    // found coordinates outside the filter's range; nullptr: always run
+    // selection flag of the pruned scans (nn_prune.cuh, nn_grid.cuh): when set, this launch only runs if *select != 0, i.e.
+    // the sort's range check or the grid probe handed the work back to the exhaustive kernels; nullptr: always run
     const int *select;
 };
 
@@ -56,77 +50,33 @@ __device__ __forceinline__ float ld_coord(const float *p) {
     return COHERENT ? __ldcg(p) : __ldg(p);
 }
 
-// v[e] (e = 0..31) per lane -> returns min over all lanes of v[lane]   (element index == lane id)
-__device__ __forceinline__ float butterfly_min32(float (&v)[32], int lane) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) {
-        const bool up = (lane & o) != 0;
-#pragma unroll
-        for (int i = 0; i < o; ++i) {
-            const float keep = up ? v[i + o] : v[i];
-            const float send = up ? v[i] : v[i + o];
-            v[i] = fminf(keep, __shfl_xor_sync(0xffffffffu, send, o));
-        }
-    }
-    return v[0];
-}
-
-#ifndef GENPC_SYM_MINB8
-#define GENPC_SYM_MINB8 2
-#endif
-#ifndef GENPC_SYM_MINB4
-#define GENPC_SYM_MINB4 2
-#endif
-#ifndef GENPC_SYM_EXPAND
-#define GENPC_SYM_EXPAND 0
-#endif
-#define GENPC_SYM_MINB(QT) ((QT) >= 8 ? GENPC_SYM_MINB8 : GENPC_SYM_MINB4)
-
 // One work item: row tile `rt` (SYM_THREADS*QT rows) x column span [c0, c0+span) of ONE cloud pair.
 // rows/cols/prow/pcol point at the first element of the pair's clouds / packed words.  colT: optional similarity
 // applied to the columns while they are staged (registration: the moving cloud), nullptr = identity.
-// PRESTAGED: the caller already holds the (NaN padded) span in `s` and has synchronised (persistent kernel).
-template <int QT, bool PRESTAGED = false, bool COHERENT = false>
+template <int QT, bool COHERENT = false>
 __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const float *__restrict__ rows, int nr, int rt,
                                             const float *__restrict__ cols, int nc, int c0, int span,
                                             const Similarity *colT, unsigned long long *__restrict__ prow_,
                                             unsigned long long *__restrict__ pcol_, int rblock_base = 0) {
     static_assert(QT % 2 == 0, "rows are folded in pairs");
-#if GENPC_SYM_REDUX == 2
-    __shared__ unsigned scol[SYM_THREADS / 32][32];
-#endif
-#if GENPC_SYM_EXPAND
-    // TIMING EXPERIMENT ONLY (tools/nn_variants.cu -DGENPC_SYM_EXPAND=1): e = |y|^2 - 2 x.y + |x|^2 in 4 packed
-    // instructions per two pairs instead of 6 -- results are NOT the reference's bits; upper bound of the norm-expansion
-    // filter without any of the exactness machinery.  See DESIGN.md section 4.1b.
-    __shared__ __align__(16) float sn[SYM_SPAN_MAX];
-#endif
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cnt = min(span, nc - c0);
     const int cnt32 = (cnt + 31) & ~31;
     const float qnan = __int_as_float(0x7fc00000);
     // ---- stage the column span ----
-    if (!PRESTAGED) {
-        const float *cp = cols + (size_t)c0 * 3;
-        for (int k = tid; k < cnt32; k += SYM_THREADS) {
-            float x = qnan, y = qnan, z = qnan;
-            if (k < cnt) {
-                x = ld_coord<COHERENT>(cp + k * 3), y = ld_coord<COHERENT>(cp + k * 3 + 1), z = ld_coord<COHERENT>(cp + k * 3 + 2);
-                if (colT != nullptr) apply_similarity(*colT, x, y, z);
-            }
-            s[0][k] = x, s[1][k] = y, s[2][k] = z;
-#if GENPC_SYM_EXPAND
-            sn[k] = fmaf(x, x, fmaf(y, y, z * z));
-#endif
+    const float *cp = cols + (size_t)c0 * 3;
+    for (int k = tid; k < cnt32; k += SYM_THREADS) {
+        float x = qnan, y = qnan, z = qnan;
+        if (k < cnt) {
+            x = ld_coord<COHERENT>(cp + k * 3), y = ld_coord<COHERENT>(cp + k * 3 + 1), z = ld_coord<COHERENT>(cp + k * 3 + 2);
+            if (colT != nullptr) apply_similarity(*colT, x, y, z);
         }
+        s[0][k] = x, s[1][k] = y, s[2][k] = z;
     }
     // ---- rows into registers (negated; NaN for out-of-range rows: they never win a min on either side) ----
     float2 nqx[QT], nqy[QT], nqz[QT];
     float best[QT];
     int bchunk[QT];
-#if GENPC_SYM_EXPAND
-    float nrm[QT];
-#endif
     const int rblock = rt * (SYM_THREADS / 32) + warp;          // global id of this warp's 32*QT-row block
     const int jbase = rblock * (32 * QT) + lane;
     const float *rp = rows;
@@ -137,20 +87,13 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
         if (j < nr)
             x = ld_coord<COHERENT>(rp + (size_t)j * 3), y = ld_coord<COHERENT>(rp + (size_t)j * 3 + 1),
             z = ld_coord<COHERENT>(rp + (size_t)j * 3 + 2);
-#if GENPC_SYM_EXPAND
-        nqx[qi] = make_float2(-2.f * x, -2.f * x);
-        nqy[qi] = make_float2(-2.f * y, -2.f * y);
-        nqz[qi] = make_float2(-2.f * z, -2.f * z);
-        nrm[qi] = fmaf(x, x, fmaf(y, y, z * z));
-#else
         nqx[qi] = make_float2(-x, -x);
         nqy[qi] = make_float2(-y, -y);
         nqz[qi] = make_float2(-z, -z);
-#endif
         best[qi] = __int_as_float(0x7f800000);
         bchunk[qi] = 0;
     }
-    if (!PRESTAGED) __syncthreads();
+    __syncthreads();
 
     const float4 *sx4 = reinterpret_cast<const float4 *>(s[0]);
     const float4 *sy4 = reinterpret_cast<const float4 *>(s[1]);
@@ -171,32 +114,6 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
                 const int g = blk * 8 + sub * (SYM_CHUNK / 4) + kk;  // float4 group index
                 const float4 X = sx4[g], Y = sy4[g], Z = sz4[g];
                 const int t = sub * SYM_CHUNK + kk * 4;               // column offset inside the block
-#if GENPC_SYM_EXPAND
-                const float4 NY = reinterpret_cast<const float4 *>(sn)[g];
-                const float2 nlo = make_float2(NY.x, NY.y), nhi = make_float2(NY.z, NY.w);
-                auto expand_x2 = [](float2 ax, float2 ay, float2 az, float2 tx, float2 ty, float2 tz, float2 ny, float nx) {
-                    return __fadd2_rn(__ffma2_rn(ax, tx, __ffma2_rn(ay, ty, __ffma2_rn(az, tz, ny))), make_float2(nx, nx));
-                };
-#pragma unroll
-                for (int qi = 0; qi < QT; qi += 2) {
-                    const float2 a0 = expand_x2(nqx[qi], nqy[qi], nqz[qi], make_float2(X.x, X.y), make_float2(Y.x, Y.y),
-                                                make_float2(Z.x, Z.y), nlo, nrm[qi]);
-                    const float2 e0 = expand_x2(nqx[qi], nqy[qi], nqz[qi], make_float2(X.z, X.w), make_float2(Y.z, Y.w),
-                                                make_float2(Z.z, Z.w), nhi, nrm[qi]);
-                    const float2 a1 = expand_x2(nqx[qi + 1], nqy[qi + 1], nqz[qi + 1], make_float2(X.x, X.y),
-                                                make_float2(Y.x, Y.y), make_float2(Z.x, Z.y), nlo, nrm[qi + 1]);
-                    const float2 e1 = expand_x2(nqx[qi + 1], nqy[qi + 1], nqz[qi + 1], make_float2(X.z, X.w),
-                                                make_float2(Y.z, Y.w), make_float2(Z.z, Z.w), nhi, nrm[qi + 1]);
-                    cm[qi] = fmin3(cm[qi], a0.x, a0.y);
-                    cm[qi] = fmin3(cm[qi], e0.x, e0.y);
-                    cm[qi + 1] = fmin3(cm[qi + 1], a1.x, a1.y);
-                    cm[qi + 1] = fmin3(cm[qi + 1], e1.x, e1.y);
-                    cacc[t + 0] = fmin3(cacc[t + 0], a0.x, a1.x);
-                    cacc[t + 1] = fmin3(cacc[t + 1], a0.y, a1.y);
-                    cacc[t + 2] = fmin3(cacc[t + 2], e0.x, e1.x);
-                    cacc[t + 3] = fmin3(cacc[t + 3], e0.y, e1.y);
-                }
-#else
 #pragma unroll
                 for (int qi = 0; qi < QT; qi += 2) {
                     const float2 a0 = sqdist_ref_x2(nqx[qi], nqy[qi], nqz[qi], make_float2(X.x, X.y),
@@ -216,7 +133,6 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
                     cacc[t + 2] = fmin3(cacc[t + 2], e0.x, e1.x);
                     cacc[t + 3] = fmin3(cacc[t + 3], e0.y, e1.y);
                 }
-#endif
             }
 #pragma unroll
             for (int qi = 0; qi < QT; ++qi) {
@@ -227,18 +143,6 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
             }
         }
         // ---- column side: warp-wide minimum of column (blk*32 + lane), published with the row-block id ----
-#if GENPC_SYM_REDUX == 2
-        // warp minimum of every column by REDUX, parked in shared memory by lane 0 (LSU pipe) and picked up with one
-        // LDS per lane -- keeps the per-column select (ISETP + SEL) off the ALU pipe, which bounds this kernel
-#pragma unroll
-        for (int c = 0; c < 32; ++c) {
-            const unsigned r = __reduce_min_sync(0xffffffffu, __float_as_uint(cacc[c]));
-            if (lane == 0) scol[warp][c] = r;
-        }
-        __syncwarp();
-        const float cmin = __uint_as_float(scol[warp][lane]);
-        __syncwarp();
-#elif GENPC_SYM_REDUX
         unsigned mine = 0x7f800000u;  // distances are >= 0: their bit patterns order like the floats
 #pragma unroll
         for (int c = 0; c < 32; ++c) {
@@ -246,9 +150,6 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
             if (lane == c) mine = r;
         }
         const float cmin = __uint_as_float(mine);
-#else
-        const float cmin = butterfly_min32(cacc, lane);
-#endif
         // every in-range column publishes, also when its minimum is +inf (NaN / overflowing coordinates): no packed word
         // is ever left unarmed, so the epilogue and the gradient kernels always see an in-range block / index
         const int col = blk * 32 + lane;
@@ -276,7 +177,7 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
 }
 
 template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_kernel(const SymParams p) {
+__global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_kernel(const SymParams p) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
     if (p.select != nullptr && *p.select == 0) return;
     int item = blockIdx.x;
@@ -286,56 +187,6 @@ __global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_kernel
     const int b = item / p.rtiles;
     nn_sym_item<QT>(s, p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, cs * p.span, p.span,
                     nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
-}
-
-// TMA-staged form (r02 experiment, GENPC_SYM_TMA=1): the column span is contiguous in the AoS cloud (span * 12 bytes), so ONE
-// bulk asynchronous copy (cp.async.bulk.shared::cluster.global, completion on an mbarrier -- the TMA engine, UBLKCP in SASS)
-// brings it into a raw shared-memory buffer while the threads load their rows; the AoS -> SoA transposition is then a
-// shared -> shared pass (12-byte lane stride: conflict free) instead of three scalar LDG -> STS per point.  Needs a 16-byte
-// aligned span start and a span size that is a multiple of 16 bytes; the caller falls back to nn_sym_kernel otherwise.
-// Measured (profiles/r02d_sym_tma.txt): no gain on C2 -- see DESIGN.md section 4.1.
-template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_tma_kernel(const SymParams p) {
-    __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
-    __shared__ __align__(128) float raw[3 * SYM_SPAN_MAX];
-    __shared__ __align__(8) unsigned long long bar;
-    if (p.select != nullptr && *p.select == 0) return;
-    int item = blockIdx.x;
-    const int cs = item % p.cspans;
-    item /= p.cspans;
-    const int rt = item % p.rtiles;
-    const int b = item / p.rtiles;
-    const int tid = threadIdx.x;
-    const int c0 = cs * p.span, cnt = min(p.span, p.nc - c0), cnt32 = (cnt + 31) & ~31;
-    const float *cp = p.cols + ((size_t)b * p.nc + c0) * 3;
-    const unsigned bytes = (unsigned)cnt * 12u;
-    const unsigned bar_a = (unsigned)__cvta_generic_to_shared(&bar);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         (unsigned)__cvta_generic_to_shared(raw)),
-                     "l"(cp), "r"(bytes), "r"(bar_a)
-                     : "memory");
-    }
-    __syncthreads();   // the barrier is initialised before anybody polls it
-    {
-        unsigned ok = 0;
-        while (!ok)
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(ok)
-                         : "r"(bar_a)
-                         : "memory");
-    }
-    const float qnan = __int_as_float(0x7fc00000);
-    for (int k = tid; k < cnt32; k += SYM_THREADS) {
-        const bool in = k < cnt;
-        s[0][k] = in ? raw[3 * k] : qnan, s[1][k] = in ? raw[3 * k + 1] : qnan, s[2][k] = in ? raw[3 * k + 2] : qnan;
-    }
-    __syncthreads();
-    nn_sym_item<QT, true>(s, p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, c0, p.span, nullptr,
-                          p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
 }
 
 // Host-fed form: same work items, but the clouds are still arriving from pinned host memory while the kernel runs.
@@ -349,7 +200,7 @@ constexpr int GATE_ERR_SLOT = GATE_MAX_CHUNKS;
 constexpr long long GATE_TIMEOUT_CLK = 4000000000LL;  // ~2 s at 1.965 GHz
 
 template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_gated_kernel(const SymParams p) {
+__global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_gated_kernel(const SymParams p) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
     if (p.select != nullptr && *p.select == 0) return;
     int item = blockIdx.x;
@@ -372,8 +223,8 @@ __global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_gated_
         }
     }
     __syncthreads();
-    nn_sym_item<QT, false, true>(s, p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, cs * p.span,
-                                 p.span, nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
+    nn_sym_item<QT, true>(s, p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, cs * p.span,
+                          p.span, nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
 }
 
 // Balanced form ("stream-K" over the distance matrix): the work of the whole launch is counted in UNITS of one row
@@ -383,8 +234,8 @@ __global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_gated_
 // +-1 whatever the problem shape: no partial last wave (C2: 1024 items over 296 slots = 3.46 waves before) and
 // B = 1 problems fill the machine.  Results are merged by the same packed atomicMin words, hence bit-identical.
 template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_balanced_kernel(const SymParams p, int total_units,
-                                                                                         int units_per_job) {
+__global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_balanced_kernel(const SymParams p, int total_units,
+                                                                          int units_per_job) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
     if (p.select != nullptr && *p.select == 0) return;
     int u = (int)((long long)total_units * blockIdx.x / gridDim.x);
@@ -401,62 +252,6 @@ __global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_balanc
         __syncthreads();  // every warp is done with the span before the next item overwrites it
     }
 }
-
-#if GENPC_SYM_SPAN_MAX <= 1024  // the double buffer must fit the 48 KB static shared-memory limit
-// Persistent form: one CTA pair per SM loops over work items handed out by an atomic counter; the NEXT item's column
-// span is copied global -> shared with cp.async (LDGSTS, 4-byte granules so the AoS -> SoA transposition happens in the
-// copy itself) into the other half of a double buffer while the current item is being scanned.
-__device__ __forceinline__ void cp_async_f32(float *smem_dst, const float *gsrc) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
-}
-
-template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) nn_sym_persistent_kernel(const SymParams p, int total, int *counter) {
-    __shared__ __align__(16) float s[2][3][SYM_SPAN_MAX];
-    __shared__ int s_next;
-    const int tid = threadIdx.x;
-    const float qnan = __int_as_float(0x7fc00000);
-    auto stage = [&](int item, int buf) {
-        if (item >= total) return;
-        const int cs = item % p.cspans;
-        const int b = (item / p.cspans) / p.rtiles;
-        const int c0 = cs * p.span;
-        const int cnt = min(p.span, p.nc - c0);
-        const int cnt32 = (cnt + 31) & ~31;
-        const float *cp = p.cols + ((size_t)b * p.nc + c0) * 3;
-        for (int k = tid; k < cnt32; k += SYM_THREADS) {
-            if (k < cnt) {
-                cp_async_f32(&s[buf][0][k], cp + k * 3);
-                cp_async_f32(&s[buf][1][k], cp + k * 3 + 1);
-                cp_async_f32(&s[buf][2][k], cp + k * 3 + 2);
-            } else {
-                s[buf][0][k] = qnan, s[buf][1][k] = qnan, s[buf][2][k] = qnan;
-            }
-        }
-    };
-    int item = blockIdx.x, buf = 0;
-    stage(item, 0);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    while (item < total) {
-        if (tid == 0) s_next = atomicAdd(counter, 1) + (int)gridDim.x;
-        __syncthreads();  // s_next visible; everybody is done with the buffer about to be refilled
-        const int next = s_next;
-        stage(next, buf ^ 1);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        __syncthreads();  // the current span has landed for every thread
-        const int cs = item % p.cspans;
-        const int rest = item / p.cspans;
-        const int rt = rest % p.rtiles;
-        const int b = rest / p.rtiles;
-        nn_sym_item<QT, true>(s[buf], p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, cs * p.span,
-                              p.span, nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
-        item = next;
-        buf ^= 1;
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-}
-#endif
 
 // Exact lowest row index of one column from its published (dist, row block) word: the calling WARP re-scans the
 // winning block (32*NS consecutive rows) for the first row whose distance equals dist.  All NS strips are loaded
@@ -513,7 +308,7 @@ __device__ __forceinline__ int sym_fix_column(const float *__restrict__ rp, int 
         return sym_fix_column_t<4>(rp, nr, cx, cy, cz, d, blk, lane);
     }
     if (rows_per_block == 64) return sym_fix_column_t<2>(rp, nr, cx, cy, cz, d, blk, lane);
-    int found = 0;  // generic (QT = 6 / 8 experiments)
+    int found = 0;  // generic: any other block height
     for (int r0 = blk * rows_per_block; r0 < (blk + 1) * rows_per_block; r0 += 32) {
         const int j = r0 + lane;
         bool hit = false;
@@ -544,7 +339,7 @@ struct EpiFuse {
     float *zero[2];         // buffers to zero-fill, or nullptr
     size_t nzero[2];        // their sizes in floats
     const unsigned *err_flag;  // host-fed launches: the feed's error word -- a timed-out gate poisons the loss with NaN
-    const int *select;         // tensor-core filter selection flag: *select == 0 -> the column words already hold exact indices
+    const int *select;         // selection flag of the pruned scans: *select == 0 -> the column words already hold exact indices
 };
 
 __device__ __forceinline__ void epi_zero_fill(float *z, size_t n, size_t g, size_t total_threads) {
@@ -580,7 +375,7 @@ static __global__ void __launch_bounds__(256) nn_sym_epilogue_kernel(const float
                                                                      float *__restrict__ dist_c, int *__restrict__ idx_c,
                                                                      const EpiFuse f) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const bool cols_exact = f.select != nullptr && *f.select == 0;   // nn_tc_kernel ran: nothing to fix up (warp-uniform)
+    const bool cols_exact = f.select != nullptr && *f.select == 0;   // a pruned scan ran: nothing to fix up (warp-uniform)
     double term = 0.0;  // sum of f(d) over the output elements this thread owns
     if (blockIdx.x >= fix_blocks) {
         const size_t n = (size_t)B * nr;

@@ -356,7 +356,7 @@ __global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) register_persistent_
 // launch 1: rows = fixed cloud (registers), cols = moving cloud (pose applied while staging).
 //           packedB[k] <- (dB_k, moving index)  exact;  packedA[j] <- (dA_j, row block of the fixed cloud).
 template <int QT>
-__global__ void __launch_bounds__(SYM_THREADS, GENPC_SYM_MINB(QT)) register_sym_scan_kernel(const RegArgs a) {
+__global__ void __launch_bounds__(SYM_THREADS, 2) register_sym_scan_kernel(const RegArgs a) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
     __shared__ Similarity T;
     if (a.select != nullptr && *a.select == 0) return;   // the pruned scan did the work
@@ -382,8 +382,6 @@ constexpr int FIX_THREADS = 512;
 // 128 -> 4.41, 256 -> 4.32, 512 -> 4.28 ms per iteration (fewer tickets / partial reductions per point); the largest
 // size that still gives every resident-CTA slot (2 per SM) one CTA is used.
 static int fix_cols_per_cta(int S, int Nc) {
-    const char *e = tunable("GENPC_FIX_COLS");  // experiments only
-    if (e != nullptr && (atoi(e) == 128 || atoi(e) == 256 || atoi(e) == 512)) return atoi(e);
     for (int cols = 512; cols > 128; cols >>= 1)
         if ((long long)S * ((Nc + cols - 1) / cols) >= 2LL * GENPC_NUM_SMS) return cols;
     return 128;
@@ -578,16 +576,11 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
     // queries per thread of the single-launch path: the real pipeline registers 1-3 K-point clouds with 4 starts -- a few
     // dozen CTAs; fewer queries per thread (more, shorter CTAs) while the grid does not fill the GPU twice over
     int QT = nn_pick_qt(Nc < Nr ? Nc : Nr);
-    const char *fq = tunable("GENPC_REGISTER_QT");  // experiments only
-    if (fq != nullptr && (atoi(fq) == 1 || atoi(fq) == 2 || atoi(fq) == 4)) {
-        QT = atoi(fq);
-    } else {
-        while (QT > 1) {
-            const long long items = (long long)((Nc + NN_THREADS * QT - 1) / (NN_THREADS * QT)) * ((Nr + NN_SPAN - 1) / NN_SPAN) +
-                                    (long long)((Nr + NN_THREADS * QT - 1) / (NN_THREADS * QT)) * ((Nc + NN_SPAN - 1) / NN_SPAN);
-            if ((long long)S * items >= 2LL * GENPC_NUM_SMS) break;
-            QT >>= 1;
-        }
+    while (QT > 1) {
+        const long long items = (long long)((Nc + NN_THREADS * QT - 1) / (NN_THREADS * QT)) * ((Nr + NN_SPAN - 1) / NN_SPAN) +
+                                (long long)((Nr + NN_THREADS * QT - 1) / (NN_THREADS * QT)) * ((Nc + NN_SPAN - 1) / NN_SPAN);
+        if ((long long)S * items >= 2LL * GENPC_NUM_SMS) break;
+        QT >>= 1;
     }
     // work items of the single-launch kernels for a given target span (NN_SPAN unless the persistent kernel picks a shorter one)
     auto set_span = [&](int span) {

@@ -1,4 +1,4 @@
-// tunables.cu -- experiment knobs of the library, read from the environment ONCE when the library is loaded.
+// tunables.cu -- run-time knobs of the library (GENPC_*), read from the environment ONCE when the library is loaded.
 //
 // r01 called getenv() on every forward (five times in the Chamfer host path alone).  The knobs now live in a small table
 // that a static initialiser fills from the environment at load time; the hot host paths only do a handful of short
@@ -19,16 +19,11 @@ struct Knob {
 
 static Knob g_knobs[] = {
     {"GENPC_CHAMFER_MODE", "", false},   // "sym" | "scan"
-    {"GENPC_SYM_QT", "", false},         {"GENPC_SYM_SPAN", "", false},     {"GENPC_SYM_PERSIST", "", false},
-    {"GENPC_SYM_BALANCED", "", false},   {"GENPC_EMD_GETMAX", "", false},   {"GENPC_EMD_TWO_LEVEL", "", false},
-    {"GENPC_EMD_DIRECT_P", "", false},   {"GENPC_FPS_MODE", "", false},     {"GENPC_FPS_CLUSTER16", "", false},
-    {"GENPC_FPS_SMEM", "", false},       {"GENPC_FIX_COLS", "", false},     {"GENPC_REGISTER_MODE", "", false},
-    {"GENPC_REGISTER_QT", "", false},    {"GENPC_REGISTER_PERSIST", "", false}, {"GENPC_CHAMFER_TC", "", false},  {"GENPC_TC_LIMIT", "", false},  {"GENPC_SYM_TMA", "", false},
-    {"GENPC_EMD_PRUNE", "", false},      {"GENPC_EMD_PRUNE_MINB", "", false},
-    {"GENPC_EMD_TAIL_SPREAD", "", false}, {"GENPC_CHAMFER_PRUNE", "", false},
-    {"GENPC_EMD_SORT", "", false},       {"GENPC_HOST_PRUNE", "", false},
-    {"GENPC_REGISTER_PRUNE", "", false}, {"GENPC_PRUNE_COOP", "", false},
-    {"GENPC_SORT_CLUSTER", "", false},
+    {"GENPC_SYM_BALANCED", "", false},   {"GENPC_CHAMFER_PRUNE", "", false}, {"GENPC_HOST_PRUNE", "", false},
+    {"GENPC_PRUNE_COOP", "", false},     {"GENPC_SORT_CLUSTER", "", false},  {"GENPC_EMD_GETMAX", "", false},
+    {"GENPC_EMD_PRUNE", "", false},      {"GENPC_EMD_SORT", "", false},      {"GENPC_FPS_MODE", "", false},
+    {"GENPC_FPS_CLUSTER16", "", false},  {"GENPC_FPS_SMEM", "", false},      {"GENPC_REGISTER_MODE", "", false},
+    {"GENPC_REGISTER_PERSIST", "", false}, {"GENPC_REGISTER_PRUNE", "", false},
 };
 constexpr int N_KNOBS = sizeof(g_knobs) / sizeof(g_knobs[0]);
 

@@ -54,13 +54,6 @@ int genpc_chamfer_forward(const float *xyz1, const float *xyz2, float *dist1, fl
                           int *idx2, int B, int N, int M, void *workspace, size_t workspace_bytes,
                           genpc_stream_t stream);
 
-/* Tensor-core filter of the forward (csrc/nn_tc.cuh): for big unit-scale problems the scan runs on tcgen05 (norm expansion as
- * a candidate filter, exact re-evaluation of the winning chunks -- outputs stay bit-identical).  It is selected on the
- * device by a precheck of the coordinate range, no API change.  The two entries below are diagnostics / test probes:
- * genpc_chamfer_tc_stats makes filter launches add {runner-up re-evaluations, whole-tile exact scans, degenerate items,
- * items} to a caller-zeroed device array (NULL: off); genpc_tc_probe dumps e(x,y) of one 128 x 256 tile as computed by the
- * tensor pipe, for the error-margin test. */
-int genpc_chamfer_tc_stats(unsigned *stats4);
 /* Diagnostics of the spatially pruned scan (GENPC_CHAMFER_PRUNE=1, csrc/nn_prune.cuh): launches add {target blocks scanned,
  * query groups that needed the tie pass, query groups, -} to the four device counters; NULL switches it off. */
 int genpc_chamfer_prune_stats(unsigned *stats4);
@@ -73,7 +66,6 @@ int genpc_chamfer_scan_kind(int B, int N, int M);
  * smaller side's clouds take one CTA each, *grid = CTAs launched (whole clusters).  The rule keeps the grid inside one wave of
  * one 1024-thread CTA per SM; GENPC_SORT_CLUSTER overrides it. */
 int genpc_chamfer_sort_layout(int B, int N, int M, int sms, int *mixed, int *grid);
-int genpc_tc_probe(const float *rows128, const float *cols256, float *e_out, genpc_stream_t stream);
 
 /* Host-fed forward: the same result as genpc_chamfer_forward, but the clouds start in HOST memory
  * (h_xyz1 [B][N][3], h_xyz2 [B][M][3]; pinned memory for an asynchronous full-speed copy) and their transfer into the

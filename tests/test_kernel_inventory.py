@@ -3,9 +3,8 @@ still exists.  An entry says why the instantiation is trusted:
 
 - "tests/<file>.py::<test>": a test that runs it and compares its result with the oracle (or, for an internal stage, the
   result of the call it belongs to);
-- "experiment: <knob>": a variant that only a tunable selects; the default dispatch never launches it;
 - "helper": cub and set-up kernels whose output is checked only through the call that uses them;
-- "not compared: <why>": a kernel the default dispatch can reach that no test compares yet (a known gap, stated).
+- "not compared: <why>": a kernel that no test compares yet (a known gap, stated).
 
 A new kernel, template instantiation or threshold therefore has to be placed here.  tools/kernel_coverage.py runs the GPU
 suite under torch.profiler and lists the instantiations that no test launched, to keep the table honest."""
@@ -55,7 +54,6 @@ def library_kernels(lib=LIB):
 
 CG = "tests/test_chamfer_gpu.py::"
 PRU = "tests/test_chamfer_prune.py::"
-TC = "tests/test_chamfer_tc.py::"
 HF = "tests/test_chamfer_host_feed.py::"
 FPS = "tests/test_fps.py::"
 EMD = "tests/test_emd.py::"
@@ -72,28 +70,19 @@ KERNELS = {
     "cub::DeviceRadixSortHistogramKernel": "helper",
     "cub::DeviceRadixSortOnesweepKernel": "helper",
     "cub::DeviceRadixSortSingleTileKernel": "helper",
-    # Chamfer: exhaustive, symmetric, tensor-core, pruned and grid scans, epilogue, gradients
+    # Chamfer: exhaustive, symmetric, pruned and grid scans, epilogue, gradients
     "genpc::nn_scan_kernel<1>": CG + "test_backward_vs_oracle",
     "genpc::nn_scan_kernel<2>": NOT_COMPARED + "sharded partial scan with 512-1023 queries (else only GENPC_CHAMFER_MODE=scan)",
     "genpc::nn_scan_kernel<4>": "tests/test_sharded.py::test_partial_scans_merge_to_the_single_gpu_result",
     "genpc::nn_unpack_kernel": CG + "test_backward_vs_oracle",
     "genpc::nn_sym_kernel<2>": NOT_COMPARED + "symmetric scan with < 1024 rows and >= 4 x SMs work items (not balanced)",
     "genpc::nn_sym_kernel<4>": "tests/test_c1_scan.py::test_c1_on_gpu_vs_oracle_and_golden",
-    "genpc::nn_sym_kernel<6>": "experiment: GENPC_SYM_QT=6",
-    "genpc::nn_sym_kernel<8>": "experiment: GENPC_SYM_QT=8",
     "genpc::nn_sym_balanced_kernel<2>": CG + "test_forward_bit_exact_vs_oracle",
     "genpc::nn_sym_balanced_kernel<4>": CG + "test_forward_bit_exact_vs_oracle",
-    "genpc::nn_sym_persistent_kernel<2>": "experiment: GENPC_SYM_PERSIST=1",
-    "genpc::nn_sym_persistent_kernel<4>": "experiment: GENPC_SYM_PERSIST=1",
-    "genpc::nn_sym_tma_kernel<4>": "experiment: GENPC_SYM_TMA=1",
     "genpc::nn_sym_gated_kernel<2>": NOT_COMPARED + "host-fed scan with fewer than 1024 rows",
     "genpc::nn_sym_gated_kernel<4>": HF + "test_host_fed_forward_bit_exact",
     "genpc::nn_sym_epilogue_kernel<false>": CG + "test_nan_and_inf_points_stay_in_range",
     "genpc::nn_sym_epilogue_kernel<true>": "tests/test_c1_scan.py::test_c1_on_gpu_vs_oracle_and_golden",
-    "genpc::nn_tc_kernel<false>": TC + "test_c2_full_batch_through_the_filter",
-    "genpc::nn_tc_kernel<true>": NOT_COMPARED + "host-fed scan through the tensor-core filter",
-    "genpc::nn_tc_precheck_kernel": TC + "test_c2_full_batch_through_the_filter",
-    "genpc::nn_tc_probe_kernel": TC + "test_error_assumption_of_the_filter_margin",
     "genpc::nn_bin_sort_kernel<1>": PRU + "test_exact_ties_and_degenerate_geometry",
     "genpc::nn_bin_sort_kernel<2>": PRU + "test_sort_cluster_layouts_bit_exact",
     "genpc::nn_bin_sort_kernel<3>": PRU + "test_sort_cluster_layouts_bit_exact",
@@ -137,9 +126,6 @@ KERNELS = {
     "genpc::emd_auction_kernel<4,3>": EMD + "test_emd_gpu_bit_exact_vs_oracle",
     "genpc::emd_auction_kernel<8,3>": EMD + "test_emd_gpu_bit_exact_vs_oracle",
     "genpc::emd_auction_kernel<16,3>": EMD + "test_emd_pruned_bid_equals_exhaustive_bid_on_adversarial_inputs",
-    "genpc::emd_auction_kernel<4,4>": "experiment: GENPC_EMD_PRUNE_MINB=4",
-    "genpc::emd_auction_kernel<8,4>": "experiment: GENPC_EMD_PRUNE_MINB=4",
-    "genpc::emd_auction_kernel<16,4>": "experiment: GENPC_EMD_PRUNE_MINB=4",
     "genpc::emd_sort_kernel": EMD + "test_emd_pruned_bid_equals_exhaustive_bid_on_adversarial_inputs",
     "genpc::emd_grad_kernel": DSP + "test_emd_batch_512_more_clouds_than_ctas",
     # FPS
@@ -221,7 +207,7 @@ def test_every_kernel_has_an_entry_and_every_entry_a_kernel(kernels):
 
 def test_entries_name_existing_tests_or_a_reason():
     for k, v in KERNELS.items():
-        if v == "helper" or v.startswith(("experiment: ", NOT_COMPARED)):
+        if v == "helper" or v.startswith(NOT_COMPARED):
             continue
         path, _, name = v.partition("::")
         assert path.startswith("tests/") and name, (k, v)

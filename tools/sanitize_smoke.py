@@ -39,8 +39,7 @@ knn_mean_distance(torch.rand(3001, 3, generator=g).to(dev), 20, True); knn_mean_
 sharded_chamfer_forward(torch.rand(1, 5001, 3, generator=g).to(dev), torch.rand(1, 3003, 3, generator=g).to(dev))
 from genpc_b200.reg_xyz import icp_point_to_point
 icp_point_to_point(torch.rand(5, 333, 3, generator=g).to(dev), torch.rand(1, 777, 3, generator=g).to(dev), 0.3, max_iteration=3)
-# ---- r02 kernels: mesh sampler, persistent small registration (one launch, several iterations), tensor-core filter (forced),
-# TMA-staged scan, NaN points, graphed loss step
+# ---- r02 kernels: mesh sampler, persistent small registration (one launch, several iterations), NaN points, graphed loss step
 from genpc_b200 import _lib
 from genpc_b200.synthetic import superquadric_mesh
 from genpc_b200.utils.glb import sample_mesh
@@ -49,11 +48,6 @@ v, f, col = superquadric_mesh(1, 12, 20)
 sample_mesh(torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev), 3001, 5, torch.from_numpy(col).to(dev), return_face=True)
 rb = RegistrationBatch(torch.rand(1, 1300, 3, generator=g).to(dev) - 0.5, torch.rand(1, 900, 3, generator=g).to(dev) - 0.5, n_starts=3)
 rb.run(5)
-with _lib.tunable(GENPC_CHAMFER_TC="1"):
-    for (B, N, M) in [(2, 700, 1300), (1, 3000, 999), (1, 513, 33)]:
-        chamfer_3DDist()(torch.rand(B, N, 3, generator=g).to(dev) - 0.5, torch.rand(B, M, 3, generator=g).to(dev) - 0.5)
-with _lib.tunable(GENPC_SYM_TMA="1"):
-    chamfer_3DDist()(torch.rand(40, 4096, 3, generator=g).to(dev), torch.rand(40, 2048, 3, generator=g).to(dev))
 a = torch.rand(2, 700, 3, generator=g); a[0, 3] = float("nan"); a[1, 5] = 3e38
 d1, d2, i1, i2 = chamfer_3DDist()(a.to(dev).requires_grad_(True), torch.rand(2, 1300, 3, generator=g).to(dev).requires_grad_(True))
 (d1[:, 10:].mean() + d2.mean()).backward()

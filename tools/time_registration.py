@@ -17,5 +17,5 @@ e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=Tr
 e0.record(); rb.run(iters); e1.record(); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1)
 L = rb.losses()
-print(json.dumps({"fix_cols": os.environ.get("GENPC_FIX_COLS", "default"), "ms_per_iter": ms / iters,
+print(json.dumps({"ms_per_iter": ms / iters,
                   "scan_iters_per_s": S * iters / (ms * 1e-3), "loss_last_sum": float(L[:, rb.t - 1].double().sum())}))
