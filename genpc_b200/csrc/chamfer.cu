@@ -269,8 +269,10 @@ constexpr int GR_PROBE_GROUPS = 128;   // sampled query groups per direction and
 static size_t prune_extra_bytes(int B, int N, int M) {
     if (B <= 8 && grid_eligible(N, M)) return grid_extra_bytes(B, N, M);
     if (!prune_eligible(B, N, M)) return 0;   // (the knob is read when the workspace is sized)
+    // sorted records (16 B per point), block boxes, chunk boxes (2 x 16 B per 8 points), bounding boxes
     return 256 + (size_t)B * ((size_t)pr_npad(N) + pr_npad(M)) * sizeof(float4) +
-           (size_t)B * 2 * ((size_t)pr_nblk(N) + pr_nblk(M)) * sizeof(float4) + (size_t)B * 2 * 8 * sizeof(float);
+           (size_t)B * 2 * ((size_t)pr_nblk(N) + pr_nblk(M)) * sizeof(float4) +
+           (size_t)B * 2 * ((size_t)pr_npad(N) / 8 + pr_npad(M) / 8) * sizeof(float4) + (size_t)B * 2 * 8 * sizeof(float);
 }
 static unsigned *g_prune_stats = nullptr;   // diagnostics (genpc_chamfer_prune_stats), nullptr in production
 
@@ -388,21 +390,26 @@ static int launch_prune_subbatch(const float *rows, const float *cols, int nr, i
     float4 *sorted1 = sorted0 + (size_t)B * pr_npad(nr);
     float4 *boxes0 = sorted1 + (size_t)B * pr_npad(nc);
     float4 *boxes1 = boxes0 + (size_t)B * 2 * pr_nblk(nr);
-    float *bbx = reinterpret_cast<float *>(boxes1 + (size_t)B * 2 * pr_nblk(nc));
+    float4 *cboxes0 = boxes1 + (size_t)B * 2 * pr_nblk(nc);
+    float4 *cboxes1 = cboxes0 + (size_t)B * 2 * (pr_npad(nr) / 8);
+    float *bbx = reinterpret_cast<float *>(cboxes1 + (size_t)B * 2 * (pr_npad(nc) / 8));
     PruneSortParams sp = {};
     sp.xyz[0] = rows + (size_t)b0 * nr * 3, sp.xyz[1] = cols + (size_t)b0 * nc * 3, sp.n[0] = nr, sp.n[1] = nc, sp.B = nb;
     sp.limit = 1e15f, sp.ctl = chunk_ctl != nullptr ? chunk_ctl : ctl, sp.hilbert = 1, sp.accumulate = accumulate ? 1 : 0;
     sp.flag = chunk_ctl != nullptr ? ctl + 1 : nullptr;
     sp.sorted[0] = sorted0 + (size_t)b0 * pr_npad(nr), sp.sorted[1] = sorted1 + (size_t)b0 * pr_npad(nc);
     sp.boxes[0] = boxes0 + (size_t)b0 * 2 * pr_nblk(nr), sp.boxes[1] = boxes1 + (size_t)b0 * 2 * pr_nblk(nc);
+    sp.cboxes[0] = cboxes0 + (size_t)b0 * 2 * (pr_npad(nr) / 8), sp.cboxes[1] = cboxes1 + (size_t)b0 * 2 * (pr_npad(nc) / 8);
     sp.bbx = bbx + (size_t)b0 * 16;
     launch_bin_sort(sp, nb, stream);
     GENPC_CHECK_LAUNCH();
     PruneParams q = {};
     q.B = nb, q.select = ctl + 1, q.stats = g_prune_stats;
-    q.q = sp.sorted[0], q.t = sp.sorted[1], q.tbox = sp.boxes[1], q.out = prow + (size_t)b0 * nr, q.nq = nr, q.nt = nc;
+    q.q = sp.sorted[0], q.t = sp.sorted[1], q.tbox = sp.boxes[1], q.tcbox = sp.cboxes[1], q.out = prow + (size_t)b0 * nr, q.nq = nr,
+    q.nt = nc;
     PruneParams q2 = q;
-    q2.q = sp.sorted[1], q2.t = sp.sorted[0], q2.tbox = sp.boxes[0], q2.out = pcol + (size_t)b0 * nc, q2.nq = nc, q2.nt = nr;
+    q2.q = sp.sorted[1], q2.t = sp.sorted[0], q2.tbox = sp.boxes[0], q2.tcbox = sp.cboxes[0], q2.out = pcol + (size_t)b0 * nc, q2.nq = nc,
+    q2.nt = nr;
     launch_prune(q, q2, stream);
     GENPC_CHECK_LAUNCH();
     return GENPC_OK;
@@ -733,7 +740,8 @@ extern "C" int genpc_chamfer_scan_kind(int B, int N, int M) {
     return prune_eligible(B, nr, nc) ? 1 : 0;
 }
 
-// diagnostics of the pruned scan: stats4 = device pointer to 4 counters (blocks scanned, groups that took the tie pass, groups, -)
+// diagnostics of the pruned scan: stats4 = device pointer to 4 counters (blocks walked, groups that took the tie pass, groups,
+// 8-target chunks evaluated; nn_grid.cuh: superblocks opened)
 extern "C" int genpc_chamfer_prune_stats(unsigned *stats4) {
     g_prune_stats = stats4;
     return GENPC_OK;

@@ -7,13 +7,14 @@
 //   1. nn_bin_sort_kernel<CS> orders every cloud along a Hilbert curve (counting sort over 8^m grid cells in shared memory;
 //      one CTA per cloud, or a thread-block cluster of CS CTAs that read each other's histograms through distributed shared
 //      memory when one CTA per cloud would leave most SMs idle) into (x, y, z, original index) records and stores the
-//      bounding box of every PR_BLOCK consecutive ones;
+//      bounding box of every PR_BLOCK consecutive ones, and of every 8 (the walk's chunks);
 //   2. nn_prune_kernel: one warp owns PR_GROUP consecutive sorted queries (one per lane -- neighbours in space).  It
 //      computes the squared distance between the group's box and every target block's box, visits the blocks nearest
 //      first (REDUX picks them) and stops at the first block farther than the group's worst running minimum: no target
-//      in it, or in any later block, can improve (or tie) any lane.  A block is fetched with one coalesced read into the
-//      warp's shared-memory slice (SoA) and walked there with the packed FP32 distance of the exhaustive kernels: the
-//      same bits.  nn_prune_coop_kernel is the form for a direction with few query groups and many target blocks: a CTA
+//      in it, or in any later block, can improve (or tie) any lane.  A block is fetched only when some lane's own point is
+//      within its box, with one coalesced read into the warp's shared-memory slice (SoA), and walked there chunk by chunk
+//      with the packed FP32 distance of the exhaustive kernels (the same bits), skipping the chunks whose box no lane is
+//      within (pr_visit_block).  nn_prune_coop_kernel is the form for a direction with few query groups and many target blocks: a CTA
 //      per group, the blocks partitioned over its eight warps, running minima shared through shared memory.
 // Exactness: the minimum of a set does not depend on the visiting order; the reported index is the LOWEST original index
 // among the targets at the minimum, as in the exhaustive kernels (the winner's 8-target chunk is re-evaluated; a lane
@@ -83,6 +84,7 @@ struct PruneSortParams {
     const float *xyz[2];   // [B][n][3]
     float4 *sorted[2];     // [B][npad]   (x, y, z, original index); NaN records pad the last block
     float4 *boxes[2];      // [B][2][nblk] lower corners, then upper corners
+    float4 *cboxes[2];     // optional [B][2][npad / 8]: the same for every 8 consecutive records (the scan's chunks; nullptr: none)
     int n[2];
     int B;
     float limit;
@@ -342,24 +344,41 @@ static __global__ void __launch_bounds__(PR_SORT_THREADS) nn_bin_sort_kernel(con
     } else {
         __syncthreads();   // the CTA's own global writes are visible to it after the barrier
     }
-    // ---- block boxes ----
+    // ---- block boxes, and the boxes of the 8-record chunks (the 8-lane stage of the same reduction) ----
+    static_assert(PR_BLOCK == 64, "a block is two 32-record rows of the warp");
+    float4 *cbx = p.cboxes[side] != nullptr ? p.cboxes[side] + (size_t)b * 2 * (npad / 8) : nullptr;
     for (int blk = cr * (PR_SORT_THREADS / 32) + warp; blk < nblk; blk += ceff * (PR_SORT_THREADS / 32)) {
-        float l[3] = {inf, inf, inf}, h[3] = {-inf, -inf, -inf};
+        float l[PR_BLOCK / 32][3], h[PR_BLOCK / 32][3];
 #pragma unroll
         for (int e = 0; e < PR_BLOCK / 32; ++e) {
             const float4 t = CS > 1 ? __ldcg(dst + blk * PR_BLOCK + e * 32 + lane) : dst[blk * PR_BLOCK + e * 32 + lane];
-            l[0] = fminf(l[0], t.x), h[0] = fmaxf(h[0], t.x);   // NaN padding is ignored
-            l[1] = fminf(l[1], t.y), h[1] = fmaxf(h[1], t.y);
-            l[2] = fminf(l[2], t.z), h[2] = fmaxf(h[2], t.z);
+            // NaN padding is ignored: an all-padding chunk keeps (+inf, -inf), a box no point is near
+            l[e][0] = fminf(inf, t.x), h[e][0] = fmaxf(-inf, t.x);
+            l[e][1] = fminf(inf, t.y), h[e][1] = fmaxf(-inf, t.y);
+            l[e][2] = fminf(inf, t.z), h[e][2] = fmaxf(-inf, t.z);
+#pragma unroll
+            for (int c = 0; c < 3; ++c)
+#pragma unroll
+                for (int o = 4; o > 0; o >>= 1) {
+                    l[e][c] = fminf(l[e][c], __shfl_xor_sync(0xffffffffu, l[e][c], o));
+                    h[e][c] = fmaxf(h[e][c], __shfl_xor_sync(0xffffffffu, h[e][c], o));
+                }
+            if (cbx != nullptr && (lane & 7) == 0) {   // records e * 32 + lane .. + 7 of the block: its chunk e * 4 + lane / 8
+                const int k = blk * (PR_BLOCK / 8) + e * 4 + (lane >> 3);
+                cbx[k] = make_float4(l[e][0], l[e][1], l[e][2], 0.f), cbx[npad / 8 + k] = make_float4(h[e][0], h[e][1], h[e][2], 0.f);
+            }
         }
 #pragma unroll
-        for (int c = 0; c < 3; ++c)
+        for (int c = 0; c < 3; ++c) {
+            l[0][c] = fminf(l[0][c], l[1][c]), h[0][c] = fmaxf(h[0][c], h[1][c]);
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                l[c] = fminf(l[c], __shfl_xor_sync(0xffffffffu, l[c], o));
-                h[c] = fmaxf(h[c], __shfl_xor_sync(0xffffffffu, h[c], o));
+            for (int o = 16; o > 4; o >>= 1) {
+                l[0][c] = fminf(l[0][c], __shfl_xor_sync(0xffffffffu, l[0][c], o));
+                h[0][c] = fmaxf(h[0][c], __shfl_xor_sync(0xffffffffu, h[0][c], o));
             }
-        if (lane == 0) bx[blk] = make_float4(l[0], l[1], l[2], 0.f), bx[nblk + blk] = make_float4(h[0], h[1], h[2], 0.f);
+        }
+        if (lane == 0)
+            bx[blk] = make_float4(l[0][0], l[0][1], l[0][2], 0.f), bx[nblk + blk] = make_float4(h[0][0], h[0][1], h[0][2], 0.f);
     }
     // ---- selection flag: the last CTA publishes "any cloud out of range, or a pair of clouds that does not overlap" (pruning
     // needs neighbours to be near: when the two boxes of a pair are further apart than a quarter of the smaller one's diagonal,
@@ -419,10 +438,11 @@ static void launch_bin_sort_cs(PruneSortParams sp, int ctas, cudaStream_t stream
 struct PruneParams {
     const float4 *q, *t;      // sorted queries [B][npad_q], sorted targets [B][npad_t]
     const float4 *tbox;       // [B][2][nblk_t]
+    const float4 *tcbox;      // [B][2][npad_t / 8]: boxes of the targets' 8-record chunks
     unsigned long long *out;  // [B][nq] packed (dist, original target index), addressed by the query's original index
     int nq, nt, B;
     const int *select;        // run only when *select == 0
-    unsigned *stats;          // optional [4]: blocks scanned, tie passes, groups, -
+    unsigned *stats;          // optional [4]: blocks fetched and walked, tie passes, groups, 8-target chunks evaluated
     int qdiv, tdiv;           // batch entry b reads queries / targets of cloud b / qdiv, b / tdiv (0 or 1: its own; registration: the
                               // starts of one scan share the fixed cloud's sorted copy)
 };
@@ -432,6 +452,73 @@ __device__ __forceinline__ int pr_f2ord(float f) {
     return i ^ ((i >> 31) & 0x7fffffff);
 }
 __device__ __forceinline__ float pr_ord2f(int i) { return __int_as_float(i ^ ((i >> 31) & 0x7fffffff)); }
+
+// Squared distance between the box [l, h] (a query group's box, or one query: l = h) and a target box [lo, hi], scaled down
+// (see the header).  Every step rounds monotonically, so it never exceeds the rounded distance (sqdist_ref) of any point of the
+// first box to any point of the second.
+__device__ __forceinline__ float pr_box_d2(float lx, float ly, float lz, float hx, float hy, float hz, float4 lo, float4 hi) {
+    const float dx = fmaxf(fmaxf(lo.x - hx, lx - hi.x), 0.f);
+    const float dy = fmaxf(fmaxf(lo.y - hy, ly - hi.y), 0.f);
+    const float dz = fmaxf(fmaxf(lo.z - hz, lz - hi.z), 0.f);
+    return __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.99999f);
+}
+
+// One visit of target block `blk` by a warp's 32 queries (one per lane; nx/ny/nz = the negated query in both halves; CBL = the
+// lane's entry of chunk box 0 for lanes 0-15).  A lane's bound is min(best, cap): its running minimum, or less when another
+// warp has already found a nearer target for the same query (cap; +inf for a warp on its own).
+//   1. each lane's point-to-block-box distance against its bound: when no lane is within it, nothing is fetched (-> false);
+//   2. the block's 64 records (SoA) and its eight chunk boxes into the warp's staging slice: one coalesced 1 KB + 256 B read;
+//   3. each 8-target chunk is evaluated only when some lane's point-to-chunk-box distance is within that lane's CURRENT bound.
+// Exactness: a chunk (or block) is skipped only when, for every lane, the box distance is strictly greater than the bound.  The
+// box distance is never above the distance the lane would compute to any target inside (pr_box_d2), and the bound is never
+// below the lane's current or final minimum, so a skipped chunk could neither lower `best` nor equal it: best, bchunk and tie are
+// those of walking every chunk, and a chunk holding a lane's final minimum is always evaluated.  Lanes without a query (padding)
+// ask for nothing.
+template <int UNR>
+__device__ __forceinline__ bool pr_visit_block(float (*st)[PR_BLOCK], float4 *sbox, const float4 *T, const float4 *BL, const float4 *BH,
+                                               const float4 *CBL, int blk, float2 nx, float2 ny, float2 nz, bool valid,
+                                               float cap, float &best, int &bchunk, bool &tie, unsigned &chunks) {
+    const int lane = threadIdx.x & 31;
+    const float qx = -nx.x, qy = -ny.x, qz = -nz.x;
+    const float inf = __int_as_float(0x7f800000);
+    // (`&`, not `&&`: the test is computed by every lane, no branch around it)
+    if (!__any_sync(0xffffffffu, valid & (pr_box_d2(qx, qy, qz, qx, qy, qz, __ldg(BL + blk), __ldg(BH + blk)) <= fminf(best, cap))))
+        return false;
+    {   // one coalesced read of the records, lanes 0-15 the chunk boxes (lower corners, then upper), walked in shared memory
+        const float4 *tg = T + blk * PR_BLOCK;
+        const float4 u0 = __ldg(tg + lane), u1 = __ldg(tg + 32 + lane);
+        const float4 cb = lane < 16 ? __ldg(CBL + blk * (PR_BLOCK / 8)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncwarp();
+        st[0][lane] = u0.x, st[1][lane] = u0.y, st[2][lane] = u0.z;
+        st[0][32 + lane] = u1.x, st[1][32 + lane] = u1.y, st[2][32 + lane] = u1.z;
+        if (lane < 16) sbox[lane] = cb;
+        __syncwarp();
+    }
+    // SoA: one LDS.128 per coordinate brings four targets as two register pairs the packed FP32 instructions take as they
+    // are (the AoS form spent 6 of its 15 instructions per target pair moving registers into pairs)
+    const float4 *sx4 = reinterpret_cast<const float4 *>(st[0]), *sy4 = reinterpret_cast<const float4 *>(st[1]),
+                 *sz4 = reinterpret_cast<const float4 *>(st[2]);
+#pragma unroll UNR
+    for (int c = 0; c < PR_BLOCK / 8; ++c) {
+        if (!__any_sync(0xffffffffu, valid & (pr_box_d2(qx, qy, qz, qx, qy, qz, sbox[c], sbox[8 + c]) <= fminf(best, cap)))) continue;
+        ++chunks;
+        float cm = inf;
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const float4 X = sx4[c * 2 + i], Y = sy4[c * 2 + i], Z = sz4[c * 2 + i];
+            const float2 a2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.x, X.y), make_float2(Y.x, Y.y), make_float2(Z.x, Z.y));
+            const float2 b2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.z, X.w), make_float2(Y.z, Y.w), make_float2(Z.z, Z.w));
+            cm = fmin3(cm, a2.x, a2.y);
+            cm = fmin3(cm, b2.x, b2.y);
+        }
+        if (cm < best) {
+            best = cm, bchunk = blk * (PR_BLOCK / 8) + c, tie = false;
+        } else if (cm == best && cm < inf) {
+            tie = true;
+        }
+    }
+    return true;
+}
 
 // Both directions of a cloud pair in ONE launch: the first ctas0 CTAs take direction d[0] (put the direction with the longer
 // per-group chains there: it is scheduled first), the rest d[1].
@@ -445,6 +532,7 @@ struct PrunePair {
 template <int BOXR>
 __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp) {
     __shared__ __align__(16) float stage[PR_THREADS / 32][3][PR_BLOCK];   // the block being walked, SoA: x[64] y[64] z[64]
+    __shared__ float4 sbox[PR_THREADS / 32][16];                           // ... and its chunk boxes: lower corners, upper corners
     const int dir = (int)blockIdx.x >= pp.ctas0 ? 1 : 0;
     const PruneParams &p = pp.d[dir];
     if (p.select != nullptr && *p.select != 0) return;
@@ -459,6 +547,8 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
     const int bt = p.tdiv > 1 ? b / p.tdiv : b, bq = p.qdiv > 1 ? b / p.qdiv : b;
     const float4 *T = p.t + (size_t)bt * pr_npad(p.nt);
     const float4 *BL = p.tbox + (size_t)bt * 2 * nblk, *BH = BL + nblk;
+    const int nchunk = pr_npad(p.nt) / 8;   // lanes 0-7 / 8-15 stage the lower / upper corners of a block's eight chunk boxes
+    const float4 *CBL = p.tcbox + (size_t)bt * 2 * nchunk + (lane >> 3) * nchunk + (lane & 7);
     const float inf = __int_as_float(0x7f800000);
     const int qi = g * PR_GROUP + lane;
     const bool valid = qi < p.nq;
@@ -481,20 +571,14 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
     for (int r = 0; r < BOXR; ++r) {
         const int blk = r * 32 + lane;
         bd[r] = inf;
-        if (blk < nblk) {
-            const float4 lo = __ldg(BL + blk), hi = __ldg(BH + blk);
-            const float dx = fmaxf(fmaxf(lo.x - ghi[0], glo[0] - hi.x), 0.f);
-            const float dy = fmaxf(fmaxf(lo.y - ghi[1], glo[1] - hi.y), 0.f);
-            const float dz = fmaxf(fmaxf(lo.z - ghi[2], glo[2] - hi.z), 0.f);
-            bd[r] = __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.99999f);
-        }
+        if (blk < nblk) bd[r] = pr_box_d2(glo[0], glo[1], glo[2], ghi[0], ghi[1], ghi[2], __ldg(BL + blk), __ldg(BH + blk));
     }
     const float2 nx = make_float2(-q.x, -q.x), ny = make_float2(-q.y, -q.y), nz = make_float2(-q.z, -q.z);
     float best = inf;
     int bchunk = 0;
     bool tie = false;
     float thr = inf;   // the largest running minimum of the group's lanes
-    unsigned scanned = 0;
+    unsigned scanned = 0, chunks = 0;
     for (;;) {
         // nearest remaining block: (distance bits without the low 9, block id); the truncation errs on the near side
         unsigned key = 0xffffffffu;
@@ -506,38 +590,11 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
 #pragma unroll
         for (int r = 0; r < BOXR; ++r)
             if (r * 32 + lane == blk) bd[r] = inf;
-        {   // one coalesced 1 KB read per block, walked in shared memory (see nn_prune2_kernel)
-            const float4 *tg = T + blk * PR_BLOCK;
-            const float4 u0 = __ldg(tg + lane), u1 = __ldg(tg + 32 + lane);
-            __syncwarp();
-            stage[wid][0][lane] = u0.x, stage[wid][1][lane] = u0.y, stage[wid][2][lane] = u0.z;
-            stage[wid][0][32 + lane] = u1.x, stage[wid][1][32 + lane] = u1.y, stage[wid][2][32 + lane] = u1.z;
-            __syncwarp();
-        }
-        // SoA: one LDS.128 per coordinate brings four targets as two register pairs the packed FP32 instructions take as they
-        // are (the AoS form spent 6 of its 15 instructions per target pair moving registers into pairs)
-        const float4 *sx4 = reinterpret_cast<const float4 *>(stage[wid][0]), *sy4 = reinterpret_cast<const float4 *>(stage[wid][1]),
-                     *sz4 = reinterpret_cast<const float4 *>(stage[wid][2]);
         // 256 target blocks and more (C3: 16384^2 inside the registration loop) keep the 2x form: 4x cost C3 9 % on the same box
         // (26 100 vs 28 600 scan-iters/s) while the 32- and 128-block instantiations gained 1-4 % (profiles/r02w_unroll_sweep.txt)
         constexpr int UNR = BOXR >= 8 ? 2 : PR_UNROLL;
-#pragma unroll UNR
-        for (int c = 0; c < PR_BLOCK / 8; ++c) {
-            float cm = inf;
-#pragma unroll
-            for (int i = 0; i < 2; ++i) {
-                const float4 X = sx4[c * 2 + i], Y = sy4[c * 2 + i], Z = sz4[c * 2 + i];
-                const float2 a2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.x, X.y), make_float2(Y.x, Y.y), make_float2(Z.x, Z.y));
-                const float2 b2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.z, X.w), make_float2(Y.z, Y.w), make_float2(Z.z, Z.w));
-                cm = fmin3(cm, a2.x, a2.y);
-                cm = fmin3(cm, b2.x, b2.y);
-            }
-            if (cm < best) {
-                best = cm, bchunk = blk * (PR_BLOCK / 8) + c, tie = false;
-            } else if (cm == best && cm < inf) {
-                tie = true;
-            }
-        }
+        if (!pr_visit_block<UNR>(stage[wid], sbox[wid], T, BL, BH, CBL, blk, nx, ny, nz, valid, inf, best, bchunk, tie, chunks))
+            continue;   // no lane's own box test passed: every minimum (and so thr) is unchanged
         ++scanned;
         thr = pr_ord2f(__reduce_max_sync(0xffffffffu, valid ? pr_f2ord(best) : (int)0x80000000));
     }
@@ -556,11 +613,7 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
     const unsigned ties = __ballot_sync(0xffffffffu, tie && valid);
     if (ties != 0u) {
         for (int blk = 0; blk < nblk; ++blk) {
-            const float4 lo = __ldg(BL + blk), hi = __ldg(BH + blk);
-            const float dx = fmaxf(fmaxf(lo.x - ghi[0], glo[0] - hi.x), 0.f);
-            const float dy = fmaxf(fmaxf(lo.y - ghi[1], glo[1] - hi.y), 0.f);
-            const float dz = fmaxf(fmaxf(lo.z - ghi[2], glo[2] - hi.z), 0.f);
-            const float s = __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.99999f);
+            const float s = pr_box_d2(glo[0], glo[1], glo[2], ghi[0], ghi[1], ghi[2], __ldg(BL + blk), __ldg(BH + blk));
             if (!(s <= thr)) continue;   // warp-uniform
             const float4 *tb = T + blk * PR_BLOCK;
             for (int i = 0; i < PR_BLOCK; ++i) {
@@ -575,6 +628,7 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
         atomicAdd(p.stats + 0, scanned);
         if (ties != 0u) atomicAdd(p.stats + 1, 1u);
         atomicAdd(p.stats + 2, 1u);
+        atomicAdd(p.stats + 3, chunks);
     }
 }
 
@@ -588,7 +642,8 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
 template <int BOXR>
 __global__ void __launch_bounds__(PR_THREADS) nn_prune_coop_kernel(const PruneParams p) {
     __shared__ __align__(16) float stage[PR_THREADS / 32][3][PR_BLOCK];
-    __shared__ unsigned s_best[PR_GROUP];                       // running minimum per query over all warps (float bits, >= 0)
+    __shared__ float4 sbox[PR_THREADS / 32][16];
+    __shared__ unsigned s_best[PR_GROUP];                      // running minimum per query over all warps (float bits, >= 0)
     __shared__ float m_best[PR_THREADS / 32][PR_GROUP];
     __shared__ int m_chunk[PR_THREADS / 32][PR_GROUP], m_tie[PR_THREADS / 32][PR_GROUP];
     if (p.select != nullptr && *p.select != 0) return;
@@ -602,6 +657,8 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_coop_kernel(const PrunePa
     const int bt = p.tdiv > 1 ? b / p.tdiv : b, bq = p.qdiv > 1 ? b / p.qdiv : b;
     const float4 *T = p.t + (size_t)bt * pr_npad(p.nt);
     const float4 *BL = p.tbox + (size_t)bt * 2 * nblk, *BH = BL + nblk;
+    const int nchunk = pr_npad(p.nt) / 8;   // lanes 0-7 / 8-15 stage the lower / upper corners of a block's eight chunk boxes
+    const float4 *CBL = p.tcbox + (size_t)bt * 2 * nchunk + (lane >> 3) * nchunk + (lane & 7);
     const float inf = __int_as_float(0x7f800000);
     const int qi = g * PR_GROUP + lane;
     const bool valid = qi < p.nq;
@@ -628,69 +685,36 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_coop_kernel(const PrunePa
     for (int r = 0; r < CBOXR; ++r) {
         const int blk = wid + WARPS * (r * 32 + lane);
         bd[r] = inf;
-        if (blk < nblk) {
-            const float4 lo = __ldg(BL + blk), hi = __ldg(BH + blk);
-            const float dx = fmaxf(fmaxf(lo.x - ghi[0], glo[0] - hi.x), 0.f);
-            const float dy = fmaxf(fmaxf(lo.y - ghi[1], glo[1] - hi.y), 0.f);
-            const float dz = fmaxf(fmaxf(lo.z - ghi[2], glo[2] - hi.z), 0.f);
-            bd[r] = __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.99999f);
-        }
+        if (blk < nblk) bd[r] = pr_box_d2(glo[0], glo[1], glo[2], ghi[0], ghi[1], ghi[2], __ldg(BL + blk), __ldg(BH + blk));
     }
     const float2 nx = make_float2(-q.x, -q.x), ny = make_float2(-q.y, -q.y), nz = make_float2(-q.z, -q.z);
     float best = inf;
     int bchunk = 0;
     bool tie = false;
     float thr = inf;   // the largest running minimum of the group's lanes
-    unsigned scanned = 0;
+    unsigned scanned = 0, chunks = 0;
     for (;;) {
         unsigned key = 0xffffffffu;   // (distance bits without the low 9, slot = r * 32 + lane of the owned block)
 #pragma unroll
         for (int r = 0; r < CBOXR; ++r) key = min(key, (__float_as_uint(bd[r]) & 0xfffffe00u) | (unsigned)(r * 32 + lane));
         key = __reduce_min_sync(0xffffffffu, key);
-        // the bound uses what ANY warp has found so far for each query
-        thr = pr_ord2f(__reduce_max_sync(0xffffffffu, valid ? pr_f2ord(fminf(best, __uint_as_float(*(volatile unsigned *)&s_best[lane])))
-                                                            : (int)0x80000000));
+        // the bound uses what ANY warp has found so far for each query (a real distance to that query: never below its minimum)
+        const float cap = __uint_as_float(*(volatile unsigned *)&s_best[lane]);
+        thr = pr_ord2f(__reduce_max_sync(0xffffffffu, valid ? pr_f2ord(fminf(best, cap)) : (int)0x80000000));
         if (key >= 0x7f800000u || !(__uint_as_float(key & 0xfffffe00u) <= thr)) break;
         const int slot = (int)(key & 0x1ffu);
 #pragma unroll
         for (int r = 0; r < CBOXR; ++r)
             if (r * 32 + lane == slot) bd[r] = inf;
-        const int blk = wid + WARPS * slot;
-        {   // one coalesced 1 KB read per block, walked in shared memory (see nn_prune2_kernel)
-            const float4 *tg = T + blk * PR_BLOCK;
-            const float4 u0 = __ldg(tg + lane), u1 = __ldg(tg + 32 + lane);
-            __syncwarp();
-            stage[wid][0][lane] = u0.x, stage[wid][1][lane] = u0.y, stage[wid][2][lane] = u0.z;
-            stage[wid][0][32 + lane] = u1.x, stage[wid][1][32 + lane] = u1.y, stage[wid][2][32 + lane] = u1.z;
-            __syncwarp();
-        }
-        // SoA: one LDS.128 per coordinate brings four targets as two register pairs the packed FP32 instructions take as they
-        // are (the AoS form spent 6 of its 15 instructions per target pair moving registers into pairs)
-        const float4 *sx4 = reinterpret_cast<const float4 *>(stage[wid][0]), *sy4 = reinterpret_cast<const float4 *>(stage[wid][1]),
-                     *sz4 = reinterpret_cast<const float4 *>(stage[wid][2]);
-#pragma unroll PR_UNROLL
-        for (int c = 0; c < PR_BLOCK / 8; ++c) {
-            float cm = inf;
-#pragma unroll
-            for (int i = 0; i < 2; ++i) {
-                const float4 X = sx4[c * 2 + i], Y = sy4[c * 2 + i], Z = sz4[c * 2 + i];
-                const float2 a2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.x, X.y), make_float2(Y.x, Y.y), make_float2(Z.x, Z.y));
-                const float2 b2 = sqdist_ref_x2(nx, ny, nz, make_float2(X.z, X.w), make_float2(Y.z, Y.w), make_float2(Z.z, Z.w));
-                cm = fmin3(cm, a2.x, a2.y);
-                cm = fmin3(cm, b2.x, b2.y);
-            }
-            if (cm < best) {
-                best = cm, bchunk = blk * (PR_BLOCK / 8) + c, tie = false;
-            } else if (cm == best && cm < inf) {
-                tie = true;
-            }
-        }
+        if (!pr_visit_block<PR_UNROLL>(stage[wid], sbox[wid], T, BL, BH, CBL, wid + WARPS * slot, nx, ny, nz, valid, cap, best, bchunk,
+                                       tie, chunks))
+            continue;
         ++scanned;
         if (valid) atomicMin(&s_best[lane], __float_as_uint(best));
     }
     // ---- merge the eight warps' results (warp 0 finishes the group) ----
     m_best[wid][lane] = best, m_chunk[wid][lane] = bchunk, m_tie[wid][lane] = tie ? 1 : 0;
-    if (p.stats != nullptr && lane == 0 && wid != 0) atomicAdd(p.stats + 0, scanned);
+    if (p.stats != nullptr && lane == 0 && wid != 0) atomicAdd(p.stats + 0, scanned), atomicAdd(p.stats + 3, chunks);
     __syncthreads();
     if (wid != 0) return;
 #pragma unroll
@@ -720,11 +744,7 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_coop_kernel(const PrunePa
     const unsigned ties = __ballot_sync(0xffffffffu, tie && valid);
     if (ties != 0u) {
         for (int blk = 0; blk < nblk; ++blk) {
-            const float4 lo = __ldg(BL + blk), hi = __ldg(BH + blk);
-            const float dx = fmaxf(fmaxf(lo.x - ghi[0], glo[0] - hi.x), 0.f);
-            const float dy = fmaxf(fmaxf(lo.y - ghi[1], glo[1] - hi.y), 0.f);
-            const float dz = fmaxf(fmaxf(lo.z - ghi[2], glo[2] - hi.z), 0.f);
-            const float s = __fmul_rn(__fmaf_rn(dz, dz, __fmaf_rn(dx, dx, __fmul_rn(dy, dy))), 0.99999f);
+            const float s = pr_box_d2(glo[0], glo[1], glo[2], ghi[0], ghi[1], ghi[2], __ldg(BL + blk), __ldg(BH + blk));
             if (!(s <= thr)) continue;   // warp-uniform
             const float4 *tb = T + blk * PR_BLOCK;
             for (int i = 0; i < PR_BLOCK; ++i) {
@@ -739,6 +759,7 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_coop_kernel(const PrunePa
         atomicAdd(p.stats + 0, scanned);
         if (ties != 0u) atomicAdd(p.stats + 1, 1u);
         atomicAdd(p.stats + 2, 1u);
+        atomicAdd(p.stats + 3, chunks);
     }
 }
 

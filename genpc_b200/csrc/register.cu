@@ -512,8 +512,10 @@ static bool register_prune_eligible(int S, int Nc, int Nr) {
 static size_t register_prune_bytes(int S, int n_starts, int Nc, int Nr) {
     if (!register_prune_eligible(S, Nc, Nr)) return 0;
     const size_t C = (size_t)S / (n_starts > 0 ? n_starts : 1);
+    // sorted records (16 B per point), block boxes, chunk boxes (2 x 16 B per 8 points)
     return 512 + (size_t)S * sizeof(Similarity) + ((size_t)S * pr_npad(Nc) + C * pr_npad(Nr)) * sizeof(float4) +
-           2 * ((size_t)S * pr_nblk(Nc) + C * pr_nblk(Nr)) * sizeof(float4);
+           2 * ((size_t)S * pr_nblk(Nc) + C * pr_nblk(Nr)) * sizeof(float4) +
+           2 * ((size_t)S * (pr_npad(Nc) / 8) + C * (pr_npad(Nr) / 8)) * sizeof(float4);
 }
 
 // symmetric path (default for big problems): rows = fixed cloud, cols = moving cloud; the one-scan-per-direction kernel
@@ -680,11 +682,14 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
         float4 *sortedM = (float4 *)w; w += (size_t)S * pr_npad(Nc) * sizeof(float4);     // moving clouds, current pose, per scan
         float4 *sortedF = (float4 *)w; w += (size_t)C * pr_npad(Nr) * sizeof(float4);     // fixed clouds, per cloud
         float4 *boxesM = (float4 *)w; w += (size_t)S * 2 * pr_nblk(Nc) * sizeof(float4);
-        float4 *boxesF = (float4 *)w;
+        float4 *boxesF = (float4 *)w; w += (size_t)C * 2 * pr_nblk(Nr) * sizeof(float4);
+        float4 *cboxesM = (float4 *)w; w += (size_t)S * 2 * (pr_npad(Nc) / 8) * sizeof(float4);
+        float4 *cboxesF = (float4 *)w;
         cudaError_t e = cudaMemsetAsync(ctl, 0, 16, stream);
         if (e != cudaSuccess) return (int)e;
         sp.xyz[0] = ref, sp.xyz[1] = complete, sp.n[0] = Nr, sp.n[1] = Nc, sp.limit = 1e15f, sp.ctl = ctl, sp.hilbert = 1;
         sp.sorted[0] = sortedF, sp.sorted[1] = sortedM, sp.boxes[0] = boxesF, sp.boxes[1] = boxesM;
+        sp.cboxes[0] = cboxesF, sp.cboxes[1] = cboxesM;
         sp.single_side = 1, sp.accumulate = 1;
         // the fixed clouds once per call (their verdict opens the flag), the moving clouds every iteration (OR-ed in)
         sp.side0 = 0, sp.B = C, sp.accumulate = 0;
@@ -696,8 +701,10 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
         qa.B = S, qa.select = ctl + 1;
         qb = qa;
         // direction A: moving point -> nearest fixed point (packedA); direction B: fixed point -> nearest moving point (packedB)
-        qa.q = sortedM, qa.t = sortedF, qa.tbox = boxesF, qa.out = a.packedA, qa.nq = Nc, qa.nt = Nr, qa.qdiv = 1, qa.tdiv = n_starts;
-        qb.q = sortedF, qb.t = sortedM, qb.tbox = boxesM, qb.out = a.packedB, qb.nq = Nr, qb.nt = Nc, qb.qdiv = n_starts, qb.tdiv = 1;
+        qa.q = sortedM, qa.t = sortedF, qa.tbox = boxesF, qa.tcbox = cboxesF, qa.out = a.packedA, qa.nq = Nc, qa.nt = Nr;
+        qa.qdiv = 1, qa.tdiv = n_starts;
+        qb.q = sortedF, qb.t = sortedM, qb.tbox = boxesM, qb.tcbox = cboxesM, qb.out = a.packedB, qb.nq = Nr, qb.nt = Nc;
+        qb.qdiv = n_starts, qb.tdiv = 1;
         const bool a_first = qa.nq <= qb.nq;
         pp.d[0] = a_first ? qa : qb, pp.d[1] = a_first ? qb : qa;
         const int g0 = (pp.d[0].nq + PR_GROUP - 1) / PR_GROUP, g1 = (pp.d[1].nq + PR_GROUP - 1) / PR_GROUP;

@@ -54,8 +54,9 @@ int genpc_chamfer_forward(const float *xyz1, const float *xyz2, float *dist1, fl
                           int *idx2, int B, int N, int M, void *workspace, size_t workspace_bytes,
                           genpc_stream_t stream);
 
-/* Diagnostics of the spatially pruned scan (GENPC_CHAMFER_PRUNE=1, csrc/nn_prune.cuh): launches add {target blocks scanned,
- * query groups that needed the tie pass, query groups, -} to the four device counters; NULL switches it off. */
+/* Diagnostics of the spatially pruned scan (GENPC_CHAMFER_PRUNE=1, csrc/nn_prune.cuh): launches add {target blocks fetched and
+ * walked, query groups that needed the tie pass, query groups, 8-target chunks evaluated (the two-level scan of large clouds:
+ * superblocks opened)} to the four device counters; NULL switches it off. */
 int genpc_chamfer_prune_stats(unsigned *stats4);
 /* Which scan genpc_chamfer_forward would queue for this shape with the current knobs (host logic only): 0 = exhaustive,
  * 1 = Hilbert-sorted pruned exact scan (batches of >= 2^30 evaluations, 2048 .. 32768 points per cloud), 2 = two-level pruned
