@@ -59,6 +59,9 @@ def test_scan_selection_host_logic():
     assert kind(8, 8192, 8192) == 0 and kind(16, 8192, 8192) == 1
     assert kind(1, 71372, 16384) == 0                                         # C1: below 2^32 evaluations
     assert kind(1, 1000000, 1000000) == 2 and kind(9, 1000000, 1000000) == 0  # C5; the grid path sorts cloud by cloud (B <= 8)
+    assert kind(8, 600000, 40000) == 2 and kind(9, 600000, 40000) == 0
+    assert kind(1, 2097152, 2048) == 2 and kind(1, 2097152, 2047) == 0        # GR_MAX_N targets; from 2^32 evaluations
+    assert kind(1, 2097153, 4096) == 0                                        # 513 superblocks: past the 9-bit superblock id
     assert kind(32, 512, 4096) == 0 and kind(4, 100, 37) == 0
     assert kind(1000, 1791, 1755) == 0                                        # the ICP scale search: clouds too small for the sort to pay
     assert kind(0, 5, 5) < 0

@@ -12,7 +12,10 @@ quietly testing another kernel.  Thresholds are derived from the device's SM cou
   step of reg_points at its real size, B > 1) and fps_reg_kernel<32, false>, bit for bit against oracle.fps, plus a float64
   check of the max-min rule that does not use the oracle;
 - EMD with B close to or above the number of co-resident CTAs (group = 1: one cloud per CTA, or a CTA looping over clouds),
-  bit for bit against the exhaustive scan and against oracle.emd_forward / oracle.emd_backward on sampled clouds."""
+  bit for bit against the exhaustive scan and against oracle.emd_forward / oracle.emd_backward on sampled clouds;
+- Chamfer with 512 to 1023 points in the cloud that sets the tile (two rows or queries per thread): nn_sym_kernel<2> for
+  batches of at least 4 x SMs work items, nn_sym_gated_kernel<2> (host-fed forward and loss), nn_scan_kernel<2> (sharded
+  partial scans and GENPC_CHAMFER_MODE=scan), bit for bit against the oracle."""
 import json
 import os
 import tempfile
@@ -412,6 +415,120 @@ def test_knn_mean_distance_every_list_size(cuda, k):
     exp = [oracle.knn_mean_distance(x, k, inc) for x in xs for inc in (True, False)]
     for g, e in zip(got, exp):
         assert np.array_equal(g.view(np.int32), e.view(np.int32))
+
+
+# ------------------------------------------------------------------------------------- Chamfer, two rows / queries per thread
+def chamfer_batch(seed, B, n):
+    """B clouds of n points: shape clouds, every third one an integer-lattice cloud (exact distance ties)."""
+    x = shape_cloud(seed, B, n)
+    x[::3] = lattice_cloud(seed + 1, B, n, side=8)[::3]
+    return x
+
+
+def same_as_oracle(got, exp, tag):
+    for g, e, name in zip(got, exp, ("dist1", "dist2", "idx1", "idx2")):
+        bad = g.view(np.int32) != e.view(np.int32)
+        assert not bad.any(), f"{tag} {name}: {bad.sum()} of {g.size} differ, first at {np.argwhere(bad)[0]}"
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("per_sm,extra,N,M", [(2, 8, 1000, 777), (4, 4, 300, 512)])
+def test_chamfer_sym_kernel_two_rows_per_thread_vs_oracle(cuda, per_sm, extra, N, M):
+    """B = per_sm * SMs + extra clouds whose larger side has 512 to 1023 points: two rows per thread, and at least 4 x SMs work
+    items, so one CTA per item (nn_sym_kernel<2>, not the balanced form).  1000 x 777: two row tiles per cloud; 300 x 512:
+    the smallest clouds the symmetric path takes, one row tile, the second cloud as rows."""
+    import torch
+
+    from genpc_b200.loss_functions import chamfer_3DDist
+
+    B = per_sm * num_sms(cuda) + extra
+    a, b = chamfer_batch(N, B, N), chamfer_batch(M + 1, B, M)
+    ta, tb = torch.from_numpy(a).to(cuda), torch.from_numpy(b).to(cuda)
+    got, ks = launched_kernels(lambda: [t.cpu().numpy() for t in chamfer_3DDist()(ta, tb)])
+    grids(ks, "genpc::nn_sym_kernel<2>")
+    same_as_oracle(got, oracle.chamfer_forward(a, b), f"{B} x {N} x {M}")
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("B,N,M,chunks", [(64, 1000, 600, 4), (5, 513, 1023, 2)])
+def test_host_fed_forward_two_rows_per_thread_vs_oracle(cuda, B, N, M, chunks):
+    """forward_from_host with fewer than 1024 points in the larger cloud: nn_sym_gated_kernel<2>, from pinned and from pageable
+    host memory."""
+    import torch
+
+    from genpc_b200.loss_functions import chamfer_3DDist
+
+    a, b = chamfer_batch(B + N, B, N), chamfer_batch(B + M + 1, B, M)
+    exp = oracle.chamfer_forward(a, b)
+    for pin in (True, False):
+        ha, hb = torch.from_numpy(a), torch.from_numpy(b)
+        if pin:
+            ha, hb = ha.pin_memory(), hb.pin_memory()
+        got, ks = launched_kernels(
+            lambda: [t.detach().cpu().numpy() for t in chamfer_3DDist().forward_from_host(ha, hb, device=cuda, chunks=chunks)[:4]])
+        grids(ks, "genpc::nn_sym_gated_kernel<2>")
+        same_as_oracle(got, exp, f"{B} x {N} x {M}, pinned={pin}")
+
+
+@pytest.mark.gpu
+def test_loss_from_host_two_rows_per_thread_equals_device_call(cuda):
+    """get_loss_from_host('cd_l2') through nn_sym_gated_kernel<2> gives the loss of the device-resident call."""
+    import torch
+
+    from genpc_b200.utils.loss_util import Completionloss
+
+    a, b = chamfer_batch(70, 64, 1000), chamfer_batch(71, 64, 600)
+    crit = Completionloss("cd_l2")
+    ref = float(crit.get_loss(torch.from_numpy(a).to(cuda), torch.from_numpy(b).to(cuda)))
+    (loss, _, _), ks = launched_kernels(
+        lambda: crit.get_loss_from_host(torch.from_numpy(a).pin_memory(), torch.from_numpy(b).pin_memory(), device=cuda, chunks=4))
+    grids(ks, "genpc::nn_sym_gated_kernel<2>")
+    assert float(loss) == ref
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("nq", [512, 1023])
+def test_partial_scan_two_queries_per_thread_merges_to_the_oracle(cuda, nq):
+    """genpc_nn_partial_packed with 512 and 1023 queries (the edges of two queries per thread, nn_scan_kernel<2>) against three
+    ragged shards of a 30 011-point lattice cloud, global indices from idx_base: the min-merge of the packed words is
+    oracle.nn_distance against the whole cloud, distance bits and lowest indices.  Queries sit at lattice and half-integer
+    positions (several equidistant targets, often in different shards)."""
+    import torch
+
+    from genpc_b200.sharded import nn_partial_packed, nn_unpack
+
+    t = lattice_cloud(80, 1, 30011, side=40)
+    rng = np.random.default_rng(nq)
+    q = (rng.integers(0, 40, (1, nq, 3)) + 0.5 * rng.integers(0, 2, (1, nq, 3))).astype(np.float32)
+    tq, tt = torch.from_numpy(q).to(cuda), torch.from_numpy(t).to(cuda)
+    cuts = (0, 7001, 19999, 30011)
+
+    def scan():
+        parts = [nn_partial_packed(tq, tt[:, lo:hi], lo) for lo, hi in zip(cuts[:-1], cuts[1:])]
+        d, i = nn_unpack(torch.stack(parts).min(0).values)
+        return d.cpu().numpy(), i.cpu().numpy()
+
+    (d, i), ks = launched_kernels(scan)
+    assert len(grids(ks, "genpc::nn_scan_kernel<2>")) == 3
+    ed, ei = oracle.nn_distance(q, t)
+    assert np.array_equal(d.view(np.int32), ed.view(np.int32)), f"{(d != ed).sum()} distances differ"
+    assert np.array_equal(i, ei), f"{(i != ei).sum()} indices differ"
+
+
+@pytest.mark.gpu
+def test_scan_mode_two_queries_per_thread_vs_oracle(cuda):
+    """GENPC_CHAMFER_MODE=scan (one scan per direction) with 700 points in the smaller cloud: nn_scan_kernel<2>."""
+    import torch
+
+    from genpc_b200 import _lib
+    from genpc_b200.loss_functions import chamfer_3DDist
+
+    a, b = chamfer_batch(90, 4, 2600), chamfer_batch(91, 4, 700)
+    ta, tb = torch.from_numpy(a).to(cuda), torch.from_numpy(b).to(cuda)
+    with _lib.tunable(GENPC_CHAMFER_MODE="scan"):
+        got, ks = launched_kernels(lambda: [t.cpu().numpy() for t in chamfer_3DDist()(ta, tb)])
+    grids(ks, "genpc::nn_scan_kernel<2>")
+    same_as_oracle(got, oracle.chamfer_forward(a, b), "scan mode, 4 x 2600 x 700")
 
 
 # ------------------------------------------------------------------------------------------------------------ Chamfer backward

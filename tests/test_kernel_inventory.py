@@ -54,6 +54,7 @@ def library_kernels(lib=LIB):
 
 CG = "tests/test_chamfer_gpu.py::"
 PRU = "tests/test_chamfer_prune.py::"
+LARGE = "tests/test_chamfer_large_clouds.py::"
 HF = "tests/test_chamfer_host_feed.py::"
 FPS = "tests/test_fps.py::"
 EMD = "tests/test_emd.py::"
@@ -72,14 +73,14 @@ KERNELS = {
     "cub::DeviceRadixSortSingleTileKernel": "helper",
     # Chamfer: exhaustive, symmetric, pruned and grid scans, epilogue, gradients
     "genpc::nn_scan_kernel<1>": CG + "test_backward_vs_oracle",
-    "genpc::nn_scan_kernel<2>": NOT_COMPARED + "sharded partial scan with 512-1023 queries (else only GENPC_CHAMFER_MODE=scan)",
+    "genpc::nn_scan_kernel<2>": DSP + "test_partial_scan_two_queries_per_thread_merges_to_the_oracle",
     "genpc::nn_scan_kernel<4>": "tests/test_sharded.py::test_partial_scans_merge_to_the_single_gpu_result",
     "genpc::nn_unpack_kernel": CG + "test_backward_vs_oracle",
-    "genpc::nn_sym_kernel<2>": NOT_COMPARED + "symmetric scan with < 1024 rows and >= 4 x SMs work items (not balanced)",
+    "genpc::nn_sym_kernel<2>": DSP + "test_chamfer_sym_kernel_two_rows_per_thread_vs_oracle",
     "genpc::nn_sym_kernel<4>": "tests/test_c1_scan.py::test_c1_on_gpu_vs_oracle_and_golden",
     "genpc::nn_sym_balanced_kernel<2>": CG + "test_forward_bit_exact_vs_oracle",
     "genpc::nn_sym_balanced_kernel<4>": CG + "test_forward_bit_exact_vs_oracle",
-    "genpc::nn_sym_gated_kernel<2>": NOT_COMPARED + "host-fed scan with fewer than 1024 rows",
+    "genpc::nn_sym_gated_kernel<2>": DSP + "test_host_fed_forward_two_rows_per_thread_vs_oracle",
     "genpc::nn_sym_gated_kernel<4>": HF + "test_host_fed_forward_bit_exact",
     "genpc::nn_sym_epilogue_kernel<false>": CG + "test_nan_and_inf_points_stay_in_range",
     "genpc::nn_sym_epilogue_kernel<true>": "tests/test_c1_scan.py::test_c1_on_gpu_vs_oracle_and_golden",
@@ -112,10 +113,10 @@ KERNELS = {
     "genpc::nn_prune2_kernel<2,true>": PRU + "test_large_clouds_take_the_grid_scan_by_default",
     "genpc::nn_prune2_kernel<4,false>": PRU + "test_large_clouds_take_the_grid_scan_by_default",
     "genpc::nn_prune2_kernel<4,true>": PRU + "test_large_clouds_take_the_grid_scan_by_default",
-    "genpc::nn_prune2_kernel<8,false>": NOT_COMPARED + "grid scan of clouds with more superblocks than the tested sizes",
-    "genpc::nn_prune2_kernel<8,true>": NOT_COMPARED + "grid scan of clouds with more superblocks than the tested sizes",
-    "genpc::nn_prune2_kernel<16,false>": NOT_COMPARED + "grid scan of clouds with more superblocks than the tested sizes",
-    "genpc::nn_prune2_kernel<16,true>": NOT_COMPARED + "grid scan of clouds with more superblocks than the tested sizes",
+    "genpc::nn_prune2_kernel<8,false>": LARGE + "test_c5_full_size_default_path",
+    "genpc::nn_prune2_kernel<8,true>": LARGE + "test_c5_full_size_default_path",
+    "genpc::nn_prune2_kernel<16,false>": LARGE + "test_grid_scan_superblock_register_edges",
+    "genpc::nn_prune2_kernel<16,true>": LARGE + "test_grid_scan_superblock_register_edges",
     "genpc::chamfer_grad_kernel<false,false>": CG + "test_unaligned_pointers_take_the_scalar_paths",
     "genpc::chamfer_grad_kernel<false,true>": DSP + "test_fused_loss_backward_with_unaligned_gradient_arrays",
     "genpc::chamfer_grad_kernel<true,false>": CG + "test_backward_vs_oracle",
