@@ -229,51 +229,58 @@ static bool grid_eligible(int nr, int nc) {
     if (k != nullptr) return atoi(k) == 2;
     return (long long)nr * nc >= (1LL << 32) && (nr > PR_MAX_N || nc > PR_MAX_N);
 }
-static size_t grid_sort_temp_bytes(int nmax) {
-    size_t t = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, t, (const unsigned *)nullptr, (unsigned *)nullptr, (const int *)nullptr, (int *)nullptr,
-                                    nmax, 0, 30);
-    return (t + 255) & ~(size_t)255;
-}
-static size_t grid_extra_bytes(int B, int N, int M) {
-    if (!grid_eligible(N, M)) return 0;
-    size_t s = 256;
-    const int n[2] = {N, M};
-    for (int i = 0; i < 2; ++i) {
-        s += (size_t)B * pr_npad(n[i]) * sizeof(float4);                                   // sorted records
-        s += (size_t)B * 2 * ((size_t)pr_nblk(n[i]) + gr_nsb(n[i])) * sizeof(float4);      // block + superblock boxes
-        s += (size_t)B * 8 * sizeof(int);                                                  // bounding box words
-    }
-    const int nmax = N > M ? N : M;
-    s += 4 * (((size_t)nmax * 4 + 255) & ~(size_t)255) + grid_sort_temp_bytes(nmax);       // keys / values in and out, cub's scratch
-    return s;
-}
-template <int SBR>
-static void launch_prune2_t(const Prune2Params &q, cudaStream_t stream, bool probe) {
+// The pruned scan of B cloud pairs (rows: the larger cloud) as genpc_chamfer_scan_kind reports it; the workspace size follows it
+static int prune_kind(int B, int nr, int nc) { return B <= 8 && grid_eligible(nr, nc) ? 2 : (prune_eligible(B, nr, nc) ? 1 : 0); }
+static void launch_prune2(const Prune2Params &q, cudaStream_t stream, bool probe) {
     const int groups = (q.nq + PR_GROUP - 1) / PR_GROUP;
     const int work = probe ? (groups + q.probe_stride - 1) / q.probe_stride : groups;
     const dim3 grid((unsigned)((work + PR_THREADS / 32 - 1) / (PR_THREADS / 32)), (unsigned)q.B);
-    if (probe) nn_prune2_kernel<SBR, true><<<grid, PR_THREADS, 0, stream>>>(q);
-    else nn_prune2_kernel<SBR, false><<<grid, PR_THREADS, 0, stream>>>(q);
-}
-static void launch_prune2(const Prune2Params &q, cudaStream_t stream, bool probe = false) {
-    const int nsb = gr_nsb(q.nt);
-    if (nsb <= 32) launch_prune2_t<1>(q, stream, probe);
-    else if (nsb <= 64) launch_prune2_t<2>(q, stream, probe);
-    else if (nsb <= 128) launch_prune2_t<4>(q, stream, probe);
-    else if (nsb <= 256) launch_prune2_t<8>(q, stream, probe);
-    else launch_prune2_t<16>(q, stream, probe);
+    pr_rows(gr_nsb(q.nt), [&](auto r) {
+        if (probe) nn_prune2_kernel<decltype(r)::value, true><<<grid, PR_THREADS, 0, stream>>>(q);
+        else nn_prune2_kernel<decltype(r)::value, false><<<grid, PR_THREADS, 0, stream>>>(q);
+    });
 }
 constexpr int GR_PROBE_GROUPS = 128;   // sampled query groups per direction and cloud
 
-static size_t prune_extra_bytes(int B, int N, int M) {
-    if (B <= 8 && grid_eligible(N, M)) return grid_extra_bytes(B, N, M);
-    if (!prune_eligible(B, N, M)) return 0;   // (the knob is read when the workspace is sized)
-    // sorted records (16 B per point), block boxes, chunk boxes (2 x 16 B per 8 points), bounding boxes
-    return 256 + (size_t)B * ((size_t)pr_npad(N) + pr_npad(M)) * sizeof(float4) +
-           (size_t)B * 2 * ((size_t)pr_nblk(N) + pr_nblk(M)) * sizeof(float4) +
-           (size_t)B * 2 * ((size_t)pr_npad(N) / 8 + pr_npad(M) / 8) * sizeof(float4) + (size_t)B * 2 * 8 * sizeof(float);
+// The forward's workspace: the packed words (rows, then columns) and the control words of the pruned scans at its start -- a
+// re-armed workspace is reused across calls -- then, from the next 256-byte boundary, the extras of pruned scan `kind`
+struct ChamferWs {
+    size_t bytes;
+    int kind;
+    unsigned long long *packed;   // [B][nr], then [B][nc]
+    int *ctl;                     // [4]: [1] selection flag, [2] / [3] accumulator and ticket of the range check; [0] unused
+    PruneSortParams prune;        // kind 1: sorted records, block and chunk boxes, every cloud's bounding box
+    GridParams grid;              // kind 2: sorted records, block and superblock boxes, bounding box words, sort keys and values
+    unsigned *keys_out;           //   ... and the radix sort's outputs (vals_out is grid.order) and scratch
+    int *vals_out;
+    void *cub_tmp;
+    size_t cub_bytes;
+};
+static ChamferWs chamfer_layout(int B, int nr, int nc, int kind, void *base = nullptr) {
+    WsCursor c{static_cast<char *>(base)};
+    ChamferWs w = {};
+    w.kind = kind, w.packed = c.take<unsigned long long>((size_t)B * nr + (size_t)B * nc);
+    w.ctl = c.take<int>(4);
+    const int n[2] = {nr, nc}, clouds[2] = {B, B};
+    if (kind != 0) c.align_base();
+    if (kind == 1) w.prune = pr_take_sorted(c, clouds, n), w.prune.bbx = c.take<float>((size_t)2 * B * 8);
+    if (kind != 2) return w.bytes = c.bytes(), w;
+    for (int i = 0; i < 2; ++i) {
+        w.grid.sorted[i] = c.take<float4>((size_t)B * pr_npad(n[i]));
+        w.grid.boxes[i] = c.take<float4>((size_t)B * 2 * pr_nblk(n[i]));
+        w.grid.sboxes[i] = c.take<float4>((size_t)B * 2 * gr_nsb(n[i]));
+    }
+    for (int i = 0; i < 2; ++i) w.grid.bb[i] = c.take<int>((size_t)B * 8);
+    // one cloud is sorted at a time: keys and values of the largest
+    const int nmax = nr > nc ? nr : nc;
+    w.grid.keys = c.take<unsigned>(nmax, 256), w.keys_out = c.take<unsigned>(nmax, 256);
+    w.grid.vals = c.take<int>(nmax, 256), w.grid.order = w.vals_out = c.take<int>(nmax, 256);
+    cub::DeviceRadixSort::SortPairs(nullptr, w.cub_bytes, (const unsigned *)nullptr, (unsigned *)nullptr, (const int *)nullptr,
+                                    (int *)nullptr, nmax, 0, 30);
+    w.cub_tmp = c.take<char>(w.cub_bytes, 256);
+    return w.bytes = c.bytes(), w;
 }
+
 static unsigned *g_prune_stats = nullptr;   // diagnostics (genpc_chamfer_prune_stats), nullptr in production
 
 // side stream + fork / join events for the cooperative kernel, one set per (device, caller stream): created on first use, kept
@@ -300,16 +307,8 @@ static PruneSide *prune_side_stream(cudaStream_t caller) {
     return &tab[used++].s;
 }
 
-static int prune_ctas(const PruneParams &q) {
-    const int groups = (q.nq + PR_GROUP - 1) / PR_GROUP;
-    return q.B * ((groups + PR_THREADS / 32 - 1) / (PR_THREADS / 32));
-}
-// both directions in one launch; the direction with fewer queries (longer chains per group: more target blocks) goes first
 static void launch_prune(const PruneParams &a, const PruneParams &b, cudaStream_t stream) {
-    PrunePair pp = {};
-    const bool a_first = a.nq <= b.nq;
-    pp.d[0] = a_first ? a : b, pp.d[1] = a_first ? b : a;
-    pp.ctas0 = prune_ctas(pp.d[0]);
+    PrunePair pp = pr_pair(a, b);
     // few query groups against many target blocks (C2's partial -> complete direction): a CTA per group, eight warps sharing
     // its chain (nn_prune_coop_kernel) on a side stream, next to the other direction; GENPC_PRUNE_COOP=0 / 1 forbids / forces it
     const long long groups0 = (long long)pp.d[0].B * ((pp.d[0].nq + PR_GROUP - 1) / PR_GROUP);
@@ -319,23 +318,13 @@ static void launch_prune(const PruneParams &a, const PruneParams &b, cudaStream_
     if (side != nullptr) {
         cudaEventRecord(side->fork, stream);
         cudaStreamWaitEvent(side->stream, side->fork, 0);
-        const int nb0 = pr_nblk(pp.d[0].nt);
-        const unsigned g0 = (unsigned)groups0;
-        if (nb0 <= 32) nn_prune_coop_kernel<1><<<g0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
-        else if (nb0 <= 64) nn_prune_coop_kernel<2><<<g0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
-        else if (nb0 <= 128) nn_prune_coop_kernel<4><<<g0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
-        else if (nb0 <= 256) nn_prune_coop_kernel<8><<<g0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
-        else nn_prune_coop_kernel<16><<<g0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
+        pr_rows(pr_nblk(pp.d[0].nt), [&](auto r) {
+            nn_prune_coop_kernel<decltype(r)::value><<<(unsigned)groups0, PR_THREADS, 0, side->stream>>>(pp.d[0]);
+        });
         cudaEventRecord(side->join, side->stream);
         pp.ctas0 = 0;   // the launch below: direction d[1] only
     }
-    const unsigned grid = (unsigned)(pp.ctas0 + prune_ctas(pp.d[1]));
-    const int nblk = pr_nblk(side != nullptr ? pp.d[1].nt : (a.nt > b.nt ? a.nt : b.nt));
-    if (nblk <= 32) nn_prune_kernel<1><<<grid, PR_THREADS, 0, stream>>>(pp);
-    else if (nblk <= 64) nn_prune_kernel<2><<<grid, PR_THREADS, 0, stream>>>(pp);
-    else if (nblk <= 128) nn_prune_kernel<4><<<grid, PR_THREADS, 0, stream>>>(pp);
-    else if (nblk <= 256) nn_prune_kernel<8><<<grid, PR_THREADS, 0, stream>>>(pp);
-    else nn_prune_kernel<16><<<grid, PR_THREADS, 0, stream>>>(pp);
+    pr_launch(pp, stream);
     if (side != nullptr) cudaStreamWaitEvent(stream, side->join, 0);
 }
 
@@ -381,81 +370,69 @@ static void launch_bin_sort(PruneSortParams sp, int nb, cudaStream_t stream) {
     else nn_bin_sort_kernel<1><<<2 * nb, PR_SORT_THREADS, 0, stream>>>(sp);
 }
 
-// Sort + pruned scan of the cloud pairs [b0, b0 + nb) of a batch (rows / cols / prow / pcol: the batch's arrays).
-static int launch_prune_subbatch(const float *rows, const float *cols, int nr, int nc, unsigned long long *prow, unsigned long long *pcol,
-                                 int B, int b0, int nb, int *ctl, void *prune_extra, bool accumulate, cudaStream_t stream,
-                                 int *chunk_ctl = nullptr) {
-    char *w = reinterpret_cast<char *>((reinterpret_cast<size_t>(prune_extra) + 255) & ~(size_t)255);
-    float4 *sorted0 = reinterpret_cast<float4 *>(w);
-    float4 *sorted1 = sorted0 + (size_t)B * pr_npad(nr);
-    float4 *boxes0 = sorted1 + (size_t)B * pr_npad(nc);
-    float4 *boxes1 = boxes0 + (size_t)B * 2 * pr_nblk(nr);
-    float4 *cboxes0 = boxes1 + (size_t)B * 2 * pr_nblk(nc);
-    float4 *cboxes1 = cboxes0 + (size_t)B * 2 * (pr_npad(nr) / 8);
-    float *bbx = reinterpret_cast<float *>(cboxes1 + (size_t)B * 2 * (pr_npad(nc) / 8));
-    PruneSortParams sp = {};
-    sp.xyz[0] = rows + (size_t)b0 * nr * 3, sp.xyz[1] = cols + (size_t)b0 * nc * 3, sp.n[0] = nr, sp.n[1] = nc, sp.B = nb;
-    sp.limit = 1e15f, sp.ctl = chunk_ctl != nullptr ? chunk_ctl : ctl, sp.hilbert = 1, sp.accumulate = accumulate ? 1 : 0;
-    sp.flag = chunk_ctl != nullptr ? ctl + 1 : nullptr;
-    sp.sorted[0] = sorted0 + (size_t)b0 * pr_npad(nr), sp.sorted[1] = sorted1 + (size_t)b0 * pr_npad(nc);
-    sp.boxes[0] = boxes0 + (size_t)b0 * 2 * pr_nblk(nr), sp.boxes[1] = boxes1 + (size_t)b0 * 2 * pr_nblk(nc);
-    sp.cboxes[0] = cboxes0 + (size_t)b0 * 2 * (pr_npad(nr) / 8), sp.cboxes[1] = cboxes1 + (size_t)b0 * 2 * (pr_npad(nc) / 8);
-    sp.bbx = bbx + (size_t)b0 * 16;
+// Sort + pruned scan of the cloud pairs [b0, b0 + nb) of a batch of B (rows / cols: the batch's clouds; w: laid out for kind 1).
+static int launch_prune_subbatch(const float *rows, const float *cols, int nr, int nc, const ChamferWs &w, int B, int b0, int nb,
+                                 bool accumulate, cudaStream_t stream, int *chunk_ctl = nullptr) {
+    PruneSortParams sp = w.prune;   // (the whole batch's buffers: advanced to pair b0 below)
+    sp.xyz[0] = rows + (size_t)b0 * nr * 3, sp.xyz[1] = cols + (size_t)b0 * nc * 3, sp.B = nb;
+    sp.limit = 1e15f, sp.ctl = chunk_ctl != nullptr ? chunk_ctl : w.ctl, sp.hilbert = 1, sp.accumulate = accumulate ? 1 : 0;
+    sp.flag = chunk_ctl != nullptr ? w.ctl + 1 : nullptr;
+    for (int i = 0; i < 2; ++i) {
+        sp.sorted[i] += (size_t)b0 * pr_npad(sp.n[i]);
+        sp.boxes[i] += (size_t)b0 * 2 * pr_nblk(sp.n[i]);
+        sp.cboxes[i] += (size_t)b0 * 2 * (pr_npad(sp.n[i]) / 8);
+    }
+    sp.bbx += (size_t)b0 * 16;
     launch_bin_sort(sp, nb, stream);
     GENPC_CHECK_LAUNCH();
     PruneParams q = {};
-    q.B = nb, q.select = ctl + 1, q.stats = g_prune_stats;
-    q.q = sp.sorted[0], q.t = sp.sorted[1], q.tbox = sp.boxes[1], q.tcbox = sp.cboxes[1], q.out = prow + (size_t)b0 * nr, q.nq = nr,
+    q.B = nb, q.select = w.ctl + 1, q.stats = g_prune_stats;
+    q.q = sp.sorted[0], q.t = sp.sorted[1], q.tbox = sp.boxes[1], q.tcbox = sp.cboxes[1], q.out = w.packed + (size_t)b0 * nr, q.nq = nr,
     q.nt = nc;
     PruneParams q2 = q;
-    q2.q = sp.sorted[1], q2.t = sp.sorted[0], q2.tbox = sp.boxes[0], q2.tcbox = sp.cboxes[0], q2.out = pcol + (size_t)b0 * nc, q2.nq = nc,
-    q2.nt = nr;
+    q2.q = sp.sorted[1], q2.t = sp.sorted[0], q2.tbox = sp.boxes[0], q2.tcbox = sp.cboxes[0],
+    q2.out = w.packed + (size_t)B * nr + (size_t)b0 * nc, q2.nq = nc, q2.nt = nr;
     launch_prune(q, q2, stream);
     GENPC_CHECK_LAUNCH();
     return GENPC_OK;
 }
 
+// The fused loss's workspace on the symmetric path: a double partial per epilogue CTA, then the ticket (in a 16-byte slot)
+static size_t fuse_layout(int B, int N, int M, void *base, EpiFuse &f) {
+    const size_t nr = (size_t)B * (N > M ? N : M), nc = (size_t)B * (N > M ? M : N);
+    WsCursor c{static_cast<char *>(base)};
+    f.partial = c.take<double>((nc + EPI_COLS_PER_CTA - 1) / EPI_COLS_PER_CTA + (nr + EPI_ROWS_PER_CTA - 1) / EPI_ROWS_PER_CTA);
+    f.ticket = c.take<unsigned>(4);
+    return c.bytes();
+}
+
 // Symmetric path: rows = the larger cloud (registers), cols = the smaller one (shared-memory sweep).
 // gate != nullptr: host-fed launch (nn_sym_gated_kernel), see genpc_chamfer_forward_host.
 static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist1, float *dist2, int *idx1, int *idx2,
-                               int B, int N, int M, unsigned long long *packed, int *ctl, cudaStream_t stream,
+                               int B, int N, int M, const ChamferWs &w, cudaStream_t stream,
                                const unsigned *gate = nullptr, unsigned gate_gen = 0, int gate_pairs = 1,
-                               const genpc_chamfer_fuse_t *fuse = nullptr, double *fuse_partial = nullptr,
-                               unsigned *fuse_ticket = nullptr, void *prune_extra = nullptr, const int *prune_chunks = nullptr) {
+                               const genpc_chamfer_fuse_t *fuse = nullptr, const int *prune_chunks = nullptr) {
     const bool swap = M > N;
     SymParams p = {};
     p.rows = swap ? xyz2 : xyz1, p.cols = swap ? xyz1 : xyz2;
     p.nr = swap ? M : N, p.nc = swap ? N : M;
     float *dist_r = swap ? dist2 : dist1, *dist_c = swap ? dist1 : dist2;
     int *idx_r = swap ? idx2 : idx1, *idx_c = swap ? idx1 : idx2;
-    p.prow = packed, p.pcol = packed + (size_t)B * p.nr;
+    p.prow = w.packed, p.pcol = w.packed + (size_t)B * p.nr;
     p.rblock_base = 0;
     p.gate = gate, p.gate_gen = gate_gen, p.gate_pairs = gate_pairs;
     p.select = nullptr;
-    // ---- spatially pruned scan (nn_prune.cuh): both it and the exhaustive kernel below are queued; the selection flag ctl[1],
-    // written by the sort's range check or by the grid probe, decides on the device which one does the work.  ctl[2] / ctl[3]:
-    // accumulator and ticket of the range check (ctl[2] also counts the probe's block visits); ctl[0] has no user ----
-    const bool use_grid = ctl != nullptr && gate == nullptr && prune_extra != nullptr && B <= 8 && grid_eligible(p.nr, p.nc);   // one sort per cloud: small batches only
-    const bool use_prune = use_grid || (ctl != nullptr && gate == nullptr && prune_extra != nullptr && prune_eligible(B, p.nr, p.nc));
+    // ---- spatially pruned scan of w.kind (0: none; the workspace holds its extras): both it and the exhaustive kernel below are
+    // queued; the selection flag ctl[1], written by the sort's range check or by the grid probe, decides on the device which one
+    // does the work.  ctl[2] / ctl[3]: accumulator and ticket of the range check (ctl[2] also counts the probe's block visits) ----
+    int *ctl = w.ctl;
+    const bool use_grid = w.kind == 2, use_prune = w.kind != 0;
     if (use_grid) {
-        char *w = reinterpret_cast<char *>((reinterpret_cast<size_t>(prune_extra) + 255) & ~(size_t)255);
-        GridParams gp = {};
+        GridParams gp = w.grid;
         gp.B = B, gp.limit = 1e15f, gp.ctl = ctl;
         gp.xyz[0] = p.rows, gp.xyz[1] = p.cols, gp.n[0] = p.nr, gp.n[1] = p.nc;
-        for (int i = 0; i < 2; ++i) {
-            gp.sorted[i] = reinterpret_cast<float4 *>(w), w += (size_t)B * pr_npad(gp.n[i]) * sizeof(float4);
-            gp.boxes[i] = reinterpret_cast<float4 *>(w), w += (size_t)B * 2 * pr_nblk(gp.n[i]) * sizeof(float4);
-            gp.sboxes[i] = reinterpret_cast<float4 *>(w), w += (size_t)B * 2 * gr_nsb(gp.n[i]) * sizeof(float4);
-        }
-        for (int i = 0; i < 2; ++i) gp.bb[i] = reinterpret_cast<int *>(w), w += (size_t)B * 8 * sizeof(int);
-        w = reinterpret_cast<char *>((reinterpret_cast<size_t>(w) + 255) & ~(size_t)255);
         const int nmax = p.nr > p.nc ? p.nr : p.nc;
-        const size_t arr = ((size_t)nmax * 4 + 255) & ~(size_t)255;
-        unsigned *keys_in = reinterpret_cast<unsigned *>(w), *keys_out = reinterpret_cast<unsigned *>(w + arr);
-        int *vals_in = reinterpret_cast<int *>(w + 2 * arr), *vals_out = reinterpret_cast<int *>(w + 3 * arr);
-        void *cub_tmp = w + 4 * arr;
-        size_t cub_bytes = grid_sort_temp_bytes(nmax);
-        gp.keys = keys_in, gp.vals = vals_in, gp.order = vals_out;
+        size_t cub_bytes = w.cub_bytes;
         int ctas = (nmax + 4095) / 4096;
         if (ctas > 4 * GENPC_NUM_SMS) ctas = 4 * GENPC_NUM_SMS;
         if (ctas < 1) ctas = 1;
@@ -465,8 +442,8 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         for (int side = 0; side < 2; ++side)
             for (int b = 0; b < B; ++b) {   // (large clouds come in small batches)
                 grid_key_kernel<<<ctas, GR_THREADS, 0, stream>>>(gp, side, b);
-                cudaError_t es = cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, (const unsigned *)keys_in, keys_out,
-                                                                 (const int *)vals_in, vals_out, gp.n[side], 0, 30, stream);
+                cudaError_t es = cub::DeviceRadixSort::SortPairs(w.cub_tmp, cub_bytes, (const unsigned *)gp.keys, w.keys_out,
+                                                                 (const int *)gp.vals, w.vals_out, gp.n[side], 0, 30, stream);
                 if (es != cudaSuccess) return (int)es;
                 grid_gather_kernel<<<ctas, GR_THREADS, 0, stream>>>(gp, side, b, side == 0 && b == 0);
             }
@@ -502,7 +479,7 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         GENPC_CHECK_LAUNCH();
     } else if (use_prune) {
         if (prune_chunks == nullptr) {
-            const int rcp = launch_prune_subbatch(p.rows, p.cols, p.nr, p.nc, p.prow, p.pcol, B, 0, B, ctl, prune_extra, false, stream);
+            const int rcp = launch_prune_subbatch(p.rows, p.cols, p.nr, p.nc, w, B, 0, B, false, stream);
             if (rcp != GENPC_OK) return rcp;
         } else {
             // the caller (host-fed batches) has already queued sort + scan chunk by chunk as the copies landed; a LATER chunk may
@@ -515,14 +492,7 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     // measured on B200 (profiles/r01c_sym_variants.txt): QT=4 at 3 CTAs/SM is within 1 % of QT=8 at 2 CTAs/SM on
     // large clouds and clearly better when the grid is small
     const int QT = p.nr >= 1024 ? 4 : 2;
-    p.rtiles = (p.nr + SYM_THREADS * QT - 1) / (SYM_THREADS * QT);
-    // column span: the largest that still gives >= 2 waves of work items (3 CTAs x 148 SMs), at least 256 columns
-    int span = SYM_SPAN_MAX;
-    const long long want = 2LL * 3 * GENPC_NUM_SMS;
-    while (span > 256 && (long long)B * p.rtiles * ((p.nc + span - 1) / span) < want) span >>= 1;
-    p.span = span;
-    p.cspans = (p.nc + span - 1) / span;
-    const long long items = (long long)B * p.rtiles * p.cspans;
+    const long long items = sym_tiling(B, p.nr, p.nc, QT, p.rtiles, p.span, p.cspans);
     if (items > 0x7fffffffLL) return GENPC_ERR_RANGE;
     // measured on B200 (profiles/r01h_sym_balanced_vs_grid.txt): with fewer than two waves of full-span work items the
     // balanced form wins (B=1 16384^2 +5 %, 3 x 5000 x 3333 +12 %); with more, one CTA per item is 4-5 % faster (resident
@@ -564,7 +534,7 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         const double f2 = (fuse->w2 != 0.f) ? (double)fuse->w2 / (double)((size_t)B * M) : 0.0;
         f.frow = swap ? f2 : f1, f.fcol = swap ? f1 : f2;
         f.use_sqrt = fuse->use_sqrt, f.rearm = 1;
-        if (fuse->loss_out != nullptr) f.partial = fuse_partial, f.ticket = fuse_ticket, f.loss_out = fuse->loss_out;
+        if (fuse->loss_out != nullptr) fuse_layout(B, N, M, fuse->loss_workspace, f), f.loss_out = fuse->loss_out;
         f.zero[0] = fuse->zero1, f.nzero[0] = (size_t)B * N * 3;
         f.zero[1] = fuse->zero2, f.nzero[1] = (size_t)B * M * 3;
         f.err_flag = gate != nullptr ? gate + GATE_ERR_SLOT : nullptr;
@@ -575,23 +545,14 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     return GENPC_OK;
 }
 
-// Number of epilogue CTAs of the symmetric path (one loss partial each), whichever cloud ends up as rows.
-static size_t sym_epilogue_ctas(int B, int N, int M) {
-    const size_t nr = (size_t)B * (N > M ? N : M), nc = (size_t)B * (N > M ? M : N);
-    return (nc + EPI_COLS_PER_CTA - 1) / EPI_COLS_PER_CTA + (nr + EPI_ROWS_PER_CTA - 1) / EPI_ROWS_PER_CTA;
-}
-
 }  // namespace genpc
 
 using namespace genpc;
 
-// packed words + 16 control bytes (selection flag, accumulator and ticket of the pruned scans; chamfer_forward_sym)
-static size_t chamfer_base_bytes(int B, int N, int M) { return ((size_t)B * N + (size_t)B * M) * sizeof(unsigned long long) + 16; }
-
 extern "C" size_t genpc_chamfer_workspace_bytes(int B, int N, int M) {
     if (B < 0 || N < 0 || M < 0) return 0;
-    // (+ the sorted copies and block boxes of the pruned scan while GENPC_CHAMFER_PRUNE=1)
-    return chamfer_base_bytes(B, N, M) + prune_extra_bytes(B, N, M);
+    const int nr = N > M ? N : M, nc = N > M ? M : N;
+    return chamfer_layout(B, nr, nc, prune_kind(B, nr, nc)).bytes;
 }
 
 static bool takes_sym_path(int N, int M) {
@@ -603,7 +564,8 @@ static bool takes_sym_path(int N, int M) {
 
 extern "C" size_t genpc_chamfer_fuse_workspace_bytes(int B, int N, int M) {
     if (B < 0 || N < 0 || M < 0) return 0;
-    const size_t a = sym_epilogue_ctas(B, N, M) * sizeof(double) + 16;  // one partial per epilogue CTA + the ticket
+    EpiFuse f;
+    const size_t a = fuse_layout(B, N, M, nullptr, f);
     const size_t b = genpc_chamfer_loss_workspace_bytes();              // non-symmetric path: the plain loss kernel
     return a > b ? a : b;
 }
@@ -656,31 +618,25 @@ extern "C" int genpc_chamfer_forward_fused(const float *xyz1, const float *xyz2,
         GENPC_CHECK_LAUNCH();
         return fuse ? fuse_tail_unfused(fuse, dist1, dist2, B, N, M, stream) : GENPC_OK;
     }
-    if (workspace == nullptr || workspace_bytes < chamfer_base_bytes(B, N, M)) return GENPC_ERR_WORKSPACE;
-    unsigned long long *packed = (unsigned long long *)workspace;
-    cudaError_t e;
+    const int nr = N > M ? N : M, nc = N > M ? M : N;
+    if (workspace == nullptr || workspace_bytes < chamfer_layout(B, nr, nc, 0).bytes) return GENPC_ERR_WORKSPACE;
     const bool sym = takes_sym_path(N, M);
+    // (a workspace sized while the knob was off stays on the exhaustive kernels)
+    int kind = sym ? prune_kind(B, nr, nc) : 0;
+    if (workspace_bytes < chamfer_layout(B, nr, nc, kind).bytes) kind = 0;
+    const ChamferWs w = chamfer_layout(B, nr, nc, kind, workspace);
+    cudaError_t e;
     if (!(sym && fuse != nullptr && fuse->workspace_armed)) {  // an armed workspace already holds all-ones words
-        e = cudaMemsetAsync(packed, 0xff, (n1 + n2) * 8, stream);
-        if (e == cudaSuccess) e = cudaMemsetAsync(packed + n1 + n2, 0, 16, stream);   // control words (selection flag, accumulator, ticket)
+        e = cudaMemsetAsync(w.packed, 0xff, (n1 + n2) * 8, stream);
+        if (e == cudaSuccess) e = cudaMemsetAsync(w.ctl, 0, 16, stream);
         if (e != cudaSuccess) return (int)e;
     }
-    if (sym) {
-        int *ctl = (int *)(packed + n1 + n2);  // control words of the pruned scans (after the packed words)
-        double *partial = fuse ? (double *)fuse->loss_workspace : nullptr;
-        unsigned *ticket = partial ? (unsigned *)(partial + sym_epilogue_ctas(B, N, M)) : nullptr;
-        // (a workspace sized while the knob was off stays on the exhaustive kernels)
-        const size_t base_bytes = chamfer_base_bytes(B, N, M);
-        void *extra = (prune_extra_bytes(B, N, M) != 0 && workspace_bytes >= base_bytes + prune_extra_bytes(B, N, M))
-                          ? (void *)((char *)(packed + n1 + n2) + 16) : nullptr;
-        return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, packed, ctl, stream, nullptr, 0, 1, fuse,
-                                   partial, ticket, extra);
-    }
+    if (sym) return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, w, stream, nullptr, 0, 1, fuse);
 
     const int QT = nn_pick_qt(N < M ? N : M);
     NNParams p;
-    fill_dir(p.dir[0], xyz1, xyz2, packed, B, N, M, QT);
-    fill_dir(p.dir[1], xyz2, xyz1, packed + n1, B, M, N, QT);
+    fill_dir(p.dir[0], xyz1, xyz2, w.packed, B, N, M, QT);
+    fill_dir(p.dir[1], xyz2, xyz1, w.packed + n1, B, M, N, QT);
     const long long items = (long long)p.dir[0].items + p.dir[1].items;
     if (items > 0x7fffffffLL) return GENPC_ERR_RANGE;
     switch (QT) {
@@ -690,7 +646,7 @@ extern "C" int genpc_chamfer_forward_fused(const float *xyz1, const float *xyz2,
     }
     GENPC_CHECK_LAUNCH();
     const size_t tot = n1 + n2;
-    nn_unpack_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(packed, dist1, idx1, n1, dist2, idx2, n2);
+    nn_unpack_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(w.packed, dist1, idx1, n1, dist2, idx2, n2);
     GENPC_CHECK_LAUNCH();
     return fuse ? fuse_tail_unfused(fuse, dist1, dist2, B, N, M, stream) : GENPC_OK;
 }
@@ -735,9 +691,7 @@ extern "C" int genpc_chamfer_sort_layout(int B, int N, int M, int sms, int *mixe
 extern "C" int genpc_chamfer_scan_kind(int B, int N, int M) {
     if (B <= 0 || N <= 0 || M <= 0) return GENPC_ERR_SHAPE;
     if (!takes_sym_path(N, M)) return 0;
-    const int nr = N > M ? N : M, nc = N > M ? M : N;
-    if (B <= 8 && grid_eligible(nr, nc)) return 2;
-    return prune_eligible(B, nr, nc) ? 1 : 0;
+    return prune_kind(B, N > M ? N : M, N > M ? M : N);
 }
 
 // diagnostics of the pruned scan: stats4 = device pointer to 4 counters (blocks walked, groups that took the tie pass, groups,
@@ -848,7 +802,8 @@ extern "C" int genpc_chamfer_forward_host_fused(genpc_host_feed_t *f, const floa
         if (n2) FEED_CHECK(cudaMemcpyAsync(xyz2, h_xyz2, n2 * 12, cudaMemcpyHostToDevice, stream));
         return genpc_chamfer_forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, workspace, workspace_bytes, fuse, stream_);
     }
-    if (workspace == nullptr || workspace_bytes < chamfer_base_bytes(B, N, M)) return GENPC_ERR_WORKSPACE;
+    const int nr_ = M > N ? M : N, nc_ = M > N ? N : M;
+    if (workspace == nullptr || workspace_bytes < chamfer_layout(B, nr_, nc_, 0).bytes) return GENPC_ERR_WORKSPACE;
     std::lock_guard<std::mutex> guard(f->lock);   // host threads sharing the handle take turns (ADVICE r01)
     if (chunks > GATE_MAX_CHUNKS) chunks = GATE_MAX_CHUNKS;
     if (chunks > B) chunks = B;
@@ -856,26 +811,22 @@ extern "C" int genpc_chamfer_forward_host_fused(genpc_host_feed_t *f, const floa
     chunks = (B + pairs - 1) / pairs;
     // ---- pruned scan (the default for batches of this size): sort + scan are queued per chunk behind an event of the chunk's
     // copies -- no kernel waits on a gate, the last chunk's sort + scan (a few tens of us) is all that follows the last copy ----
-    const int nr_ = M > N ? M : N, nc_ = M > N ? N : M;
     // MEASURED r02 (C2 forward from pinned memory, same box, tools/time_hostfeed.py -> profiles/r02w_time_hostfeed.json): gated
     // exhaustive launch 0.326-0.334 ms (6 / 8 chunks), this path 0.260-0.270 ms (2-6 chunks, one stream per chunk; all chunks on the
     // caller's stream: 0.81 ms, each chunk's sort + scan bound by its own latency).  Before the sort kernel spread a cloud over a
     // cluster a chunk of five clouds was five 55-us CTAs and the two paths tied (0.371 vs 0.361 ms per step) -- default since then;
     // GENPC_HOST_PRUNE=0 keeps the gated launch.
     const char *hp = tunable("GENPC_HOST_PRUNE");
-    if ((hp == nullptr || atoi(hp) == 1) && prune_eligible(B, nr_, nc_) && !(B <= 8 && grid_eligible(nr_, nc_)) &&
-        workspace_bytes >= chamfer_base_bytes(B, N, M) + prune_extra_bytes(B, N, M)) {
-        unsigned long long *packed = (unsigned long long *)workspace;
-        int *ctl = (int *)(packed + n1 + n2);
-        void *extra = (void *)((char *)ctl + 16);
+    if ((hp == nullptr || atoi(hp) == 1) && prune_kind(B, nr_, nc_) == 1 && workspace_bytes >= chamfer_layout(B, nr_, nc_, 1).bytes) {
+        const ChamferWs w = chamfer_layout(B, nr_, nc_, 1, workspace);
         const float *rows = M > N ? xyz2 : xyz1, *cols = M > N ? xyz1 : xyz2;
         FEED_CHECK(cudaEventRecord(f->ready, stream));
         FEED_CHECK(cudaStreamWaitEvent(f->copy_stream, f->ready, 0));
         if (!(fuse != nullptr && fuse->workspace_armed)) {
-            FEED_CHECK(cudaMemsetAsync(packed, 0xff, (n1 + n2) * 8, stream));
-            FEED_CHECK(cudaMemsetAsync(ctl, 0, 16, stream));
+            FEED_CHECK(cudaMemsetAsync(w.packed, 0xff, (n1 + n2) * 8, stream));
+            FEED_CHECK(cudaMemsetAsync(w.ctl, 0, 16, stream));
         } else {
-            FEED_CHECK(cudaMemsetAsync(ctl + 1, 0, 4, stream));   // the chunks OR their verdicts into the selection flag
+            FEED_CHECK(cudaMemsetAsync(w.ctl + 1, 0, 4, stream));   // the chunks OR their verdicts into the selection flag
         }
         FEED_CHECK(cudaEventRecord(f->fork, stream));
         // TWO chunks whatever the caller asked for: a chunk costs ~15 driver calls (copies, events, sort, fork / join of the side
@@ -894,17 +845,13 @@ extern "C" int genpc_chamfer_forward_host_fused(genpc_host_feed_t *f, const floa
             FEED_CHECK(cudaEventRecord(f->chunk_ev[c], f->copy_stream));
             FEED_CHECK(cudaStreamWaitEvent(f->cstream[c], f->fork, 0));
             FEED_CHECK(cudaStreamWaitEvent(f->cstream[c], f->chunk_ev[c], 0));
-            const int rcs = launch_prune_subbatch(rows, cols, nr_, nc_, packed, packed + (size_t)B * nr_, B, b0, nb, ctl, extra, true,
-                                                  f->cstream[c], f->cctl + 4 * c);
+            const int rcs = launch_prune_subbatch(rows, cols, nr_, nc_, w, B, b0, nb, true, f->cstream[c], f->cctl + 4 * c);
             if (rcs != GENPC_OK) return rcs;
             FEED_CHECK(cudaEventRecord(f->done_ev[c], f->cstream[c]));
         }
         for (int c = 0; c < chunks; ++c) FEED_CHECK(cudaStreamWaitEvent(stream, f->done_ev[c], 0));
-        double *partial = fuse ? (double *)fuse->loss_workspace : nullptr;
-        unsigned *ticket = partial ? (unsigned *)(partial + sym_epilogue_ctas(B, N, M)) : nullptr;
         const int marker = chunks;
-        return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, packed, ctl, stream, nullptr, 0, 1, fuse, partial, ticket,
-                                   extra, &marker);
+        return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, w, stream, nullptr, 0, 1, fuse, &marker);
     }
     const unsigned gen = ++f->gen;
     if (gen % FEED_RING == 0) FEED_CHECK(cudaEventSynchronize(f->copied));  // the ring slot about to be reused has been read
@@ -924,15 +871,12 @@ extern "C" int genpc_chamfer_forward_host_fused(genpc_host_feed_t *f, const floa
                                    cudaMemcpyHostToDevice, f->copy_stream));
         FEED_CHECK(cudaMemcpyAsync(f->gate + c, src, sizeof(unsigned), cudaMemcpyHostToDevice, f->copy_stream));
     }
-    unsigned long long *packed = (unsigned long long *)workspace;
+    const ChamferWs w = chamfer_layout(B, nr_, nc_, 0, workspace);
     if (!(fuse != nullptr && fuse->workspace_armed)) {
-        FEED_CHECK(cudaMemsetAsync(packed, 0xff, (n1 + n2) * 8, stream));
-        FEED_CHECK(cudaMemsetAsync(packed + n1 + n2, 0, 16, stream));
+        FEED_CHECK(cudaMemsetAsync(w.packed, 0xff, (n1 + n2) * 8, stream));
+        FEED_CHECK(cudaMemsetAsync(w.ctl, 0, 16, stream));
     }
-    double *partial = fuse ? (double *)fuse->loss_workspace : nullptr;
-    unsigned *ticket = partial ? (unsigned *)(partial + sym_epilogue_ctas(B, N, M)) : nullptr;
-    const int rc = chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, packed, (int *)(packed + n1 + n2), stream, f->gate,
-                                       gen, pairs, fuse, partial, ticket);
+    const int rc = chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, w, stream, f->gate, gen, pairs, fuse);
     if (rc != GENPC_OK) return rc;
     FEED_CHECK(cudaEventRecord(f->copied, f->copy_stream));
     FEED_CHECK(cudaStreamWaitEvent(stream, f->copied, 0));  // later work on the caller's stream sees complete clouds
@@ -1021,12 +965,7 @@ extern "C" int genpc_chamfer_sym_partial(const float *rows_shard, const float *c
     p.nr = nr_shard, p.nc = nc, p.rblock_base = row_base / 128;
     p.gate = nullptr, p.gate_gen = 0, p.gate_pairs = 1;
     p.select = nullptr;
-    p.rtiles = (nr_shard + SYM_THREADS * 4 - 1) / (SYM_THREADS * 4);
-    int span = SYM_SPAN_MAX;
-    const long long want = 2LL * 3 * GENPC_NUM_SMS;
-    while (span > 256 && (long long)B * p.rtiles * ((nc + span - 1) / span) < want) span >>= 1;
-    p.span = span, p.cspans = (nc + span - 1) / span;
-    const long long items = (long long)B * p.rtiles * p.cspans;
+    const long long items = sym_tiling(B, nr_shard, nc, 4, p.rtiles, p.span, p.cspans);
     if (items > 0x7fffffffLL) return GENPC_ERR_RANGE;
     nn_sym_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
     GENPC_CHECK_LAUNCH();

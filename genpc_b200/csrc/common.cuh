@@ -24,6 +24,27 @@ namespace genpc {
 // genpc_set_tunable(); nullptr when unset.  Never calls getenv() (tunables.cu).
 const char *tunable(const char *name);
 
+// Lays out a workspace region by region.  Without a base, take() only adds up the bytes, so ONE function per workspace both
+// sizes it and carves it.  Alignments are offsets from the base, except after align_base().
+struct WsCursor {
+    char *base;   // nullptr: sizing only
+    size_t off = 0, before = 0;
+    template <typename T>
+    T *take(size_t count, size_t align = alignof(T)) {
+        off = (off + align - 1) / align * align;
+        T *p = base != nullptr ? reinterpret_cast<T *>(base + off) : nullptr;
+        off += count * sizeof(T);
+        return p;
+    }
+    // Continue at the next 256-byte boundary of the address.  The size reserves the worst-case pad of 255 bytes, so it is
+    // exact whatever the base; later alignments are offsets from the boundary.
+    void align_base() {
+        if (base != nullptr) base += off + (256 - reinterpret_cast<size_t>(base + off) % 256) % 256;
+        before += off + 255, off = 0;
+    }
+    size_t bytes() const { return before + off; }
+};
+
 // The whole library is compiled with -fmad=false: every contraction below is explicit, because the
 // reference's indices depend on the exact rounding order (SURVEY.md section 2b).
 

@@ -1008,18 +1008,26 @@ extern "C" int genpc_emd_trace_read(unsigned long long *host, int count) {
 }
 #endif
 
-extern "C" size_t genpc_emd_workspace_bytes(int B) { return B < 0 ? 0 : ((size_t)B * 4 + 4) * sizeof(int); }
+// The forward's workspace: the control words (flags, tickets, lowest prices, barriers: B each, then four scratch words of the
+// sort's range check) and, for the pruned Bid, from the next 256-byte offset the sorted targets and their block boxes
+struct EmdWs {
+    size_t bytes;
+    int *ctl;
+    float4 *tsort, *boxes;
+};
+static EmdWs emd_layout(int B, int n, bool pruned, void *base = nullptr) {
+    WsCursor c{static_cast<char *>(base)};
+    EmdWs w = {};
+    w.ctl = c.take<int>(4 * (size_t)B + 4);
+    if (pruned) w.tsort = c.take<float4>((size_t)B * n, 256), w.boxes = c.take<float4>((size_t)B * (n / EMD_BLOCK) * 2);
+    return w.bytes = c.bytes(), w;
+}
 
-static size_t emd_ctl_bytes(int B) { return (genpc_emd_workspace_bytes(B) + 255) & ~(size_t)255; }
+extern "C" size_t genpc_emd_workspace_bytes(int B) { return B < 0 ? 0 : emd_layout(B, 0, false).bytes; }
 
-// the pruned Bid needs the sorted targets (16 B each) and the block boxes behind the control words
 static bool emd_prune_feasible(int n) { return n >= EMD_BLOCK && n % EMD_BLOCK == 0 && n <= EMD_PRUNE_MAX_N; }
 
-extern "C" size_t genpc_emd_workspace_bytes_n(int B, int n) {
-    if (B < 0 || n < 0) return 0;
-    if (!emd_prune_feasible(n)) return genpc_emd_workspace_bytes(B);
-    return emd_ctl_bytes(B) + (size_t)B * n * sizeof(float4) + (size_t)B * (n / EMD_BLOCK) * 2 * sizeof(float4);
-}
+extern "C" size_t genpc_emd_workspace_bytes_n(int B, int n) { return B < 0 || n < 0 ? 0 : emd_layout(B, n, emd_prune_feasible(n)).bytes; }
 
 extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *dist, int *assignment, float *price,
                                  int *assignment_inv, int *bid, float *bid_increments, float *max_increments,
@@ -1061,12 +1069,12 @@ extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *di
     if (e != cudaSuccess) return (int)e;
     const int resident = sms * per_sm;
     if (resident <= 0) return (int)cudaErrorLaunchOutOfResources;
+    const EmdWs w = emd_layout(B, n, prune, workspace);
     EmdArgs a = {};
     a.xyz1 = xyz1, a.xyz2 = xyz2, a.dist = dist, a.assignment = assignment, a.price = price;
     a.assignment_inv = assignment_inv, a.bid = bid, a.bid_increments = bid_increments;
     a.max_increments = max_increments, a.unass_idx = unass_idx, a.unass_cnt = unass_cnt, a.max_idx = max_idx;
-    a.flags = (int *)workspace, a.tickets = (int *)workspace + B, a.pmin = (float *)workspace + 2 * (size_t)B;
-    a.bars = (int *)workspace + 3 * (size_t)B;
+    a.flags = w.ctl, a.tickets = w.ctl + B, a.pmin = (float *)(w.ctl + 2 * (size_t)B), a.bars = w.ctl + 3 * (size_t)B;
     a.B = B, a.n = n, a.eps = eps, a.iters = iters;
     int grid;
     if (B >= resident) {
@@ -1090,8 +1098,6 @@ extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *di
     a.getmax_lowest = (gm != nullptr && strcmp(gm, "lowest") == 0) ? 1 : 0;
     if ((reinterpret_cast<size_t>(xyz2) & 7) != 0 || (reinterpret_cast<size_t>(price) & 7) != 0) a.direct_p = 0;  // LDG.64
     if (prune) {
-        float4 *tsort = reinterpret_cast<float4 *>(static_cast<char *>(workspace) + emd_ctl_bytes(B));
-        float4 *boxes = tsort + (size_t)B * n;
         int np2 = 1, idxbits = 0;
         while (np2 < n) np2 <<= 1, ++idxbits;
         int mbits = (31 - idxbits) / 3;   // cell << idxbits | index stays below the 0xffffffff padding key
@@ -1110,15 +1116,15 @@ extern "C" int genpc_emd_forward(const float *xyz1, const float *xyz2, float *di
         if (sk == nullptr || strcmp(sk, "bitonic") != 0) {
             PruneSortParams sp = {};
             sp.xyz[0] = xyz2, sp.xyz[1] = xyz2, sp.n[0] = n, sp.n[1] = n, sp.B = B, sp.limit = 3.0e38f;
-            sp.sorted[0] = tsort, sp.sorted[1] = tsort, sp.boxes[0] = boxes, sp.boxes[1] = boxes;
-            sp.ctl = (int *)workspace + 4 * (size_t)B;   // scratch words of the range check (unused here)
+            sp.sorted[0] = sp.sorted[1] = w.tsort, sp.boxes[0] = sp.boxes[1] = w.boxes;
+            sp.ctl = w.ctl + 4 * (size_t)B;   // scratch words of the range check (unused here)
             sp.hilbert = (sk == nullptr || strcmp(sk, "morton") != 0) ? 1 : 0;
             nn_bin_sort_kernel<1><<<B, PR_SORT_THREADS, 0, stream>>>(sp);   // grid = B: side 0 only
         } else {
-            emd_sort_kernel<<<B, EMD_SORT_THREADS, smem, stream>>>(xyz2, tsort, boxes, n, np2, idxbits, mbits);
+            emd_sort_kernel<<<B, EMD_SORT_THREADS, smem, stream>>>(xyz2, w.tsort, w.boxes, n, np2, idxbits, mbits);
         }
         GENPC_CHECK_LAUNCH();
-        a.tsort = tsort, a.boxes = boxes;
+        a.tsort = w.tsort, a.boxes = w.boxes;
     }
     void *kargs[] = {(void *)&a};
     e = cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(EMD_THREADS), kargs, 0, stream);

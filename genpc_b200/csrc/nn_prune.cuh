@@ -25,6 +25,8 @@
 #pragma once
 #include <cooperative_groups.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 #include "nn_core.cuh"   // Similarity / apply_similarity (registration: the moving cloud is sorted in its current pose)
 
@@ -44,6 +46,17 @@ constexpr int PR_THREADS = 256;
 
 __host__ __device__ inline int pr_nblk(int n) { return (n + PR_BLOCK - 1) / PR_BLOCK; }
 __host__ __device__ inline int pr_npad(int n) { return pr_nblk(n) * PR_BLOCK; }
+
+// Calls f(std::integral_constant<int, R>()) with the rows R = 1 / 2 / 4 / 8 / 16 of 32 box distances that a lane of the pruned
+// kernels keeps in registers for `n` target blocks (or superblocks): the smallest R with R * 32 >= n
+template <typename F>
+static void pr_rows(int n, F &&f) {
+    if (n <= 32) f(std::integral_constant<int, 1>());
+    else if (n <= 64) f(std::integral_constant<int, 2>());
+    else if (n <= 128) f(std::integral_constant<int, 4>());
+    else if (n <= 256) f(std::integral_constant<int, 8>());
+    else f(std::integral_constant<int, 16>());
+}
 
 // 3 * BITS-bit Hilbert index of a grid cell (Skilling, "Programming the Hilbert curve", 2004: axes -> transpose -> interleave).
 // Consecutive indices are always neighbouring cells, so ANY run of consecutive sorted points is spatially connected; a
@@ -415,6 +428,15 @@ static __global__ void __launch_bounds__(PR_SORT_THREADS) nn_bin_sort_kernel(con
     }
 }
 
+// The sort's outputs (sorted records, block boxes, chunk boxes) for clouds[i] clouds of n[i] points on side i of a pruned scan
+static inline PruneSortParams pr_take_sorted(WsCursor &c, const int clouds[2], const int n[2]) {
+    PruneSortParams sp = {};
+    for (int i = 0; i < 2; ++i) sp.n[i] = n[i], sp.sorted[i] = c.take<float4>((size_t)clouds[i] * pr_npad(n[i]));
+    for (int i = 0; i < 2; ++i) sp.boxes[i] = c.take<float4>((size_t)clouds[i] * 2 * pr_nblk(n[i]));
+    for (int i = 0; i < 2; ++i) sp.cboxes[i] = c.take<float4>((size_t)clouds[i] * 2 * (pr_npad(n[i]) / 8));
+    return sp;
+}
+
 // `ctas` CTAs (rounded up to whole clusters) as thread-block clusters of CS
 template <int CS>
 static void launch_bin_sort_cs(PruneSortParams sp, int ctas, cudaStream_t stream) {
@@ -525,7 +547,6 @@ __device__ __forceinline__ bool pr_visit_block(float (*st)[PR_BLOCK], float4 *sb
 struct PrunePair {
     PruneParams d[2];
     int ctas0;
-    int ctas1_unused;   // (host-side bookkeeping of the registration loop)
 };
 
 // grid = sum over the two directions of B * ceil(groups / 8) CTAs of 8 warps; BOXR * 32 >= nblk of either target cloud
@@ -630,6 +651,26 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
         atomicAdd(p.stats + 2, 1u);
         atomicAdd(p.stats + 3, chunks);
     }
+}
+
+// CTAs of one direction in nn_prune_kernel: eight query groups per CTA
+static inline int pr_ctas(const PruneParams &q) {
+    const int groups = (q.nq + PR_GROUP - 1) / PR_GROUP;
+    return q.B * ((groups + PR_THREADS / 32 - 1) / (PR_THREADS / 32));
+}
+// Both directions of a cloud pair: the one with fewer queries (longer chains per group: more target blocks) goes first
+static inline PrunePair pr_pair(const PruneParams &a, const PruneParams &b) {
+    PrunePair pp = {};
+    const bool a_first = a.nq <= b.nq;
+    pp.d[0] = a_first ? a : b, pp.d[1] = a_first ? b : a;
+    pp.ctas0 = pr_ctas(pp.d[0]);
+    return pp;
+}
+// nn_prune_kernel over the pair: pp.ctas0 CTAs for d[0] (0: d[0] is launched elsewhere), then d[1]'s
+static inline void pr_launch(const PrunePair &pp, cudaStream_t stream) {
+    const unsigned grid = (unsigned)(pp.ctas0 + pr_ctas(pp.d[1]));
+    const int nt = pp.ctas0 == 0 || pp.d[1].nt > pp.d[0].nt ? pp.d[1].nt : pp.d[0].nt;
+    pr_rows(pr_nblk(nt), [&](auto r) { nn_prune_kernel<decltype(r)::value><<<grid, PR_THREADS, 0, stream>>>(pp); });
 }
 
 // Cooperative form for a direction with FEW query groups and many target blocks (C2: 2048 groups against 256 blocks each): one

@@ -43,6 +43,17 @@ struct SymParams {
     const int *select;
 };
 
+// Work items of the symmetric scan over B cloud pairs: row tiles of SYM_THREADS * QT rows x column spans, the span the largest
+// that still gives >= 2 waves of work items (3 CTAs x SMs), at least 256 columns.  Returns B * rtiles * cspans.
+static inline long long sym_tiling(int B, int nr, int nc, int QT, int &rtiles, int &span, int &cspans) {
+    rtiles = (nr + SYM_THREADS * QT - 1) / (SYM_THREADS * QT);
+    span = SYM_SPAN_MAX;
+    const long long want = 2LL * 3 * GENPC_NUM_SMS;
+    while (span > 256 && (long long)B * rtiles * ((nc + span - 1) / span) < want) span >>= 1;
+    cspans = (nc + span - 1) / span;
+    return (long long)B * rtiles * cspans;
+}
+
 // Coordinates arriving by DMA while the kernel is resident must not go through the non-coherent path (ld.global.nc
 // assumes data that is read-only for the whole launch): gated launches read them with ld.global.cg instead.
 template <bool COHERENT>

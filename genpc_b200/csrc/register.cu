@@ -509,14 +509,6 @@ static bool register_prune_eligible(int S, int Nc, int Nr) {
     const double groups = (double)S * ((double)Nc + (double)Nr) / PR_GROUP;
     return Nc >= 1024 && Nr >= 1024 && (double)S * (double)Nc * (double)Nr >= (double)(1LL << 30) && groups >= 20000.0;
 }
-static size_t register_prune_bytes(int S, int n_starts, int Nc, int Nr) {
-    if (!register_prune_eligible(S, Nc, Nr)) return 0;
-    const size_t C = (size_t)S / (n_starts > 0 ? n_starts : 1);
-    // sorted records (16 B per point), block boxes, chunk boxes (2 x 16 B per 8 points)
-    return 512 + (size_t)S * sizeof(Similarity) + ((size_t)S * pr_npad(Nc) + C * pr_npad(Nr)) * sizeof(float4) +
-           2 * ((size_t)S * pr_nblk(Nc) + C * pr_nblk(Nr)) * sizeof(float4) +
-           2 * ((size_t)S * (pr_npad(Nc) / 8) + C * (pr_npad(Nr) / 8)) * sizeof(float4);
-}
 
 // symmetric path (default for big problems): rows = fixed cloud, cols = moving cloud; the one-scan-per-direction kernel
 // stays for tiny fixed clouds and for A/B runs (GENPC_REGISTER_MODE=scan).  Measured on B200
@@ -539,15 +531,34 @@ static size_t register_partial_slots(int Nc, int Nr) {
     return fix_ctas > items ? fix_ctas : items;
 }
 
-static size_t register_base_bytes(int S, int Nc, int Nr) {
-    return ((size_t)S * Nc + (size_t)S * Nr) * 8 + (size_t)S * register_partial_slots(Nc, Nr) * 14 * sizeof(double) +
-           3 * (size_t)S * sizeof(int);   // tickets, iter_done, arrivals
+// The workspace of S scans of C clouds: packed words, partial sums and counters; for the pruned scan, from the next 256-byte
+// boundary, its control words, the scans' similarities and the sorted copies and boxes (side 0: the fixed clouds, side 1: the moving)
+struct RegWs {
+    size_t bytes;
+    RegArgs args;           // packedA, packedB, partials, counters (tickets, iter_done, arrivals)
+    int *ctl;
+    Similarity *sims;
+    PruneSortParams sort;   // sorted records, block and chunk boxes
+};
+static RegWs register_layout(int S, int C, int Nc, int Nr, bool pruned, void *base = nullptr) {
+    WsCursor c{static_cast<char *>(base)};
+    RegWs w = {};
+    w.args.packedA = c.take<unsigned long long>((size_t)S * Nc);
+    w.args.packedB = c.take<unsigned long long>((size_t)S * Nr);
+    w.args.partials = c.take<double>((size_t)S * register_partial_slots(Nc, Nr) * 14);
+    w.args.counters = c.take<int>(3 * (size_t)S);
+    if (!pruned) return w.bytes = c.bytes(), w;
+    const int clouds[2] = {C, S}, n[2] = {Nr, Nc};
+    c.align_base();
+    w.ctl = c.take<int>(4), w.sims = c.take<Similarity>(S, 16);
+    w.sort = pr_take_sorted(c, clouds, n);
+    return w.bytes = c.bytes(), w;
 }
 
 extern "C" size_t genpc_register_workspace_bytes(int S, int Nc, int Nr) {
     if (S < 0 || Nc < 0 || Nr < 0) return 0;
-    // (+ the pruned scan's copies, sized for one start per cloud -- the largest case; genpc_register_run checks what it needs)
-    return register_base_bytes(S, Nc, Nr) + register_prune_bytes(S, 1, Nc, Nr);
+    // (with the pruned scan's extras: sized for one start per cloud -- the largest case; genpc_register_run checks what it needs)
+    return register_layout(S, S, Nc, Nr, register_prune_eligible(S, Nc, Nr)).bytes;
 }
 
 // Kernel launches one Adam iteration costs at this problem size (1: single-launch path, 2: symmetric scan + finish).
@@ -566,13 +577,13 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
     cudaStream_t stream = (cudaStream_t)stream_;
     if (S <= 0 || n_starts <= 0 || S % n_starts != 0 || Nc <= 0 || Nr <= 0 || iters < 0 || t_start < 0) return GENPC_ERR_SHAPE;
     if (loss_hist != nullptr && t_start + iters > T) return GENPC_ERR_SHAPE;
-    if (workspace == nullptr || workspace_bytes < register_base_bytes(S, Nc, Nr)) return GENPC_ERR_WORKSPACE;
-    RegArgs a = {};
+    const int C = S / n_starts;
+    if (workspace == nullptr || workspace_bytes < register_layout(S, C, Nc, Nr, false).bytes) return GENPC_ERR_WORKSPACE;
+    const bool sym = register_takes_sym_path(S, Nc, Nr);
+    const bool prune = sym && register_prune_eligible(S, Nc, Nr) && workspace_bytes >= register_layout(S, C, Nc, Nr, true).bytes;
+    const RegWs w = register_layout(S, C, Nc, Nr, prune, workspace);
+    RegArgs a = w.args;
     a.complete = complete, a.center = center, a.ref = ref, a.params = params, a.adam_m = adam_m, a.adam_v = adam_v;
-    a.packedA = (unsigned long long *)workspace;
-    a.packedB = a.packedA + (size_t)S * Nc;
-    a.partials = (double *)(a.packedB + (size_t)S * Nr);
-    a.counters = (int *)(a.partials + (size_t)S * register_partial_slots(Nc, Nr) * 14);
     a.loss_hist = loss_hist;
     a.S = S, a.n_starts = n_starts, a.Nc = Nc, a.Nr = Nr, a.T = T;
     // queries per thread of the single-launch path: the real pipeline registers 1-3 K-point clouds with 4 starts -- a few
@@ -598,21 +609,14 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
     };
     long long grid = set_span(NN_SPAN);
     if (grid > 0x7fffffffLL) return GENPC_ERR_RANGE;
-    const bool sym = register_takes_sym_path(S, Nc, Nr);
     const int SQT = Nr >= 1024 ? 4 : 2;
     long long sgrid = 0, fgrid = 0;
     const int fix_cols = fix_cols_per_cta(S, Nc);
     if (sym) {
-        a.rtiles = (Nr + SYM_THREADS * SQT - 1) / (SYM_THREADS * SQT);
-        int span = SYM_SPAN_MAX;
-        const long long want = 2LL * 3 * GENPC_NUM_SMS;
-        while (span > 256 && (long long)S * a.rtiles * ((Nc + span - 1) / span) < want) span >>= 1;
-        a.span = span;
-        a.cspans = (Nc + span - 1) / span;
+        sgrid = sym_tiling(S, Nr, Nc, SQT, a.rtiles, a.span, a.cspans);
         a.rows_per_block = 32 * SQT;
         a.fix_ctas = (Nc + fix_cols - 1) / fix_cols;
         a.ticket_total = a.fix_ctas;
-        sgrid = (long long)S * a.rtiles * a.cspans;
         fgrid = (long long)S * a.fix_ctas;
         if (sgrid > 0x7fffffffLL || fgrid > 0x7fffffffLL) return GENPC_ERR_RANGE;
     }
@@ -667,49 +671,28 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
         grid = set_span(NN_SPAN);   // not co-resident: one launch per iteration with full spans
     }
     // ---- pruned scan set-up: control words, similarities, sorted copies behind the base workspace ----
-    const bool prune = sym && register_prune_eligible(S, Nc, Nr) &&
-                       workspace_bytes >= register_base_bytes(S, Nc, Nr) + register_prune_bytes(S, n_starts, Nc, Nr);
-    PruneSortParams sp = {};
+    PruneSortParams sp = w.sort;
     PrunePair pp = {};
-    Similarity *sims = nullptr;
     if (prune) {
-        const int C = S / n_starts;
-        char *w = (char *)workspace + register_base_bytes(S, Nc, Nr);
-        w = (char *)(((size_t)w + 255) & ~(size_t)255);
-        int *ctl = (int *)w;
-        w += 256;
-        sims = (Similarity *)w, w += (((size_t)S * sizeof(Similarity)) + 15) & ~(size_t)15;
-        float4 *sortedM = (float4 *)w; w += (size_t)S * pr_npad(Nc) * sizeof(float4);     // moving clouds, current pose, per scan
-        float4 *sortedF = (float4 *)w; w += (size_t)C * pr_npad(Nr) * sizeof(float4);     // fixed clouds, per cloud
-        float4 *boxesM = (float4 *)w; w += (size_t)S * 2 * pr_nblk(Nc) * sizeof(float4);
-        float4 *boxesF = (float4 *)w; w += (size_t)C * 2 * pr_nblk(Nr) * sizeof(float4);
-        float4 *cboxesM = (float4 *)w; w += (size_t)S * 2 * (pr_npad(Nc) / 8) * sizeof(float4);
-        float4 *cboxesF = (float4 *)w;
-        cudaError_t e = cudaMemsetAsync(ctl, 0, 16, stream);
+        cudaError_t e = cudaMemsetAsync(w.ctl, 0, 16, stream);
         if (e != cudaSuccess) return (int)e;
-        sp.xyz[0] = ref, sp.xyz[1] = complete, sp.n[0] = Nr, sp.n[1] = Nc, sp.limit = 1e15f, sp.ctl = ctl, sp.hilbert = 1;
-        sp.sorted[0] = sortedF, sp.sorted[1] = sortedM, sp.boxes[0] = boxesF, sp.boxes[1] = boxesM;
-        sp.cboxes[0] = cboxesF, sp.cboxes[1] = cboxesM;
+        sp.xyz[0] = ref, sp.xyz[1] = complete, sp.limit = 1e15f, sp.ctl = w.ctl, sp.hilbert = 1;
         sp.single_side = 1, sp.accumulate = 1;
         // the fixed clouds once per call (their verdict opens the flag), the moving clouds every iteration (OR-ed in)
         sp.side0 = 0, sp.B = C, sp.accumulate = 0;
         nn_bin_sort_kernel<1><<<C, PR_SORT_THREADS, 0, stream>>>(sp);
         GENPC_CHECK_LAUNCH();
-        sp.side0 = 1, sp.B = S, sp.accumulate = 1, sp.src_div[1] = n_starts, sp.sim[1] = sims;
-        a.select = ctl + 1;
+        sp.side0 = 1, sp.B = S, sp.accumulate = 1, sp.src_div[1] = n_starts, sp.sim[1] = w.sims;
+        a.select = w.ctl + 1;
         PruneParams qa = {}, qb = {};
-        qa.B = S, qa.select = ctl + 1;
+        qa.B = S, qa.select = w.ctl + 1;
         qb = qa;
         // direction A: moving point -> nearest fixed point (packedA); direction B: fixed point -> nearest moving point (packedB)
-        qa.q = sortedM, qa.t = sortedF, qa.tbox = boxesF, qa.tcbox = cboxesF, qa.out = a.packedA, qa.nq = Nc, qa.nt = Nr;
+        qa.q = sp.sorted[1], qa.t = sp.sorted[0], qa.tbox = sp.boxes[0], qa.tcbox = sp.cboxes[0], qa.out = a.packedA, qa.nq = Nc, qa.nt = Nr;
         qa.qdiv = 1, qa.tdiv = n_starts;
-        qb.q = sortedF, qb.t = sortedM, qb.tbox = boxesM, qb.tcbox = cboxesM, qb.out = a.packedB, qb.nq = Nr, qb.nt = Nc;
+        qb.q = sp.sorted[0], qb.t = sp.sorted[1], qb.tbox = sp.boxes[1], qb.tcbox = sp.cboxes[1], qb.out = a.packedB, qb.nq = Nr, qb.nt = Nc;
         qb.qdiv = n_starts, qb.tdiv = 1;
-        const bool a_first = qa.nq <= qb.nq;
-        pp.d[0] = a_first ? qa : qb, pp.d[1] = a_first ? qb : qa;
-        const int g0 = (pp.d[0].nq + PR_GROUP - 1) / PR_GROUP, g1 = (pp.d[1].nq + PR_GROUP - 1) / PR_GROUP;
-        pp.ctas0 = S * ((g0 + PR_THREADS / 32 - 1) / (PR_THREADS / 32));
-        pp.ctas1_unused = S * ((g1 + PR_THREADS / 32 - 1) / (PR_THREADS / 32));
+        pp = pr_pair(qa, qb);
     }
     for (int it = 0; it < iters; ++it) {
         const int t = t_start + it;
@@ -719,15 +702,9 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
         a.bc2_sqrt = (float)sqrt(1.0 - pow(0.999, (double)(t + 1)));
         if (sym) {
             if (prune) {
-                register_sims_kernel<<<(S + 127) / 128, 128, 0, stream>>>(a, sims);
+                register_sims_kernel<<<(S + 127) / 128, 128, 0, stream>>>(a, w.sims);
                 nn_bin_sort_kernel<1><<<S, PR_SORT_THREADS, 0, stream>>>(sp);
-                const unsigned pgrid = (unsigned)(pp.ctas0 + pp.ctas1_unused);
-                const int nblk = pr_nblk(Nc > Nr ? Nc : Nr);
-                if (nblk <= 32) nn_prune_kernel<1><<<pgrid, PR_THREADS, 0, stream>>>(pp);
-                else if (nblk <= 64) nn_prune_kernel<2><<<pgrid, PR_THREADS, 0, stream>>>(pp);
-                else if (nblk <= 128) nn_prune_kernel<4><<<pgrid, PR_THREADS, 0, stream>>>(pp);
-                else if (nblk <= 256) nn_prune_kernel<8><<<pgrid, PR_THREADS, 0, stream>>>(pp);
-                else nn_prune_kernel<16><<<pgrid, PR_THREADS, 0, stream>>>(pp);
+                pr_launch(pp, stream);
                 GENPC_CHECK_LAUNCH();
             }
             if (SQT == 4) register_sym_scan_kernel<4><<<(unsigned)sgrid, SYM_THREADS, 0, stream>>>(a);
