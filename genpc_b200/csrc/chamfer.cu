@@ -499,9 +499,14 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     // CTAs drift out of phase, so staging / publishing of one overlaps the scan of the other)
     const char *bm = tunable("GENPC_SYM_BALANCED");
     const bool few_items = (long long)B * p.rtiles * ((p.nc + SYM_SPAN_MAX - 1) / SYM_SPAN_MAX) < 4LL * GENPC_NUM_SMS;
-    // (the pruned grid scan queues this launch only as the device-selected fall-back: a fixed-size grid returns at once,
-    // one CTA per work item of a 1M x 1M pair spent 0.8 ms launching CTAs that do nothing)
-    const bool balanced = (bm == nullptr) ? ((GENPC_DEFAULT_BALANCED && few_items) || use_grid) : (atoi(bm) != 0);
+    // Behind a pruned scan this launch is only the device-selected fall-back, and a fixed-size grid returns at once: one CTA per
+    // work item of a 1M x 1M pair spent 0.8 ms launching CTAs that do nothing (grid scan), and C2's 2048 items were a 3-4 us
+    // launch between the pruned scan and the epilogue.  When the fall-back does run (out-of-range, far-apart or collapsed clouds)
+    // C2-sized batches pay the balanced form's 4-5 % (above) -- inputs already off the fast path.  Behind the Hilbert-sorted
+    // pruned scan it is also a programmatic dependent (launch_pdl): of nn_prune_kernel, or of the join with the cooperative kernel
+    const bool balanced = (bm == nullptr) ? ((GENPC_DEFAULT_BALANCED && few_items) || use_prune) : (atoi(bm) != 0);
+    const bool dep = w.kind == 1;
+    cudaError_t es = cudaSuccess;
     if (gate != nullptr) {
         if (QT >= 4) nn_sym_gated_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
         else nn_sym_gated_kernel<2><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
@@ -511,12 +516,15 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         const long long units = (long long)B * p.rtiles * upj;
         if (units > 0x7fffffffLL) return GENPC_ERR_RANGE;
         const int grid = (int)(units < 2LL * GENPC_NUM_SMS ? units : 2LL * GENPC_NUM_SMS);
-        if (QT == 4) nn_sym_balanced_kernel<4><<<grid, SYM_THREADS, 0, stream>>>(p, (int)units, upj);
-        else nn_sym_balanced_kernel<2><<<grid, SYM_THREADS, 0, stream>>>(p, (int)units, upj);
+        auto kb = QT == 4 ? nn_sym_balanced_kernel<4> : nn_sym_balanced_kernel<2>;
+        if (dep) es = launch_pdl(kb, dim3(grid), dim3(SYM_THREADS), stream, p, (int)units, upj);
+        else kb<<<grid, SYM_THREADS, 0, stream>>>(p, (int)units, upj);
     } else {
-        if (QT == 4) nn_sym_kernel<4><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
-        else nn_sym_kernel<2><<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
+        auto kg = QT == 4 ? nn_sym_kernel<4> : nn_sym_kernel<2>;
+        if (dep) es = launch_pdl(kg, dim3((unsigned)items), dim3(SYM_THREADS), stream, p);
+        else kg<<<(unsigned)items, SYM_THREADS, 0, stream>>>(p);
     }
+    if (es != cudaSuccess) return (int)es;
     GENPC_CHECK_LAUNCH();
     const size_t nrw = (size_t)B * p.nr, ncw = (size_t)B * p.nc;
     const unsigned fix_blocks = (unsigned)((ncw + EPI_COLS_PER_CTA - 1) / EPI_COLS_PER_CTA);
@@ -525,9 +533,11 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     memset(&f, 0, sizeof(f));
     // column words are exact iff the pruned scan did the work (ctl[1] == 0)
     f.select = use_prune ? ctl + 1 : nullptr;
+    // the epilogue is a programmatic dependent of the scan launched above (whichever it is: every one of them triggers early)
+    const dim3 egrid(fix_blocks + unpack_blocks);
     if (fuse == nullptr) {
-        nn_sym_epilogue_kernel<false><<<fix_blocks + unpack_blocks, 256, 0, stream>>>(
-            p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT, fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
+        es = launch_pdl(nn_sym_epilogue_kernel<false>, egrid, dim3(256), stream, p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT,
+                        fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
     } else {
         // dist1 belongs to xyz1: the row cloud unless the clouds were swapped
         const double f1 = (fuse->w1 != 0.f) ? (double)fuse->w1 / (double)((size_t)B * N) : 0.0;
@@ -538,10 +548,10 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
         f.zero[0] = fuse->zero1, f.nzero[0] = (size_t)B * N * 3;
         f.zero[1] = fuse->zero2, f.nzero[1] = (size_t)B * M * 3;
         f.err_flag = gate != nullptr ? gate + GATE_ERR_SLOT : nullptr;
-        nn_sym_epilogue_kernel<true><<<fix_blocks + unpack_blocks, 256, 0, stream>>>(
-            p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT, fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
+        es = launch_pdl(nn_sym_epilogue_kernel<true>, egrid, dim3(256), stream, p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT,
+                        fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
     }
-    GENPC_CHECK_LAUNCH();
+    if (es != cudaSuccess) return (int)es;
     return GENPC_OK;
 }
 

@@ -45,6 +45,23 @@ struct WsCursor {
     size_t bytes() const { return before + off; }
 };
 
+// Programmatic dependent launch: kernel<<<grid, block, 0, stream>>>(args...) may be dispatched while the kernel before it on
+// `stream` is still draining (from the moment every CTA of that kernel has called cudaTriggerProgrammaticLaunchCompletion()
+// or exited), so the launch latency between two of the library's kernels overlaps the first one's tail.  A kernel launched
+// this way calls cudaGridDependencySynchronize() in every CTA before it touches global memory that an earlier launch on the
+// stream reads or writes (and before it can exit, so that its own completion still implies its predecessor's); only parameter
+// decoding and index math come first.
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid, cfg.blockDim = block, cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr, cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
 // The whole library is compiled with -fmad=false: every contraction below is explicit, because the
 // reference's indices depend on the exact rounding order (SURVEY.md section 2b).
 

@@ -130,6 +130,7 @@ static __global__ void prune_rearm_kernel(unsigned long long *words, size_t n, c
 // barrier.  One CTA per 16384-point cloud was 55 us of C2's 170 us forward with 84 of the 148 SMs idle.
 template <int CS>
 static __global__ void __launch_bounds__(PR_SORT_THREADS) nn_bin_sort_kernel(const PruneSortParams p) {
+    cudaTriggerProgrammaticLaunchCompletion();   // the pruned scan behind it (launch_pdl) may take the SMs the sort leaves free
     __shared__ __align__(16) int hist[PR_MAX_CELLS];
     __shared__ __align__(16) int slot[CS > 1 ? PR_MAX_CELLS : 4];   // CS > 1: next free slot per cell (hist stays readable for the siblings)
     __shared__ float sred[6][PR_SORT_THREADS / 32];
@@ -556,6 +557,8 @@ __global__ void __launch_bounds__(PR_THREADS) nn_prune_kernel(const PrunePair pp
     __shared__ float4 sbox[PR_THREADS / 32][16];                           // ... and its chunk boxes: lower corners, upper corners
     const int dir = (int)blockIdx.x >= pp.ctas0 ? 1 : 0;
     const PruneParams &p = pp.d[dir];
+    cudaGridDependencySynchronize();   // launched behind the sort (pr_launch): its records, boxes and selection flag are complete
+    cudaTriggerProgrammaticLaunchCompletion();
     if (p.select != nullptr && *p.select != 0) return;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int groups = (p.nq + PR_GROUP - 1) / PR_GROUP;
@@ -666,11 +669,12 @@ static inline PrunePair pr_pair(const PruneParams &a, const PruneParams &b) {
     pp.ctas0 = pr_ctas(pp.d[0]);
     return pp;
 }
-// nn_prune_kernel over the pair: pp.ctas0 CTAs for d[0] (0: d[0] is launched elsewhere), then d[1]'s
+// nn_prune_kernel over the pair: pp.ctas0 CTAs for d[0] (0: d[0] is launched elsewhere), then d[1]'s; a programmatic dependent
+// of the sort queued before it
 static inline void pr_launch(const PrunePair &pp, cudaStream_t stream) {
     const unsigned grid = (unsigned)(pp.ctas0 + pr_ctas(pp.d[1]));
     const int nt = pp.ctas0 == 0 || pp.d[1].nt > pp.d[0].nt ? pp.d[1].nt : pp.d[0].nt;
-    pr_rows(pr_nblk(nt), [&](auto r) { nn_prune_kernel<decltype(r)::value><<<grid, PR_THREADS, 0, stream>>>(pp); });
+    pr_rows(pr_nblk(nt), [&](auto r) { launch_pdl(nn_prune_kernel<decltype(r)::value>, dim3(grid), dim3(PR_THREADS), stream, pp); });
 }
 
 // Cooperative form for a direction with FEW query groups and many target blocks (C2: 2048 groups against 256 blocks each): one

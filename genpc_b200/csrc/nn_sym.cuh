@@ -190,6 +190,8 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
 template <int QT>
 __global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_kernel(const SymParams p) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
+    cudaGridDependencySynchronize();   // a programmatic dependent of the pruned scan when it is that scan's fall-back
+    cudaTriggerProgrammaticLaunchCompletion();
     if (p.select != nullptr && *p.select == 0) return;
     int item = blockIdx.x;
     const int cs = item % p.cspans;
@@ -213,6 +215,7 @@ constexpr long long GATE_TIMEOUT_CLK = 4000000000LL;  // ~2 s at 1.965 GHz
 template <int QT>
 __global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_gated_kernel(const SymParams p) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
+    cudaTriggerProgrammaticLaunchCompletion();   // (never launched as a dependent: it follows memsets)
     if (p.select != nullptr && *p.select == 0) return;
     int item = blockIdx.x;
     const int cs = item % p.cspans;
@@ -248,6 +251,8 @@ template <int QT>
 __global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_balanced_kernel(const SymParams p, int total_units,
                                                                           int units_per_job) {
     __shared__ __align__(16) float s[3][SYM_SPAN_MAX];
+    cudaGridDependencySynchronize();   // a programmatic dependent of the pruned scan when it is that scan's fall-back
+    cudaTriggerProgrammaticLaunchCompletion();
     if (p.select != nullptr && *p.select == 0) return;
     int u = (int)((long long)total_units * blockIdx.x / gridDim.x);
     const int u_end = (int)((long long)total_units * (blockIdx.x + 1) / gridDim.x);
@@ -386,6 +391,9 @@ static __global__ void __launch_bounds__(256) nn_sym_epilogue_kernel(const float
                                                                      float *__restrict__ dist_c, int *__restrict__ idx_c,
                                                                      const EpiFuse f) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    // a programmatic dependent of the scan: the packed words, the selection flag, the outputs and the gradient accumulators are
+    // all touched below this point
+    cudaGridDependencySynchronize();
     const bool cols_exact = f.select != nullptr && *f.select == 0;   // a pruned scan ran: nothing to fix up (warp-uniform)
     double term = 0.0;  // sum of f(d) over the output elements this thread owns
     if (blockIdx.x >= fix_blocks) {
