@@ -75,6 +75,8 @@ _SIGNATURES = {
     "genpc_register_launches_per_iter": (_int, [_int, _int, _int]),
     "genpc_register_run": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _int, _int, _int,
                                   _dbl, _dbl, _dbl, _flt, _flt, _flt, _vp, _sz, _int, _vp]),
+    "genpc_register_run_ragged": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _int, _int,
+                                         _int, _dbl, _dbl, _dbl, _flt, _flt, _flt, _vp, _sz, _int, _vp]),
 }
 
 

@@ -18,6 +18,9 @@
 // Large problems (S*Nc*Nr >= 2e8) use the symmetric scan instead (register_sym_scan_kernel: every distance evaluated
 // once for both directions, nn_sym.cuh) followed by register_finish_kernel (per-point index fix-up, then the same
 // ticketed finalize): two launches per iteration, 1.34x faster at 64 x 16384^2.
+// Ragged batches (genpc_register_run_ragged: per-cloud point counts inside padded strides) run register_step_kernel, one
+// launch per iteration, whatever the size: each cloud's scans stop at its own counts and its loss is the mean over its own
+// points.  The persistent, symmetric and pruned kernels keep their equal-size code (no per-cloud counts there).
 #include <cstdlib>
 #include <cstring>
 
@@ -52,6 +55,11 @@ struct RegArgs {
     const int *select;
     int nn_span;   // targets per work item of the single-launch / persistent kernels (256, 512 or NN_SPAN)
 };
+
+// points of `cloud` (clamped to [1, stride] so that no index leaves the cloud whatever a caller passes)
+__device__ __forceinline__ int cloud_len(const int *len, int cloud, int stride) {
+    return len == nullptr ? stride : min(max(__ldg(len + cloud), 1), stride);
+}
 
 __device__ __forceinline__ void load_similarity(const float *par, const float *center, Similarity &T) {
     rot6d_to_matrix(par, T.R);
@@ -191,8 +199,26 @@ __device__ __noinline__ void finalize_scan(const RegArgs &a, int scan, const Sim
     pose_update(a, scan, T, tot, st);
 }
 
+// A scan of a ragged batch is finalised as an equal-size scan of its own counts: a copy of the arguments whose Nc / Nr are the
+// cloud's counts and whose base pointers are moved so that THIS scan's cloud and packed words sit where the stride-based
+// addressing of finalize_scan expects them (moved by cloud * (stride - count) points: still inside the buffers).  The loss
+// coefficients, loops and re-arm then stop at the counts, and finalize_scan stays the equal-size code.
+__device__ __forceinline__ RegArgs cloud_args(const RegArgs &a, const int *nc_len, const int *nr_len, int scan, int cloud) {
+    RegArgs b = a;
+    const int nc = cloud_len(nc_len, cloud, a.Nc), nr = cloud_len(nr_len, cloud, a.Nr);
+    b.complete = a.complete + (size_t)cloud * (a.Nc - nc) * 3;
+    b.ref = a.ref + (size_t)cloud * (a.Nr - nr) * 3;
+    b.packedA = a.packedA + (size_t)scan * (a.Nc - nc);
+    b.packedB = a.packedB + (size_t)scan * (a.Nr - nr);
+    b.Nc = nc, b.Nr = nr;
+    return b;
+}
+
 template <int QT>
-__global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) register_step_kernel(const RegArgs a) {
+// nc_len / nr_len: points of each moving / fixed cloud [C] of a ragged batch (the rest of its Nc / Nr stride is padding that is
+// never read); nullptr: every cloud fills its stride.  (Kernel arguments rather than RegArgs fields: the other kernels, which
+// take no ragged batches, keep their argument block and code.)
+__global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) register_step_kernel(const RegArgs a, const int *nc_len, const int *nr_len) {
     __shared__ __align__(16) float s[3][NN_SPAN];
     __shared__ Similarity T;
     __shared__ int is_last;
@@ -204,15 +230,34 @@ __global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) register_step_kernel
     __syncthreads();
     const float *V = a.complete + (size_t)cloud * a.Nc * 3;
     const float *Rf = a.ref + (size_t)cloud * a.Nr * 3;
-    if (item < a.itemsA) {  // A: moving queries vs fixed targets
-        const int ts = item % a.tsplitsA, qt = item / a.tsplitsA;
-        nn_scan_item<QT>(s, V, a.Nc, qt * (NN_THREADS * QT), Rf, a.Nr, ts * NN_SPAN, 0, &T, nullptr,
-                         a.packedA + (size_t)scan * a.Nc);
-    } else {                // B: fixed queries vs moving targets
-        item -= a.itemsA;
-        const int ts = item % a.tsplitsB, qt = item / a.tsplitsB;
-        nn_scan_item<QT>(s, Rf, a.Nr, qt * (NN_THREADS * QT), V, a.Nc, ts * NN_SPAN, 0, nullptr, &T,
-                         a.packedB + (size_t)scan * a.Nr);
+    if (nc_len == nullptr) {
+        if (item < a.itemsA) {  // A: moving queries vs fixed targets
+            const int ts = item % a.tsplitsA, qt = item / a.tsplitsA;
+            nn_scan_item<QT>(s, V, a.Nc, qt * (NN_THREADS * QT), Rf, a.Nr, ts * NN_SPAN, 0, &T, nullptr,
+                             a.packedA + (size_t)scan * a.Nc);
+        } else {                // B: fixed queries vs moving targets
+            item -= a.itemsA;
+            const int ts = item % a.tsplitsB, qt = item / a.tsplitsB;
+            nn_scan_item<QT>(s, Rf, a.Nr, qt * (NN_THREADS * QT), V, a.Nc, ts * NN_SPAN, 0, nullptr, &T,
+                             a.packedB + (size_t)scan * a.Nr);
+        }
+    } else {
+        // ragged batch: the grid is sized by the strides, so an item whose query tile or target span lies wholly in the
+        // cloud's padding skips the scan -- with no target it would still publish (+inf, out-of-cloud index) -- and only
+        // takes its ticket
+        const int nc = cloud_len(nc_len, cloud, a.Nc), nr = cloud_len(nr_len, cloud, a.Nr);
+        if (item < a.itemsA) {
+            const int ts = item % a.tsplitsA, qt = item / a.tsplitsA;
+            if (qt * (NN_THREADS * QT) < nc && ts * NN_SPAN < nr)
+                nn_scan_item<QT>(s, V, nc, qt * (NN_THREADS * QT), Rf, nr, ts * NN_SPAN, 0, &T, nullptr,
+                                 a.packedA + (size_t)scan * a.Nc);
+        } else {
+            item -= a.itemsA;
+            const int ts = item % a.tsplitsB, qt = item / a.tsplitsB;
+            if (qt * (NN_THREADS * QT) < nr && ts * NN_SPAN < nc)
+                nn_scan_item<QT>(s, Rf, nr, qt * (NN_THREADS * QT), V, nc, ts * NN_SPAN, 0, nullptr, &T,
+                                 a.packedB + (size_t)scan * a.Nr);
+        }
     }
     // ---- ticket: the last CTA of this scan reduces loss + gradient and steps the optimiser ----
     __threadfence();
@@ -221,7 +266,8 @@ __global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) register_step_kernel
     __syncthreads();
     if (is_last) {
         __threadfence();
-        finalize_scan(a, scan, T, sh, adam_step_from_args(a));
+        if (nc_len == nullptr) finalize_scan(a, scan, T, sh, adam_step_from_args(a));
+        else finalize_scan(cloud_args(a, nc_len, nr_len, scan, cloud), scan, T, sh, adam_step_from_args(a));
     }
 }
 
@@ -569,17 +615,21 @@ extern "C" int genpc_register_launches_per_iter(int S, int Nc, int Nr) {
     return register_prune_eligible(S, Nc, Nr) ? 5 : 2;
 }
 
-extern "C" int genpc_register_run(const float *complete, const float *center, const float *ref, float *params,
-                                  float *adam_m, float *adam_v, float *loss_hist, int S, int n_starts, int Nc, int Nr,
-                                  int iters, int t_start, int T, double lr_rot, double lr_trans, double lr_scale,
-                                  float w_fwd, float w_inv, float cd_weight, void *workspace, size_t workspace_bytes,
-                                  int reset_workspace, genpc_stream_t stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
+// Both entry points.  nc_len / nr_len (device, [C]): points of each cloud for a ragged batch, nullptr for an equal-size one.
+// A ragged batch always takes register_step_kernel, one launch per iteration: the persistent, symmetric and pruned kernels
+// have no per-cloud sizes (carrying them in the persistent kernel raised its register allocation and cost the equal-size
+// small registrations up to 1 us per iteration).
+static int register_run(const float *complete, const float *center, const float *ref, const int *nc_len, const int *nr_len,
+                        float *params, float *adam_m, float *adam_v, float *loss_hist, int S, int n_starts, int Nc, int Nr,
+                        int iters, int t_start, int T, double lr_rot, double lr_trans, double lr_scale, float w_fwd,
+                        float w_inv, float cd_weight, void *workspace, size_t workspace_bytes, int reset_workspace,
+                        cudaStream_t stream) {
     if (S <= 0 || n_starts <= 0 || S % n_starts != 0 || Nc <= 0 || Nr <= 0 || iters < 0 || t_start < 0) return GENPC_ERR_SHAPE;
     if (loss_hist != nullptr && t_start + iters > T) return GENPC_ERR_SHAPE;
     const int C = S / n_starts;
     if (workspace == nullptr || workspace_bytes < register_layout(S, C, Nc, Nr, false).bytes) return GENPC_ERR_WORKSPACE;
-    const bool sym = register_takes_sym_path(S, Nc, Nr);
+    const bool ragged = nc_len != nullptr;
+    const bool sym = !ragged && register_takes_sym_path(S, Nc, Nr);
     const bool prune = sym && register_prune_eligible(S, Nc, Nr) && workspace_bytes >= register_layout(S, C, Nc, Nr, true).bytes;
     const RegWs w = register_layout(S, C, Nc, Nr, prune, workspace);
     RegArgs a = w.args;
@@ -629,7 +679,7 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
         if (e != cudaSuccess) return (int)e;
     }
     // ---- small problems: one cooperative launch runs all the iterations (register_persistent_kernel) ----
-    if (!sym && iters > 1) {
+    if (!sym && !ragged && iters > 1) {
         const char *pk = tunable("GENPC_REGISTER_PERSIST");
         int dev = 0, sms = 0, per_sm = 0;
         cudaGetDevice(&dev);
@@ -717,11 +767,32 @@ extern "C" int genpc_register_run(const float *complete, const float *center, co
             continue;
         }
         switch (QT) {
-            case 4: register_step_kernel<4><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a); break;
-            case 2: register_step_kernel<2><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a); break;
-            default: register_step_kernel<1><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a); break;
+            case 4: register_step_kernel<4><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a, nc_len, nr_len); break;
+            case 2: register_step_kernel<2><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a, nc_len, nr_len); break;
+            default: register_step_kernel<1><<<(unsigned)grid, NN_THREADS, 0, stream>>>(a, nc_len, nr_len); break;
         }
         GENPC_CHECK_LAUNCH();
     }
     return GENPC_OK;
+}
+
+extern "C" int genpc_register_run(const float *complete, const float *center, const float *ref, float *params,
+                                  float *adam_m, float *adam_v, float *loss_hist, int S, int n_starts, int Nc, int Nr,
+                                  int iters, int t_start, int T, double lr_rot, double lr_trans, double lr_scale,
+                                  float w_fwd, float w_inv, float cd_weight, void *workspace, size_t workspace_bytes,
+                                  int reset_workspace, genpc_stream_t stream) {
+    return register_run(complete, center, ref, nullptr, nullptr, params, adam_m, adam_v, loss_hist, S, n_starts, Nc, Nr, iters,
+                        t_start, T, lr_rot, lr_trans, lr_scale, w_fwd, w_inv, cd_weight, workspace, workspace_bytes,
+                        reset_workspace, (cudaStream_t)stream);
+}
+
+extern "C" int genpc_register_run_ragged(const float *complete, const float *center, const float *ref, const int *complete_len,
+                                         const int *ref_len, float *params, float *adam_m, float *adam_v, float *loss_hist,
+                                         int S, int n_starts, int Nc, int Nr, int iters, int t_start, int T, double lr_rot,
+                                         double lr_trans, double lr_scale, float w_fwd, float w_inv, float cd_weight,
+                                         void *workspace, size_t workspace_bytes, int reset_workspace, genpc_stream_t stream) {
+    if (complete_len == nullptr || ref_len == nullptr) return GENPC_ERR_SHAPE;
+    return register_run(complete, center, ref, complete_len, ref_len, params, adam_m, adam_v, loss_hist, S, n_starts, Nc, Nr,
+                        iters, t_start, T, lr_rot, lr_trans, lr_scale, w_fwd, w_inv, cd_weight, workspace, workspace_bytes,
+                        reset_workspace, (cudaStream_t)stream);
 }

@@ -94,22 +94,63 @@ class ObjectPoseOptim(nn.Module):
         return None, R_obj, scale
 
 
+def pad_clouds(clouds):
+    """List of [n_i,3] tensors -> (zero-padded [C, max n_i, 3] float32 tensor, lengths [C] int32), on the first cloud's device."""
+    if len(clouds) == 0:
+        raise ValueError("pad_clouds: no clouds")
+    clouds = [torch.as_tensor(c) for c in clouds]
+    for c in clouds:
+        if c.dim() != 2 or c.shape[1] != 3 or c.shape[0] < 1:
+            raise ValueError(f"pad_clouds: every cloud must be [n,3] with n >= 1, got {tuple(c.shape)}")
+    dev = clouds[0].device
+    lengths = torch.tensor([c.shape[0] for c in clouds], dtype=torch.int32)
+    out = torch.zeros(len(clouds), int(lengths.max()), 3, dtype=torch.float32, device=dev)
+    for i, c in enumerate(clouds):
+        out[i, :c.shape[0]] = c.to(device=dev, dtype=torch.float32)
+    return out, lengths.to(dev)
+
+
+def cloud_centers(complete, lengths=None):
+    """Centroid of every moving cloud [C,3] (register_buffer('center'), :362): over its own `lengths[i]` points when given.
+    Each is the same reduction as a cloud of that size alone ([1,n,3].mean(1)), so a pair of a ragged batch and its solo
+    run start from the same centre."""
+    if lengths is None:
+        return complete.mean(1).contiguous()
+    ln = [int(v) for v in lengths.cpu()]
+    return torch.stack([complete[i:i + 1, :n].mean(1)[0] for i, n in enumerate(ln)]).contiguous()
+
+
 class RegistrationBatch:
     """S = C * n_starts independent pose optimisations advanced by one fused kernel launch per iteration.
 
     complete [C,Nc,3] (moving, e.g. generated shape), partial [C,Nr,3] (fixed scan), float32 CUDA tensors.
     Multi-start k of every cloud pair begins at Ry(k*90 deg) (:518-523), trans 0, scale 0.75 (:367-369).
+
+    Ragged batch: complete_lengths / partial_lengths (int tensors [C], either may be omitted = full stride) give each
+    pair's point counts; its points are the first rows of its stride and the rest is padding that is never read.  Each
+    pair's loss is the mean over its own points and its centre the mean of its own moving points, so its trajectory is
+    the one it has alone (partial sums in another order: within float rounding).  A ragged batch always runs one fused
+    launch per iteration (register_step_kernel, csrc/register.cu): not the persistent kernel a small equal-size batch
+    takes, nor the symmetric path that is faster above S*Nc*Nr ~ 2e8.  from_clouds() builds one from lists of clouds.
     """
 
-    def __init__(self, complete, partial, n_starts=4, lr=0.01, w_fwd=1.0, w_inv=0.5, cd_weight=3.0, max_iters=501):
+    def __init__(self, complete, partial, n_starts=4, lr=0.01, w_fwd=1.0, w_inv=0.5, cd_weight=3.0, max_iters=501,
+                 complete_lengths=None, partial_lengths=None):
         _lib.require_cuda(complete, partial)
         self.complete = complete.contiguous().float()
         self.partial = partial.contiguous().float()
         C, self.Nc, _ = self.complete.shape
         self.Nr = self.partial.shape[1]
+        if self.partial.shape[0] != C:
+            raise ValueError(f"RegistrationBatch: {C} moving clouds but {self.partial.shape[0]} fixed ones")
         dev = self.complete.device
         self.device, self.C, self.n_starts, self.S = dev, C, n_starts, C * n_starts
-        self.center = self.complete.mean(1).contiguous()
+        self.ragged = complete_lengths is not None or partial_lengths is not None
+        self.complete_lengths = self.partial_lengths = None
+        if self.ragged:
+            self.complete_lengths = self._lengths(complete_lengths, self.Nc, "complete_lengths")
+            self.partial_lengths = self._lengths(partial_lengths, self.Nr, "partial_lengths")
+        self.center = cloud_centers(self.complete, self.complete_lengths)
         p = torch.zeros(self.S, 10, device=dev)
         for k in range(n_starts):
             p[k::n_starts, :6] = get_init_rot("y", k * 90, dev)
@@ -125,18 +166,46 @@ class RegistrationBatch:
         self._ws = torch.empty(n, dtype=torch.uint8, device=dev)
         self._ws_bytes = n
 
+    def _lengths(self, lengths, stride, name):
+        """Host-side check of a per-pair point count tensor -> int32 [C] on the batch's device (None: every pair fills the stride)."""
+        if lengths is None:
+            return torch.full((self.C,), stride, dtype=torch.int32, device=self.device)
+        ln = torch.as_tensor(lengths)
+        if ln.dtype.is_floating_point or ln.dtype.is_complex or ln.dtype == torch.bool:
+            raise TypeError(f"RegistrationBatch: {name} must be an integer tensor, got {ln.dtype}")
+        if tuple(ln.shape) != (self.C,):
+            raise ValueError(f"RegistrationBatch: {name} must have shape ({self.C},), got {tuple(ln.shape)}")
+        host = ln.cpu()
+        if bool((host < 1).any()) or bool((host > stride).any()):
+            raise ValueError(f"RegistrationBatch: {name} must lie in [1, {stride}], got {host.tolist()}")
+        return host.to(dtype=torch.int32, device=self.device).contiguous()
+
+    @classmethod
+    def from_clouds(cls, completes, partials, **kw):
+        """Ragged batch from lists of [n_i,3] moving and [m_i,3] fixed clouds: zero-padded to the largest of each, with
+        their point counts (pad_clouds).  Keyword arguments as for the constructor."""
+        if len(completes) != len(partials):
+            raise ValueError(f"from_clouds: {len(completes)} moving clouds but {len(partials)} fixed ones")
+        complete, nc = pad_clouds(completes)
+        partial, nr = pad_clouds(partials)
+        return cls(complete, partial.to(complete.device), complete_lengths=nc, partial_lengths=nr, **kw)
+
     def run(self, iters):
         """Enqueue `iters` Adam iterations on the current stream (no synchronisation)."""
         if self.t + iters > self.T:
             raise _lib.GenpcError("RegistrationBatch: max_iters exceeded")
+        common = (self.S, self.n_starts, self.Nc, self.Nr, int(iters), self.t, self.T, float(self.lr),
+                  float(self.lr * 0.2), float(self.lr * 0.1), float(self.w_fwd), float(self.w_inv), float(self.cd_weight),
+                  _lib.ptr(self._ws), self._ws_bytes, 1 if self.t == 0 else 0, _lib.current_stream(self.device))
+        state = (_lib.ptr(self.params), _lib.ptr(self.adam_m), _lib.ptr(self.adam_v), _lib.ptr(self.loss_hist))
+        clouds = (_lib.ptr(self.complete), _lib.ptr(self.center), _lib.ptr(self.partial))
         with torch.cuda.device(self.device):
-            rc = _lib.lib().genpc_register_run(
-                _lib.ptr(self.complete), _lib.ptr(self.center), _lib.ptr(self.partial), _lib.ptr(self.params),
-                _lib.ptr(self.adam_m), _lib.ptr(self.adam_v), _lib.ptr(self.loss_hist), self.S, self.n_starts,
-                self.Nc, self.Nr, int(iters), self.t, self.T, float(self.lr), float(self.lr * 0.2),
-                float(self.lr * 0.1), float(self.w_fwd), float(self.w_inv), float(self.cd_weight),
-                _lib.ptr(self._ws), self._ws_bytes, 1 if self.t == 0 else 0, _lib.current_stream(self.device))
-        _lib.check(rc, "genpc_register_run")
+            if self.ragged:
+                rc = _lib.lib().genpc_register_run_ragged(*clouds, _lib.ptr(self.complete_lengths),
+                                                          _lib.ptr(self.partial_lengths), *state, *common)
+            else:
+                rc = _lib.lib().genpc_register_run(*clouds, *state, *common)
+        _lib.check(rc, "genpc_register_run_ragged" if self.ragged else "genpc_register_run")
         self.t += iters
         return self
 
@@ -161,10 +230,15 @@ class RegistrationBatch:
         return T
 
     def transformed(self, params=None):
-        """pts = R(s(V-c))+c+t for every scan (torch ops; for inspection, not the hot path)."""
+        """pts = R(s(V-c))+c+t for every scan (torch ops; for inspection, not the hot path).  For a ragged batch the clouds
+        keep their padded stride: rows at or past a pair's length are meaningless."""
         p = self.params if params is None else params
-        V = self.complete.repeat_interleave(self.n_starts, 0) if p.shape[0] == self.S else self.complete
-        c = V.mean(1, keepdim=True)
+        per_scan = p.shape[0] == self.S
+        V = self.complete.repeat_interleave(self.n_starts, 0) if per_scan else self.complete
+        if self.ragged:
+            c = (self.center.repeat_interleave(self.n_starts, 0) if per_scan else self.center)[:, None]
+        else:
+            c = V.mean(1, keepdim=True)
         R = rotation_6d_to_matrix(p[:, :6])
         local = (V - c) * torch.exp(p[:, 9])[:, None, None]
         return torch.einsum("sij,snj->sni", R, local) + c + p[:, None, 6:9]
@@ -179,6 +253,18 @@ def object_pose_optimization_points(complete_xyz, partial_xyz, lr=0.005, iters=3
     rb = RegistrationBatch(c, p, n_starts=cam_bias_num, lr=lr, max_iters=iters + 1)
     rb.run(iters + 1)
     return rb.transforms()[0].detach().cpu().numpy()
+
+
+def object_pose_optimization_points_batch(completes, partials, lr=0.005, iters=300, cam_bias_num=4, device=None):
+    """object_pose_optimization_points for many cloud pairs of any sizes in one ragged batch (lists of [n_i,3] moving and
+    [m_i,3] fixed clouds): every pair runs its own 4 multi-starts x (iters+1) Adam steps, exactly as alone up to float
+    rounding.  -> numpy [C,4,4], the transform of each pair's best start."""
+    device = device or torch.device("cuda:0")
+    cs = [torch.as_tensor(c, dtype=torch.float32, device=device) for c in completes]
+    ps = [torch.as_tensor(p, dtype=torch.float32, device=device) for p in partials]
+    rb = RegistrationBatch.from_clouds(cs, ps, n_starts=cam_bias_num, lr=lr, max_iters=iters + 1)
+    rb.run(iters + 1)
+    return rb.transforms().detach().cpu().numpy()
 
 
 def load_point_cloud(point_path, device, radius=0.05, num_points=5000, seed=0):

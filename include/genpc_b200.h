@@ -295,6 +295,21 @@ int genpc_register_run(const float *complete, const float *center, const float *
                        int iters, int t_start, int T, double lr_rot, double lr_trans, double lr_scale,
                        float w_fwd, float w_inv, float cd_weight, void *workspace, size_t workspace_bytes,
                        int reset_workspace, genpc_stream_t stream);
+/* Ragged batch: the same loop for cloud pairs of different sizes in one call.  Arguments are those of
+ * genpc_register_run plus complete_len / ref_len (device int32 [C], never NULL): pair c has complete_len[c] moving
+ * and ref_len[c] fixed points, stored at the start of its Nc / Nr stride; Nc / Nr are the padded strides and size
+ * everything else (workspace: genpc_register_workspace_bytes(S,Nc,Nr)).  Each pair's loss is the mean over its own
+ * points, so its trajectory is the one it has alone (up to the order of the partial sums); rows past a length are
+ * never read (any value, NaN included).  Lengths are clamped to [1, Nc] / [1, Nr] on the device.  A ragged call always
+ * runs one fused launch per iteration, at every size and whatever GENPC_REGISTER_MODE / GENPC_REGISTER_PERSIST say: the
+ * persistent (all iterations in one launch), symmetric and pruned forms are not used, so a small ragged batch costs
+ * the per-iteration launch chain and above S*Nc*Nr ~ 2e8 it is slower than an equal-size call.  Never synchronises; GENPC_ERR_SHAPE for a NULL
+ * length pointer and for the shape errors of genpc_register_run. */
+int genpc_register_run_ragged(const float *complete, const float *center, const float *ref, const int *complete_len,
+                              const int *ref_len, float *params, float *adam_m, float *adam_v, float *loss_hist,
+                              int S, int n_starts, int Nc, int Nr, int iters, int t_start, int T, double lr_rot,
+                              double lr_trans, double lr_scale, float w_fwd, float w_inv, float cd_weight,
+                              void *workspace, size_t workspace_bytes, int reset_workspace, genpc_stream_t stream);
 
 #ifdef __cplusplus
 }
