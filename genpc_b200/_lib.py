@@ -47,6 +47,10 @@ _SIGNATURES = {
                                            ctypes.POINTER(ChamferFuse), _vp]),
     "genpc_chamfer_forward_host_fused": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp,
                                                 _sz, ctypes.POINTER(ChamferFuse), _vp]),
+    "genpc_chamfer_forward_ragged": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _vp, _sz,
+                                            ctypes.POINTER(ChamferFuse), _vp]),
+    "genpc_chamfer_loss_backward_ragged": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _flt, _flt, _vp, _vp,
+                                                  _int, _int, _int, _vp]),
     "genpc_chamfer_backward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _vp]),
     "genpc_chamfer_loss_workspace_bytes": (_sz, []),
     "genpc_chamfer_loss": (_int, [_vp, _vp, _sz, _sz, _int, _flt, _flt, _vp, _vp, _sz, _vp]),

@@ -6,6 +6,10 @@
 Same argument order, caller-allocated outputs written in place, return 1 on success (the reference
 returns 1 / 0 and prints, chamfer3D.cu:145-151); failures raise instead of being silently ignored.
 Work is enqueued on the CURRENT torch stream (the reference uses the legacy default stream).
+
+Ragged batches (forward_ragged, no reference counterpart): pair b has len1[b] points at the start of its N-stride in xyz1 and
+len2[b] at the start of its M-stride in xyz2 (genpc_chamfer_forward_ragged); rows past a length are never read and get
+dist 0 / idx -1.  `lengths` checks such an argument.
 """
 import torch
 
@@ -17,7 +21,37 @@ def _chk(t, dtype, name):
         raise _lib.GenpcError(f"{name} must be a contiguous {dtype} tensor")
 
 
+def lengths(xyz1, xyz2, len1=None, len2=None):
+    """Per-pair point counts of a ragged batch -> (len1, len2) as contiguous int32 [B] tensors on the clouds' device, or None
+    when both are None (an equal-size batch).  An omitted side means every cloud of it fills its stride.  Shape, device and
+    dtype are checked here; the values are clamped to [0, stride] on the device (no host synchronisation)."""
+    if len1 is None and len2 is None:
+        return None
+    B = xyz1.shape[0]
+    out = []
+    for ln, xyz, name in ((len1, xyz1, "len1"), (len2, xyz2, "len2")):
+        if ln is None:
+            out.append(torch.full((B,), xyz.shape[1], dtype=torch.int32, device=xyz.device))
+            continue
+        if not isinstance(ln, torch.Tensor):
+            raise _lib.GenpcError(f"{name} must be a tensor")
+        if ln.dtype.is_floating_point or ln.dtype.is_complex or ln.dtype == torch.bool:
+            raise _lib.GenpcError(f"{name} must be an integer tensor, got {ln.dtype}")
+        if tuple(ln.shape) != (B,):
+            raise _lib.GenpcError(f"{name} must have shape ({B},), got {tuple(ln.shape)}")
+        if ln.device != xyz.device:
+            raise _lib.GenpcError(f"{name} is on {ln.device}, the clouds on {xyz.device}")
+        out.append(ln.to(torch.int32).contiguous())
+    return tuple(out)
+
+
 def forward(xyz1, xyz2, dist1, dist2, idx1, idx2):
+    return forward_ragged(xyz1, xyz2, dist1, dist2, idx1, idx2)
+
+
+def forward_ragged(xyz1, xyz2, dist1, dist2, idx1, idx2, len1=None, len2=None):
+    """`forward` for a ragged batch (len1 / len2: see `lengths`; both None: exactly `forward`).  A separate name keeps
+    `forward`'s parameters the reference's."""
     _lib.require_cuda(xyz1, xyz2, dist1, dist2, idx1, idx2)
     for t, n in ((xyz1, "xyz1"), (xyz2, "xyz2"), (dist1, "dist1"), (dist2, "dist2")):
         _chk(t, torch.float32, n)
@@ -25,14 +59,20 @@ def forward(xyz1, xyz2, dist1, dist2, idx1, idx2):
         _chk(t, torch.int32, n)
     B, N, _ = xyz1.shape
     M = xyz2.shape[1]
+    lens = lengths(xyz1, xyz2, len1, len2)
     L = _lib.lib()
     with torch.cuda.device(xyz1.device):
         nbytes = L.genpc_chamfer_workspace_bytes(B, N, M)
         ws = torch.empty(max(nbytes, 8), dtype=torch.uint8, device=xyz1.device)
-        rc = L.genpc_chamfer_forward(_lib.ptr(xyz1), _lib.ptr(xyz2), _lib.ptr(dist1), _lib.ptr(dist2),
-                                     _lib.ptr(idx1), _lib.ptr(idx2), B, N, M, _lib.ptr(ws), nbytes,
-                                     _lib.current_stream(xyz1.device))
-    _lib.check(rc, "genpc_chamfer_forward")
+        stream = _lib.current_stream(xyz1.device)
+        if lens is None:
+            rc = L.genpc_chamfer_forward(_lib.ptr(xyz1), _lib.ptr(xyz2), _lib.ptr(dist1), _lib.ptr(dist2),
+                                         _lib.ptr(idx1), _lib.ptr(idx2), B, N, M, _lib.ptr(ws), nbytes, stream)
+        else:
+            rc = L.genpc_chamfer_forward_ragged(_lib.ptr(xyz1), _lib.ptr(xyz2), _lib.ptr(lens[0]), _lib.ptr(lens[1]),
+                                                _lib.ptr(dist1), _lib.ptr(dist2), _lib.ptr(idx1), _lib.ptr(idx2), B, N, M,
+                                                _lib.ptr(ws), nbytes, None, stream)
+    _lib.check(rc, "genpc_chamfer_forward" if lens is None else "genpc_chamfer_forward_ragged")
     return 1
 
 
@@ -65,11 +105,12 @@ def step_workspace(device, B, N, M):
 
 
 def forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, zero1=None, zero2=None, loss=None, h_xyz1=None, h_xyz2=None,
-                  chunks=6):
+                  chunks=6, lengths=None):
     """No pybind counterpart: `forward` through genpc_chamfer_forward_fused on a cached, re-armed workspace (no memset
     after the first call of a shape).  zero1 / zero2: optional tensors the epilogue zero-fills (the gradient
     accumulators `backward` adds into); loss = (out_scalar, use_sqrt, w1, w2): optional fused loss reduction;
-    h_xyz1 / h_xyz2: host-fed form (see forward_host)."""
+    h_xyz1 / h_xyz2: host-fed form (see forward_host); lengths = (len1, len2) as returned by `lengths()`: ragged batch
+    (genpc_chamfer_forward_ragged, per-pair means in the loss), sharing the cached workspace with equal-size calls."""
     _lib.require_cuda(xyz1, xyz2, dist1, dist2, idx1, idx2)
     for t, n in ((xyz1, "xyz1"), (xyz2, "xyz2"), (dist1, "dist1"), (dist2, "dist2")):
         _chk(t, torch.float32, n)
@@ -87,7 +128,14 @@ def forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, zero1=None, zero2=None, 
                                 zero2.data_ptr() if zero2 is not None else None)
         ws.armed = False   # stays False if the call below fails half-way
         stream = _lib.current_stream(dev)
-        if h_xyz1 is None:
+        if lengths is not None:
+            if h_xyz1 is not None:
+                raise _lib.GenpcError("ragged batches have no host-fed form")
+            rc = L.genpc_chamfer_forward_ragged(_lib.ptr(xyz1), _lib.ptr(xyz2), _lib.ptr(lengths[0]), _lib.ptr(lengths[1]),
+                                                _lib.ptr(dist1), _lib.ptr(dist2), _lib.ptr(idx1), _lib.ptr(idx2), B, N, M,
+                                                _lib.ptr(ws.packed), ws.packed_bytes, fuse, stream)
+            _lib.check(rc, "genpc_chamfer_forward_ragged")
+        elif h_xyz1 is None:
             rc = L.genpc_chamfer_forward_fused(_lib.ptr(xyz1), _lib.ptr(xyz2), _lib.ptr(dist1), _lib.ptr(dist2), _lib.ptr(idx1),
                                                _lib.ptr(idx2), B, N, M, _lib.ptr(ws.packed), ws.packed_bytes, fuse, stream)
             _lib.check(rc, "genpc_chamfer_forward_fused")
@@ -100,7 +148,8 @@ def forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, zero1=None, zero2=None, 
                                                     _lib.ptr(idx2), B, N, M, int(chunks), _lib.ptr(ws.packed), ws.packed_bytes,
                                                     fuse, stream)
             _lib.check(rc, "genpc_chamfer_forward_host_fused")
-        ws.armed = (max(N, M) >= 512 and min(N, M) > 0)   # the symmetric path re-arms the packed words
+        # the symmetric path re-arms the packed words; a ragged call takes it whenever there is a word
+        ws.armed = min(N, M) > 0 and (lengths is not None or max(N, M) >= 512)
     return 1
 
 

@@ -131,17 +131,23 @@ __device__ __forceinline__ void scatter_aggregated(float *go, bool valid, size_t
 // LOSS = true : backward of the fused loss -- graddist = upstream[0] * w / n (* 0.5 / sqrt(d) for the L1 forms, inf at d == 0
 //               exactly as torch's sqrt backward, loss_util.py:37); gd1 / gd2 are the forward's distances; w2 == 0 drops the
 //               second direction.
+// len1 / len2 (LOSS only; nullptr: full strides): points of each cloud of a ragged batch -- the mean of pair b's side runs over
+// len[b] points, so graddist = upstream[0] * w / (B * len[b]); rows past a length and neighbours past the other cloud's length
+// contribute nothing (genpc_chamfer_loss_backward_ragged).
 template <bool VEC, bool LOSS>
 __global__ void __launch_bounds__(256) chamfer_grad_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2,
                                                           const float *__restrict__ gd1, const float *__restrict__ gd2,
                                                           const int *__restrict__ idx1, const int *__restrict__ idx2,
                                                           const float *__restrict__ upstream, int use_sqrt, float w1, float w2,
-                                                          float *gx1, float *gx2, int B, int N, int M) {
+                                                          float *gx1, float *gx2, int B, int N, int M,
+                                                          const int *__restrict__ len1 = nullptr,
+                                                          const int *__restrict__ len2 = nullptr) {
     const size_t n1 = (size_t)B * N, n2 = (LOSS && w2 == 0.f) ? 0 : (size_t)B * M;
     const size_t nthreads = (size_t)gridDim.x * blockDim.x, g0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     bool valid[GRAD_R];
     int dir[GRAD_R], nn[GRAD_R];
+    int lown[GRAD_R], loth[GRAD_R];   // ragged batch: points of the row's own cloud and of the other one
     size_t i[GRAD_R], t[GRAD_R];
     float x1[GRAD_R], y1[GRAD_R], z1[GRAD_R], gsc[GRAD_R], tx[GRAD_R], ty[GRAD_R], tz[GRAD_R];
     const float up = LOSS ? __ldg(upstream) : 0.f;
@@ -151,7 +157,12 @@ __global__ void __launch_bounds__(256) chamfer_grad_kernel(const float *__restri
         valid[r] = i[r] < n1 + n2;
         dir[r] = (valid[r] && i[r] >= n1) ? 1 : 0;
         if (dir[r]) i[r] -= n1;
-        nn[r] = 0, x1[r] = y1[r] = z1[r] = gsc[r] = 0.f;
+        nn[r] = 0, x1[r] = y1[r] = z1[r] = gsc[r] = 0.f, lown[r] = loth[r] = 0;
+        if (LOSS && len1 != nullptr && valid[r]) {   // ragged batch: a padding row is never read
+            const int na = dir[r] ? M : N, b = (int)(i[r] / na);
+            lown[r] = sym_len(dir[r] ? len2 : len1, b, na), loth[r] = sym_len(dir[r] ? len1 : len2, b, dir[r] ? N : M);
+            valid[r] = (int)(i[r] - (size_t)b * na) < lown[r];
+        }
         if (valid[r]) {
             const float *a = dir[r] ? xyz2 : xyz1;
             nn[r] = __ldg((dir[r] ? idx2 : idx1) + i[r]);
@@ -164,6 +175,7 @@ __global__ void __launch_bounds__(256) chamfer_grad_kernel(const float *__restri
         const int no = dir[r] ? N : M, na = dir[r] ? M : N;
         // an index outside [0, no) (caller-supplied garbage) contributes nothing instead of touching foreign memory
         valid[r] = valid[r] && (unsigned)nn[r] < (unsigned)no;
+        if (LOSS && len1 != nullptr) valid[r] = valid[r] && nn[r] < loth[r];
         t[r] = 0, tx[r] = ty[r] = tz[r] = 0.f;
         if (valid[r]) {
             const float *o = dir[r] ? xyz1 : xyz2;
@@ -171,7 +183,8 @@ __global__ void __launch_bounds__(256) chamfer_grad_kernel(const float *__restri
             const float x2 = __ldg(o + t[r] * 3), y2 = __ldg(o + t[r] * 3 + 1), z2 = __ldg(o + t[r] * 3 + 2);
             float gd = gsc[r];
             if (LOSS) {
-                gd = __fmul_rn(up, __fdiv_rn(dir[r] ? w2 : w1, (float)(dir[r] ? (size_t)B * M : n1)));
+                const size_t cnt = len1 != nullptr ? (size_t)B * lown[r] : (dir[r] ? (size_t)B * M : n1);
+                gd = __fmul_rn(up, __fdiv_rn(dir[r] ? w2 : w1, (float)cnt));
                 if (use_sqrt) gd = __fmul_rn(gd, __fdiv_rn(0.5f, __fsqrt_rn(gsc[r])));
             }
             const float g = __fmul_rn(gd, 2.f);
@@ -408,14 +421,17 @@ static size_t fuse_layout(int B, int N, int M, void *base, EpiFuse &f) {
 
 // Symmetric path: rows = the larger cloud (registers), cols = the smaller one (shared-memory sweep).
 // gate != nullptr: host-fed launch (nn_sym_gated_kernel), see genpc_chamfer_forward_host.
+// len1 / len2 != nullptr: ragged batch (genpc_chamfer_forward_ragged; w laid out for kind 0, no gate).
 static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist1, float *dist2, int *idx1, int *idx2,
                                int B, int N, int M, const ChamferWs &w, cudaStream_t stream,
                                const unsigned *gate = nullptr, unsigned gate_gen = 0, int gate_pairs = 1,
-                               const genpc_chamfer_fuse_t *fuse = nullptr, const int *prune_chunks = nullptr) {
+                               const genpc_chamfer_fuse_t *fuse = nullptr, const int *prune_chunks = nullptr,
+                               const int *len1 = nullptr, const int *len2 = nullptr) {
     const bool swap = M > N;
     SymParams p = {};
     p.rows = swap ? xyz2 : xyz1, p.cols = swap ? xyz1 : xyz2;
     p.nr = swap ? M : N, p.nc = swap ? N : M;
+    p.len_r = swap ? len2 : len1, p.len_c = swap ? len1 : len2;
     float *dist_r = swap ? dist2 : dist1, *dist_c = swap ? dist1 : dist2;
     int *idx_r = swap ? idx2 : idx1, *idx_c = swap ? idx1 : idx2;
     p.prow = w.packed, p.pcol = w.packed + (size_t)B * p.nr;
@@ -504,7 +520,9 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     // launch between the pruned scan and the epilogue.  When the fall-back does run (out-of-range, far-apart or collapsed clouds)
     // C2-sized batches pay the balanced form's 4-5 % (above) -- inputs already off the fast path.  Behind the Hilbert-sorted
     // pruned scan it is also a programmatic dependent (launch_pdl): of nn_prune_kernel, or of the join with the cooperative kernel
-    const bool balanced = (bm == nullptr) ? ((GENPC_DEFAULT_BALANCED && few_items) || use_prune) : (atoi(bm) != 0);
+    // A ragged batch always takes the item grid (nn_sym_kernel): the balanced form has no per-cloud lengths (SymParams)
+    const bool balanced = p.len_r == nullptr &&
+                          ((bm == nullptr) ? ((GENPC_DEFAULT_BALANCED && few_items) || use_prune) : (atoi(bm) != 0));
     const bool dep = w.kind == 1;
     cudaError_t es = cudaSuccess;
     if (gate != nullptr) {
@@ -533,15 +551,18 @@ static int chamfer_forward_sym(const float *xyz1, const float *xyz2, float *dist
     memset(&f, 0, sizeof(f));
     // column words are exact iff the pruned scan did the work (ctl[1] == 0)
     f.select = use_prune ? ctl + 1 : nullptr;
+    f.len_r = p.len_r, f.len_c = p.len_c;
     // the epilogue is a programmatic dependent of the scan launched above (whichever it is: every one of them triggers early)
     const dim3 egrid(fix_blocks + unpack_blocks);
     if (fuse == nullptr) {
         es = launch_pdl(nn_sym_epilogue_kernel<false>, egrid, dim3(256), stream, p.rows, p.cols, p.prow, p.pcol, B, p.nr, p.nc, 32 * QT,
                         fix_blocks, dist_r, idx_r, dist_c, idx_c, f);
     } else {
-        // dist1 belongs to xyz1: the row cloud unless the clouds were swapped
-        const double f1 = (fuse->w1 != 0.f) ? (double)fuse->w1 / (double)((size_t)B * N) : 0.0;
-        const double f2 = (fuse->w2 != 0.f) ? (double)fuse->w2 / (double)((size_t)B * M) : 0.0;
+        // dist1 belongs to xyz1: the row cloud unless the clouds were swapped; a ragged batch divides each term by its pair's
+        // length in the epilogue, the 1 / B here
+        const bool ragged = len1 != nullptr;
+        const double f1 = (fuse->w1 != 0.f) ? (double)fuse->w1 / (double)(ragged ? (size_t)B : (size_t)B * N) : 0.0;
+        const double f2 = (fuse->w2 != 0.f) ? (double)fuse->w2 / (double)(ragged ? (size_t)B : (size_t)B * M) : 0.0;
         f.frow = swap ? f2 : f1, f.fcol = swap ? f1 : f2;
         f.use_sqrt = fuse->use_sqrt, f.rearm = 1;
         if (fuse->loss_out != nullptr) fuse_layout(B, N, M, fuse->loss_workspace, f), f.loss_out = fuse->loss_out;
@@ -666,6 +687,41 @@ extern "C" int genpc_chamfer_forward(const float *xyz1, const float *xyz2, float
                                      size_t workspace_bytes, genpc_stream_t stream_) {
     return genpc_chamfer_forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, workspace, workspace_bytes, nullptr,
                                        stream_);
+}
+
+// Ragged batch: pair b has len1[b] / len2[b] points at the start of its N / M stride (clamped to [0, stride] on the device); rows
+// past a length are never read and get dist 0 / idx -1, like every row of a pair whose other cloud is empty.  Always the
+// exhaustive symmetric scan, at every size: the per-direction, pruned, grid and host-fed scans have no per-cloud counts.
+extern "C" int genpc_chamfer_forward_ragged(const float *xyz1, const float *xyz2, const int *len1, const int *len2, float *dist1,
+                                            float *dist2, int *idx1, int *idx2, int B, int N, int M, void *workspace,
+                                            size_t workspace_bytes, const genpc_chamfer_fuse_t *fuse, genpc_stream_t stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (len1 == nullptr || len2 == nullptr || B < 0 || N < 0 || M < 0) return GENPC_ERR_SHAPE;
+    int rc = fuse_check(fuse, B, N, M);
+    if (rc != GENPC_OK) return rc;
+    const size_t n1 = (size_t)B * N, n2 = (size_t)B * M;
+    cudaError_t e = cudaSuccess;
+    if (n1 == 0 || n2 == 0) {
+        // every pair has an empty side: no row has a neighbour, and the loss (a mean of zeros, or of nothing) is 0
+        if (n1 && e == cudaSuccess) e = cudaMemsetAsync(dist1, 0, n1 * 4, stream);
+        if (n1 && e == cudaSuccess) e = cudaMemsetAsync(idx1, 0xff, n1 * 4, stream);
+        if (n2 && e == cudaSuccess) e = cudaMemsetAsync(dist2, 0, n2 * 4, stream);
+        if (n2 && e == cudaSuccess) e = cudaMemsetAsync(idx2, 0xff, n2 * 4, stream);
+        if (e != cudaSuccess) return (int)e;
+        return fuse ? fuse_tail_unfused(fuse, dist1, dist2, B, N, M, stream) : GENPC_OK;
+    }
+    const int nr = N > M ? N : M, nc = N > M ? M : N;
+    if (workspace == nullptr || workspace_bytes < chamfer_layout(B, nr, nc, 0).bytes) return GENPC_ERR_WORKSPACE;
+    // chamfer_forward_sym's range check of its item grid, before anything is queued
+    int rtiles = 0, span = 0, cspans = 0;
+    if (sym_tiling(B, nr, nc, nr >= 1024 ? 4 : 2, rtiles, span, cspans) > 0x7fffffffLL) return GENPC_ERR_RANGE;
+    const ChamferWs w = chamfer_layout(B, nr, nc, 0, workspace);
+    if (!(fuse != nullptr && fuse->workspace_armed)) {  // (the fused epilogue re-arms every word, padding rows' included)
+        e = cudaMemsetAsync(w.packed, 0xff, (n1 + n2) * 8, stream);
+        if (e == cudaSuccess) e = cudaMemsetAsync(w.ctl, 0, 16, stream);
+        if (e != cudaSuccess) return (int)e;
+    }
+    return chamfer_forward_sym(xyz1, xyz2, dist1, dist2, idx1, idx2, B, N, M, w, stream, nullptr, 0, 1, fuse, nullptr, len1, len2);
 }
 
 extern "C" int genpc_chamfer_backward(const float *xyz1, const float *xyz2, const float *graddist1,
@@ -1066,11 +1122,10 @@ extern "C" int genpc_chamfer_loss(const float *dist1, const float *dist2, size_t
     return GENPC_OK;
 }
 
-extern "C" int genpc_chamfer_loss_backward(const float *xyz1, const float *xyz2, const float *dist1, const float *dist2,
-                                           const int *idx1, const int *idx2, const float *upstream, int use_sqrt,
-                                           float w1, float w2, float *gradxyz1, float *gradxyz2, int B, int N, int M,
-                                           genpc_stream_t stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
+// Both loss backward entries; len1 / len2: a ragged batch's lengths, nullptr for an equal-size one.
+static int loss_backward(const float *xyz1, const float *xyz2, const int *len1, const int *len2, const float *dist1,
+                         const float *dist2, const int *idx1, const int *idx2, const float *upstream, int use_sqrt, float w1,
+                         float w2, float *gradxyz1, float *gradxyz2, int B, int N, int M, cudaStream_t stream) {
     if (B < 0 || N < 0 || M < 0) return GENPC_ERR_SHAPE;
     if (N == 0 || M == 0 || B == 0) return GENPC_OK;
     const size_t tot = (size_t)B * N + ((w2 != 0.f) ? (size_t)B * M : 0);
@@ -1078,10 +1133,27 @@ extern "C" int genpc_chamfer_loss_backward(const float *xyz1, const float *xyz2,
     const unsigned grid = (unsigned)((tot + 256 * GRAD_R - 1) / (256 * GRAD_R));
     if (vec)
         chamfer_grad_kernel<true, true><<<grid, 256, 0, stream>>>(xyz1, xyz2, dist1, dist2, idx1, idx2, upstream, use_sqrt, w1, w2,
-                                                                 gradxyz1, gradxyz2, B, N, M);
+                                                                 gradxyz1, gradxyz2, B, N, M, len1, len2);
     else
         chamfer_grad_kernel<false, true><<<grid, 256, 0, stream>>>(xyz1, xyz2, dist1, dist2, idx1, idx2, upstream, use_sqrt, w1, w2,
-                                                                  gradxyz1, gradxyz2, B, N, M);
+                                                                  gradxyz1, gradxyz2, B, N, M, len1, len2);
     GENPC_CHECK_LAUNCH();
     return GENPC_OK;
+}
+
+extern "C" int genpc_chamfer_loss_backward(const float *xyz1, const float *xyz2, const float *dist1, const float *dist2,
+                                           const int *idx1, const int *idx2, const float *upstream, int use_sqrt,
+                                           float w1, float w2, float *gradxyz1, float *gradxyz2, int B, int N, int M,
+                                           genpc_stream_t stream) {
+    return loss_backward(xyz1, xyz2, nullptr, nullptr, dist1, dist2, idx1, idx2, upstream, use_sqrt, w1, w2, gradxyz1, gradxyz2, B,
+                         N, M, (cudaStream_t)stream);
+}
+
+extern "C" int genpc_chamfer_loss_backward_ragged(const float *xyz1, const float *xyz2, const int *len1, const int *len2,
+                                                  const float *dist1, const float *dist2, const int *idx1, const int *idx2,
+                                                  const float *upstream, int use_sqrt, float w1, float w2, float *gradxyz1,
+                                                  float *gradxyz2, int B, int N, int M, genpc_stream_t stream) {
+    if (len1 == nullptr || len2 == nullptr) return GENPC_ERR_SHAPE;
+    return loss_backward(xyz1, xyz2, len1, len2, dist1, dist2, idx1, idx2, upstream, use_sqrt, w1, w2, gradxyz1, gradxyz2, B, N,
+                         M, (cudaStream_t)stream);
 }

@@ -41,7 +41,17 @@ struct SymParams {
     // selection flag of the pruned scans (nn_prune.cuh, nn_grid.cuh): when set, this launch only runs if *select != 0, i.e.
     // the sort's range check or the grid probe handed the work back to the exhaustive kernels; nullptr: always run
     const int *select;
+    // ragged batches (genpc_chamfer_forward_ragged): points of each row / column cloud [B], the rest of its nr / nc stride is
+    // padding that is never read; nullptr: every cloud fills its stride
+    // (nn_sym_kernel only: the balanced form cuts its units by the strides, not by the real work, and carrying the row length
+    // into it cost it 12-16 more bytes of spills)
+    const int *len_r, *len_c;
 };
+
+// points of cloud b of a ragged batch, clamped to [0, stride] so that no index leaves the cloud whatever a caller passes
+__device__ __forceinline__ int sym_len(const int *len, int b, int stride) {
+    return len == nullptr ? stride : min(max(__ldg(len + b), 0), stride);
+}
 
 // Work items of the symmetric scan over B cloud pairs: row tiles of SYM_THREADS * QT rows x column spans, the span the largest
 // that still gives >= 2 waves of work items (3 CTAs x SMs), at least 256 columns.  Returns B * rtiles * cspans.
@@ -64,11 +74,16 @@ __device__ __forceinline__ float ld_coord(const float *p) {
 // One work item: row tile `rt` (SYM_THREADS*QT rows) x column span [c0, c0+span) of ONE cloud pair.
 // rows/cols/prow/pcol point at the first element of the pair's clouds / packed words.  colT: optional similarity
 // applied to the columns while they are staged (registration: the moving cloud), nullptr = identity.
+// nr_pub >= nr >= 1 (ragged batch: nr is the row cloud's length, nr_pub its stride): rows [nr, nr_pub) are not read -- they
+// hold NaN like the rows past the cloud, so they never win a column -- but publish into their own (padding) packed words, which
+// nobody reads and the fused epilogue re-arms.  (Bounding the loads themselves by the length, or the publishing, cost
+// nn_sym_kernel<4> 12 more bytes of spills: ptxas -v.)
 template <int QT, bool COHERENT = false>
 __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const float *__restrict__ rows, int nr, int rt,
                                             const float *__restrict__ cols, int nc, int c0, int span,
                                             const Similarity *colT, unsigned long long *__restrict__ prow_,
-                                            unsigned long long *__restrict__ pcol_, int rblock_base = 0) {
+                                            unsigned long long *__restrict__ pcol_, int rblock_base = 0, int nr_pub = -1) {
+    if (nr_pub < 0) nr_pub = nr;
     static_assert(QT % 2 == 0, "rows are folded in pairs");
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cnt = min(span, nc - c0);
@@ -95,9 +110,12 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
     for (int qi = 0; qi < QT; ++qi) {
         const int j = jbase + qi * 32;
         float x = qnan, y = qnan, z = qnan;
-        if (j < nr)
-            x = ld_coord<COHERENT>(rp + (size_t)j * 3), y = ld_coord<COHERENT>(rp + (size_t)j * 3 + 1),
-            z = ld_coord<COHERENT>(rp + (size_t)j * 3 + 2);
+        if (j < nr_pub) {   // (rows [nr, nr_pub): a real row is loaded and replaced by NaN -- see above)
+            const int jr = min(j, nr - 1);
+            x = ld_coord<COHERENT>(rp + (size_t)jr * 3), y = ld_coord<COHERENT>(rp + (size_t)jr * 3 + 1),
+            z = ld_coord<COHERENT>(rp + (size_t)jr * 3 + 2);
+            if (j >= nr) x = y = z = qnan;
+        }
         nqx[qi] = make_float2(-x, -x);
         nqy[qi] = make_float2(-y, -y);
         nqz[qi] = make_float2(-z, -z);
@@ -172,7 +190,7 @@ __device__ __forceinline__ void nn_sym_item(float (*s)[SYM_SPAN_MAX], const floa
 #pragma unroll
     for (int qi = 0; qi < QT; ++qi) {
         const int j = jbase + qi * 32;
-        if (j >= nr) continue;
+        if (j >= nr_pub) continue;
         // every in-range row publishes, also when its minimum stayed +inf (NaN / overflowing coordinates: the re-scan finds
         // no match and reports the first column of the span, like nn_scan_item) -- no packed word is ever left unarmed
         const float qx = -nqx[qi].x, qy = -nqy[qi].x, qz = -nqz[qi].x;
@@ -198,8 +216,12 @@ __global__ void __launch_bounds__(SYM_THREADS, 2) nn_sym_kernel(const SymParams 
     item /= p.cspans;
     const int rt = item % p.rtiles;
     const int b = item / p.rtiles;
-    nn_sym_item<QT>(s, p.rows + (size_t)b * p.nr * 3, p.nr, rt, p.cols + (size_t)b * p.nc * 3, p.nc, cs * p.span, p.span,
-                    nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base);
+    // a ragged batch's grid is sized by the strides: an item whose row tile or column span lies wholly in the pair's padding
+    // has nothing to do (CTA-uniform)
+    const int nr = sym_len(p.len_r, b, p.nr), nc = sym_len(p.len_c, b, p.nc);
+    if (rt * (SYM_THREADS * QT) >= nr || cs * p.span >= nc) return;
+    nn_sym_item<QT>(s, p.rows + (size_t)b * p.nr * 3, nr, rt, p.cols + (size_t)b * p.nc * 3, nc, cs * p.span, p.span,
+                    nullptr, p.prow + (size_t)b * p.nr, p.pcol + (size_t)b * p.nc, p.rblock_base, p.nr);
 }
 
 // Host-fed form: same work items, but the clouds are still arriving from pinned host memory while the kernel runs.
@@ -349,13 +371,17 @@ struct EpiFuse {
     double *partial;        // one slot per epilogue CTA; nullptr: no loss
     unsigned *ticket;       // zero between launches (re-armed by the last CTA)
     float *loss_out;        // device scalar
-    double fcol, frow;      // loss = fcol * sum_cols f(d) + frow * sum_rows f(d)   (w / count; 0 drops the side)
+    double fcol, frow;      // loss = fcol * sum_cols f(d) + frow * sum_rows f(d)   (w / count; 0 drops the side);
+                            // ragged batch: each term is f(d) / len[b] and fcol / frow are w / B
     int use_sqrt;           // f = sqrt or identity
     int rearm;              // store all-ones back into every packed word after reading it
     float *zero[2];         // buffers to zero-fill, or nullptr
     size_t nzero[2];        // their sizes in floats
     const unsigned *err_flag;  // host-fed launches: the feed's error word -- a timed-out gate poisons the loss with NaN
     const int *select;         // selection flag of the pruned scans: *select == 0 -> the column words already hold exact indices
+    // ragged batch (SymParams::len_r / len_c; nullptr: full strides): a row or column past its cloud's length, or of a pair whose
+    // other cloud is empty, has no neighbour -- it gets dist 0, idx -1 and no loss term; the fix-up stops at the row length
+    const int *len_r, *len_c;
 };
 
 __device__ __forceinline__ void epi_zero_fill(float *z, size_t n, size_t g, size_t total_threads) {
@@ -399,56 +425,106 @@ static __global__ void __launch_bounds__(256) nn_sym_epilogue_kernel(const float
     if (blockIdx.x >= fix_blocks) {
         const size_t n = (size_t)B * nr;
         const size_t i0 = (size_t)(blockIdx.x - fix_blocks) * EPI_ROWS_PER_CTA + threadIdx.x;
-        unsigned long long w[EPI_RPT];
-#pragma unroll
-        for (int k = 0; k < EPI_RPT; ++k) {
-            const size_t i = i0 + (size_t)k * 256;
-            w[k] = (i < n) ? __ldcg(prow + i) : 0ull;
-        }
-#pragma unroll
-        for (int k = 0; k < EPI_RPT; ++k) {
-            const size_t i = i0 + (size_t)k * 256;
-            if (i < n) {
-                const float d = __uint_as_float((unsigned)(w[k] >> 32));
+        if (f.len_r != nullptr) {
+            // ragged batch, one row at a time (a division per row in the unrolled form below raised the registers of every
+            // epilogue launch from 32 / 47 to 64): a row past its cloud's length, or of a pair whose column cloud is empty, has no
+            // neighbour; the loss term of a row is f(d) / (its cloud's length)
+#pragma unroll 1
+            for (int k = 0; k < EPI_RPT; ++k) {
+                const size_t i = i0 + (size_t)k * 256;
+                if (i >= n) break;
+                const int b = (int)(i / (size_t)nr), len = sym_len(f.len_r, b, nr);
+                const bool has_nn = (int)(i - (size_t)b * nr) < len && sym_len(f.len_c, b, nc) > 0;
+                const unsigned long long w = __ldcg(prow + i);
+                const float d = has_nn ? __uint_as_float((unsigned)(w >> 32)) : 0.f;
                 dist_r[i] = d;
-                idx_r[i] = (int)(unsigned)(w[k] & 0xffffffffu);
+                idx_r[i] = has_nn ? (int)(unsigned)(w & 0xffffffffu) : -1;
                 if (FUSED) {
                     if (f.rearm) prow[i] = ~0ull;
-                    term += (double)(f.use_sqrt ? __fsqrt_rn(d) : d);
+                    if (has_nn) term += (double)(f.use_sqrt ? __fsqrt_rn(d) : d) / (double)len;
+                }
+            }
+        } else {
+            unsigned long long w[EPI_RPT];
+#pragma unroll
+            for (int k = 0; k < EPI_RPT; ++k) {
+                const size_t i = i0 + (size_t)k * 256;
+                w[k] = (i < n) ? __ldcg(prow + i) : 0ull;
+            }
+#pragma unroll
+            for (int k = 0; k < EPI_RPT; ++k) {
+                const size_t i = i0 + (size_t)k * 256;
+                if (i < n) {
+                    const float d = __uint_as_float((unsigned)(w[k] >> 32));
+                    dist_r[i] = d;
+                    idx_r[i] = (int)(unsigned)(w[k] & 0xffffffffu);
+                    if (FUSED) {
+                        if (f.rearm) prow[i] = ~0ull;
+                        term += (double)(f.use_sqrt ? __fsqrt_rn(d) : d);
+                    }
                 }
             }
         }
     } else {
         const size_t n = (size_t)B * nc;
         const size_t w0 = ((size_t)blockIdx.x * 8 + warp) * EPI_CPW;  // first column of this warp
-        const size_t mine = w0 + (lane % EPI_CPW);
-        unsigned long long my_w = 0ull;
-        float mx = 0.f, my = 0.f, mz = 0.f;
-        size_t my_base = 0;
-        if (mine < n) {
-            my_w = __ldcg(pcol + mine);
-            mx = __ldg(cols + mine * 3), my = __ldg(cols + mine * 3 + 1), mz = __ldg(cols + mine * 3 + 2);
-            my_base = (mine / nc) * (size_t)nr * 3;
-        }
-        int my_found = 0;
+        if (f.len_r != nullptr) {
+            // ragged batch, one column at a time for the same reason: a column past its cloud's length, or of a pair whose row
+            // cloud is empty, has no neighbour (and is never read); the fix-up reads the row cloud up to its length only, and the
+            // loss term of a column is f(d) / (its cloud's length)
+#pragma unroll 1
+            for (int k = 0; k < EPI_CPW; ++k) {
+                const size_t c = w0 + k;
+                if (c >= n) break;  // warp-uniform
+                const int b = (int)(c / nc), len = sym_len(f.len_c, b, nc);
+                const int rows_b = (int)(c - (size_t)b * nc) < len ? sym_len(f.len_r, b, nr) : 0;   // warp-uniform
+                const unsigned long long word = __ldcg(pcol + c);
+                float d = 0.f;
+                int found = -1;
+                if (rows_b > 0) {
+                    d = __uint_as_float((unsigned)(word >> 32));
+                    found = sym_fix_column(rows + (size_t)b * nr * 3, rows_b, rows_per_block, __ldg(cols + c * 3), __ldg(cols + c * 3 + 1),
+                                           __ldg(cols + c * 3 + 2), d, (int)(unsigned)(word & 0xffffffffu), lane);
+                }
+                if (lane == 0) {
+                    dist_c[c] = d;
+                    idx_c[c] = found;
+                    if (FUSED) {
+                        if (f.rearm) pcol[c] = ~0ull;
+                        if (rows_b > 0) term += (double)(f.use_sqrt ? __fsqrt_rn(d) : d) / (double)len;
+                    }
+                }
+            }
+        } else {
+            const size_t mine = w0 + (lane % EPI_CPW);
+            unsigned long long my_w = 0ull;
+            float mx = 0.f, my = 0.f, mz = 0.f;
+            size_t my_base = 0;
+            if (mine < n) {
+                my_w = __ldcg(pcol + mine);
+                mx = __ldg(cols + mine * 3), my = __ldg(cols + mine * 3 + 1), mz = __ldg(cols + mine * 3 + 2);
+                my_base = (mine / nc) * (size_t)nr * 3;
+            }
+            int my_found = 0;
 #pragma unroll
-        for (int k = 0; k < EPI_CPW; ++k) {
-            if (w0 + k >= n) break;  // warp-uniform
-            const unsigned long long word = __shfl_sync(0xffffffffu, my_w, k);
-            const float cx = __shfl_sync(0xffffffffu, mx, k), cy = __shfl_sync(0xffffffffu, my, k), cz = __shfl_sync(0xffffffffu, mz, k);
-            const size_t base = __shfl_sync(0xffffffffu, my_base, k);
-            const int found = cols_exact ? (int)(unsigned)(word & 0xffffffffu)
-                                         : sym_fix_column(rows + base, nr, rows_per_block, cx, cy, cz,
-                                                          __uint_as_float((unsigned)(word >> 32)), (int)(unsigned)(word & 0xffffffffu), lane);
-            if (lane == k) my_found = found;
-        }
-        if (lane < EPI_CPW && mine < n) {
-            const float d = __uint_as_float((unsigned)(my_w >> 32));
-            dist_c[mine] = d;
-            idx_c[mine] = my_found;
-            if (FUSED) {
-                if (f.rearm) pcol[mine] = ~0ull;
-                term = (double)(f.use_sqrt ? __fsqrt_rn(d) : d);
+            for (int k = 0; k < EPI_CPW; ++k) {
+                if (w0 + k >= n) break;  // warp-uniform
+                const unsigned long long word = __shfl_sync(0xffffffffu, my_w, k);
+                const float cx = __shfl_sync(0xffffffffu, mx, k), cy = __shfl_sync(0xffffffffu, my, k), cz = __shfl_sync(0xffffffffu, mz, k);
+                const size_t base = __shfl_sync(0xffffffffu, my_base, k);
+                const int found = cols_exact ? (int)(unsigned)(word & 0xffffffffu)
+                                             : sym_fix_column(rows + base, nr, rows_per_block, cx, cy, cz,
+                                                              __uint_as_float((unsigned)(word >> 32)), (int)(unsigned)(word & 0xffffffffu), lane);
+                if (lane == k) my_found = found;
+            }
+            if (lane < EPI_CPW && mine < n) {
+                const float d = __uint_as_float((unsigned)(my_w >> 32));
+                dist_c[mine] = d;
+                idx_c[mine] = my_found;
+                if (FUSED) {
+                    if (f.rearm) pcol[mine] = ~0ull;
+                    term = (double)(f.use_sqrt ? __fsqrt_rn(d) : d);
+                }
             }
         }
     }

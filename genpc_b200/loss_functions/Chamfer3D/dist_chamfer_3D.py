@@ -1,6 +1,7 @@
 """Chamfer distance module -- drop-in for the reference's loss_functions/Chamfer3D/dist_chamfer_3D.py (:26-74).
 
     dist1, dist2, idx1, idx2 = chamfer_3DDist()(input1, input2)        # [B,N,3], [B,M,3] CUDA tensors
+    dist1, dist2, idx1, idx2 = chamfer_3DDist()(input1, input2, lengths1, lengths2)   # ragged batch
 
 dist1[b,j] = min_k |input1[b,j] - input2[b,k]|^2 with idx1 the arg-min (lowest index on ties), dist2/idx2 the other
 direction; differentiable w.r.t. both inputs.  GPU tensors only, exactly like the reference (:25) -- a CPU tensor
@@ -9,6 +10,12 @@ raises instead of silently falling back.
 What differs from the reference is only where memory lives: outputs and gradients are created on the inputs' device
 (the reference allocates them on the CPU and copies them over on every call, :33-42 and :56-60), the kernels write
 every output element so no zero-fill is needed, and launches go to the current stream.
+
+Ragged batch (no reference counterpart): lengths1 / lengths2, integer tensors [B] on the inputs' device (either may be
+omitted = full stride), give each pair's point counts; pair b's points are the first rows of its stride and the rest is
+padding that is never read.  Valid rows are what the pair alone gives, bit for bit; rows with no neighbour (padding, or a
+pair whose other cloud is empty) get dist 0 and idx -1 and receive no gradient.  Lists of clouds: pad them with
+genpc_b200.optim_registration.diff_obj_pose.pad_clouds, which returns the padded batch and its lengths.
 """
 import torch
 from torch import nn
@@ -33,11 +40,12 @@ def _grad_buffers(ctx, xyz1, xyz2):
 
 class chamfer_3DFunction(Function):
     @staticmethod
-    def forward(ctx, xyz1, xyz2):
+    def forward(ctx, xyz1, xyz2, len1=None, len2=None):
         dist1, idx1 = _outputs(xyz1, xyz1.shape[1])
         dist2, idx2 = _outputs(xyz2, xyz2.shape[1])
         ctx.grads = _grad_buffers(ctx, xyz1, xyz2)
-        chamfer_3D.forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, ctx.grads[0], ctx.grads[1])
+        lengths = None if len1 is None else (len1, len2)
+        chamfer_3D.forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, ctx.grads[0], ctx.grads[1], lengths=lengths)
         ctx.save_for_backward(xyz1, xyz2, idx1, idx2)
         ctx.mark_non_differentiable(idx1, idx2)
         return dist1, dist2, idx1, idx2
@@ -52,7 +60,7 @@ class chamfer_3DFunction(Function):
         if grads[0] is None:
             grads = torch.zeros_like(xyz1), torch.zeros_like(xyz2)
         chamfer_3D.backward(xyz1, xyz2, grads[0], grads[1], graddist1.contiguous(), graddist2.contiguous(), idx1, idx2)
-        return grads
+        return grads + (None, None)
 
 
 class chamfer_3DHostFunction(Function):
@@ -71,7 +79,7 @@ class chamfer_3DHostFunction(Function):
 
     @staticmethod
     def backward(ctx, graddist1, graddist2, gradidx1, gradidx2):
-        return chamfer_3DFunction.backward(ctx, graddist1, graddist2, gradidx1, gradidx2) + (None, None, None)
+        return chamfer_3DFunction.backward(ctx, graddist1, graddist2, gradidx1, gradidx2)[:2] + (None, None, None)
 
 
 def host_leaves(h1, h2, device=None):
@@ -82,8 +90,10 @@ def host_leaves(h1, h2, device=None):
 
 
 class chamfer_3DDist(nn.Module):
-    def forward(self, input1, input2):
-        return chamfer_3DFunction.apply(input1.contiguous(), input2.contiguous())
+    def forward(self, input1, input2, lengths1=None, lengths2=None):
+        a, b = input1.contiguous(), input2.contiguous()
+        lens = chamfer_3D.lengths(a, b, lengths1, lengths2)
+        return chamfer_3DFunction.apply(a, b, *(lens if lens is not None else (None, None)))
 
     def forward_from_host(self, input1, input2, device=None, chunks=6):
         """`forward` for CPU (pinned) inputs -- the reference's `chamfer(x.cuda(), y.cuda())` with the host-to-device

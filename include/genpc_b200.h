@@ -123,6 +123,33 @@ int genpc_chamfer_forward_host_fused(genpc_host_feed_t *feed, const float *h_xyz
                                      int chunks, void *workspace, size_t workspace_bytes,
                                      const genpc_chamfer_fuse_t *fuse, genpc_stream_t stream);
 
+/* Ragged batch: Chamfer distances (and, through `fuse`, the loss step) of cloud pairs of different sizes in one call.
+ * len1 / len2 are device int32 [B] arrays, never NULL: pair b has len1[b] points at the start of its N-stride in xyz1 and
+ * len2[b] at the start of its M-stride in xyz2; the device clamps them to [0, N] / [0, M] (0 is allowed).  Rows past a length
+ * are never read (any value, NaN included).  For j < len1[b], dist1[b,j] / idx1[b,j] are bit for bit what
+ * genpc_chamfer_forward returns for that pair alone on the sliced clouds (lowest index on ties); the same for dist2 / idx2.  A
+ * row with no neighbour to report -- a padding row, or any row of a pair whose other cloud is empty -- gets dist 0 and idx -1,
+ * so the gradient kernels give it zero gradient.  Fused loss: loss_out[0] = (1/B) sum_b [w1 mean_{j<len1[b]} f(dist1) +
+ * w2 mean_{k<len2[b]} f(dist2)], a side with no points contributing 0 (lengths at the strides: the equal-size loss up to
+ * summation order); zero-fill and re-arming as genpc_chamfer_forward_fused (every packed word, padding rows' included, so a fused
+ * call leaves the workspace armed for the next call of either kind).  Workspaces: genpc_chamfer_workspace_bytes(B,N,M) and
+ * genpc_chamfer_fuse_workspace_bytes(B,N,M).  A ragged call always runs the exhaustive symmetric scan, at every size: not the
+ * per-direction scan of small clouds, nor the pruned scans (so a ragged batch of >= 2^30 evaluations with >= 2048 points per
+ * cloud runs at the exhaustive rate, slower than an equal-size call), nor a host-fed launch.  GENPC_ERR_SHAPE for a NULL length
+ * pointer or negative sizes, GENPC_ERR_WORKSPACE for a missing or too small workspace, GENPC_ERR_RANGE as the plain entry; all
+ * before anything is queued.
+ * genpc_chamfer_loss_backward_ragged is genpc_chamfer_loss_backward for the fused ragged loss: graddist = upstream[0] * w /
+ * (B * len[b]) (* 0.5 / sqrt(dist) for f = sqrt); rows past a length contribute nothing.  The gradient of dist1 / dist2 of a
+ * ragged forward goes through genpc_chamfer_backward unchanged (rows with idx -1 contribute nothing). */
+int genpc_chamfer_forward_ragged(const float *xyz1, const float *xyz2, const int *len1, const int *len2, float *dist1,
+                                 float *dist2, int *idx1, int *idx2, int B, int N, int M, void *workspace,
+                                 size_t workspace_bytes, const genpc_chamfer_fuse_t *fuse /* NULL: plain forward */,
+                                 genpc_stream_t stream);
+int genpc_chamfer_loss_backward_ragged(const float *xyz1, const float *xyz2, const int *len1, const int *len2,
+                                       const float *dist1, const float *dist2, const int *idx1, const int *idx2,
+                                       const float *upstream, int use_sqrt, float w1, float w2, float *gradxyz1,
+                                       float *gradxyz2, int B, int N, int M, genpc_stream_t stream);
+
 /* Replaces chamfer_3D.backward (chamfer_cuda.cpp:22-27 -> chamfer_cuda_backward, chamfer3D.cu:176-195,
  * kernel NmDistanceGradKernel :155-174).  ACCUMULATES into gradxyz1/gradxyz2, which must arrive zeroed
  * exactly as in the reference (dist_chamfer_3D.py:56-57). */
