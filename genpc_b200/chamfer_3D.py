@@ -77,8 +77,10 @@ def forward_ragged(xyz1, xyz2, dist1, dist2, idx1, idx2, len1=None, len2=None):
 
 
 class _StepWorkspace:
-    """Scratch of one forward shape on one (device, stream): the packed-word workspace, which the fused epilogue leaves
-    re-armed (all-ones) so that the next call skips the memset, and the loss partials + ticket (zeroed once)."""
+    """Scratch of one forward shape on one (device, stream): the packed-word workspace, which every successful fused call
+    leaves re-armed (all-ones) so that the next call skips the memset, and the loss partials + tickets (zeroed once).  The
+    cache below drops an entry when it is full or when a knob changes the size; a CUDA graph captured on an entry bakes its
+    pointers in, so the graph's owner keeps a reference (GraphedLossStep.workspace)."""
 
     def __init__(self, device, B, N, M):
         L = _lib.lib()
@@ -91,8 +93,17 @@ class _StepWorkspace:
 _step_ws = {}
 
 
+def _step_key(device, B, N, M):
+    return (device.index, torch.cuda.current_stream(device).cuda_stream, B, N, M)
+
+
+def cached_step_workspace(device, B, N, M):
+    """The cached workspace of this shape on the current stream of `device`, or None (nothing is created)."""
+    return _step_ws.get(_step_key(device, B, N, M))
+
+
 def step_workspace(device, B, N, M):
-    key = (device.index, torch.cuda.current_stream(device).cuda_stream, B, N, M)
+    key = _step_key(device, B, N, M)
     ws = _step_ws.get(key)
     if ws is not None and ws.packed_bytes != _lib.lib().genpc_chamfer_workspace_bytes(B, N, M):
         ws = None   # the size depends on the scan the library would pick now (a knob was flipped): start over, unarmed
@@ -107,7 +118,8 @@ def step_workspace(device, B, N, M):
 def forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, zero1=None, zero2=None, loss=None, h_xyz1=None, h_xyz2=None,
                   chunks=6, lengths=None):
     """No pybind counterpart: `forward` through genpc_chamfer_forward_fused on a cached, re-armed workspace (no memset
-    after the first call of a shape).  zero1 / zero2: optional tensors the epilogue zero-fills (the gradient
+    after the first call of a shape).  Whether the packed words are armed is the library's rule, not the caller's guess:
+    after a successful fused call they are, on every path it may take.  zero1 / zero2: optional tensors the epilogue zero-fills (the gradient
     accumulators `backward` adds into); loss = (out_scalar, use_sqrt, w1, w2): optional fused loss reduction;
     h_xyz1 / h_xyz2: host-fed form (see forward_host); lengths = (len1, len2) as returned by `lengths()`: ragged batch
     (genpc_chamfer_forward_ragged, per-pair means in the loss), sharing the cached workspace with equal-size calls."""
@@ -148,8 +160,9 @@ def forward_fused(xyz1, xyz2, dist1, dist2, idx1, idx2, zero1=None, zero2=None, 
                                                     _lib.ptr(idx2), B, N, M, int(chunks), _lib.ptr(ws.packed), ws.packed_bytes,
                                                     fuse, stream)
             _lib.check(rc, "genpc_chamfer_forward_host_fused")
-        # the symmetric path re-arms the packed words; a ragged call takes it whenever there is a word
-        ws.armed = min(N, M) > 0 and (lengths is not None or max(N, M) >= 512)
+        # every fused call that reaches the scan leaves the packed words all-ones, whichever path the library took (symmetric,
+        # pruned, per-direction, host-fed, ragged); an empty cloud leaves them untouched
+        ws.armed = min(N, M) > 0
     return 1
 
 

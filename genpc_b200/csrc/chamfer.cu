@@ -65,12 +65,15 @@ __global__ void __launch_bounds__(NN_THREADS, NN_MINBLOCKS) nn_scan_kernel(const
                      idx_base, nullptr, nullptr, out + (size_t)b * nq);
 }
 
-__global__ void nn_unpack_kernel(const unsigned long long *__restrict__ packed, float *__restrict__ dist1,
+// rearm: store all-ones back into every word after reading it, as the fused symmetric epilogue does (a fused call on the
+// per-direction path leaves the workspace armed too)
+__global__ void nn_unpack_kernel(unsigned long long *__restrict__ packed, float *__restrict__ dist1,
                                  int *__restrict__ idx1, size_t n1, float *__restrict__ dist2,
-                                 int *__restrict__ idx2, size_t n2) {
+                                 int *__restrict__ idx2, size_t n2, int rearm) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n1 + n2) return;
     const unsigned long long w = packed[i];
+    if (rearm) packed[i] = ~0ull;
     const float dv = __uint_as_float((unsigned int)(w >> 32));
     const int iv = (int)(unsigned int)(w & 0xffffffffu);
     if (i < n1) {
@@ -593,12 +596,17 @@ static bool takes_sym_path(int N, int M) {
     return want_sym && N > 0 && M > 0 && (N > M ? N : M) >= 512;
 }
 
+// The loss workspace holds the fused epilogue's partials and ticket, then, from the next 16-byte boundary, those of the plain loss
+// kernel (the per-direction path).  Each kernel zeroes only its own ticket, so the two must not overlap: one workspace serves
+// calls of either path in any order (GENPC_CHAMFER_MODE flipped between calls of one shape).
+static size_t plain_loss_offset(int B, int N, int M) {
+    EpiFuse f;
+    return (fuse_layout(B, N, M, nullptr, f) + 15) & ~(size_t)15;
+}
+
 extern "C" size_t genpc_chamfer_fuse_workspace_bytes(int B, int N, int M) {
     if (B < 0 || N < 0 || M < 0) return 0;
-    EpiFuse f;
-    const size_t a = fuse_layout(B, N, M, nullptr, f);
-    const size_t b = genpc_chamfer_loss_workspace_bytes();              // non-symmetric path: the plain loss kernel
-    return a > b ? a : b;
+    return plain_loss_offset(B, N, M) + genpc_chamfer_loss_workspace_bytes();
 }
 
 // The unfused tail of a fused call, for the shapes that do not take the symmetric path (tiny or empty clouds).
@@ -615,8 +623,10 @@ static int fuse_tail_unfused(const genpc_chamfer_fuse_t *fuse, const float *dist
         if (e != cudaSuccess) return (int)e;
     }
     if (fuse->loss_out == nullptr) return GENPC_OK;
-    return genpc_chamfer_loss(dist1, dist2, n1, n2, fuse->use_sqrt, fuse->w1, fuse->w2, fuse->loss_out, fuse->loss_workspace,
-                              fuse->loss_workspace_bytes, (genpc_stream_t)stream);
+    const size_t off = plain_loss_offset(B, N, M);
+    return genpc_chamfer_loss(dist1, dist2, n1, n2, fuse->use_sqrt, fuse->w1, fuse->w2, fuse->loss_out,
+                              static_cast<char *>(fuse->loss_workspace) + off, fuse->loss_workspace_bytes - off,
+                              (genpc_stream_t)stream);
 }
 
 static int fuse_check(const genpc_chamfer_fuse_t *fuse, int B, int N, int M) {
@@ -657,7 +667,8 @@ extern "C" int genpc_chamfer_forward_fused(const float *xyz1, const float *xyz2,
     if (workspace_bytes < chamfer_layout(B, nr, nc, kind).bytes) kind = 0;
     const ChamferWs w = chamfer_layout(B, nr, nc, kind, workspace);
     cudaError_t e;
-    if (!(sym && fuse != nullptr && fuse->workspace_armed)) {  // an armed workspace already holds all-ones words
+    // an armed workspace already holds all-ones words: a fused call on either path leaves them so
+    if (!(fuse != nullptr && fuse->workspace_armed)) {
         e = cudaMemsetAsync(w.packed, 0xff, (n1 + n2) * 8, stream);
         if (e == cudaSuccess) e = cudaMemsetAsync(w.ctl, 0, 16, stream);
         if (e != cudaSuccess) return (int)e;
@@ -677,7 +688,8 @@ extern "C" int genpc_chamfer_forward_fused(const float *xyz1, const float *xyz2,
     }
     GENPC_CHECK_LAUNCH();
     const size_t tot = n1 + n2;
-    nn_unpack_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(w.packed, dist1, idx1, n1, dist2, idx2, n2);
+    nn_unpack_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(w.packed, dist1, idx1, n1, dist2, idx2, n2,
+                                                                        fuse != nullptr ? 1 : 0);
     GENPC_CHECK_LAUNCH();
     return fuse ? fuse_tail_unfused(fuse, dist1, dist2, B, N, M, stream) : GENPC_OK;
 }
@@ -1001,7 +1013,8 @@ extern "C" int genpc_nn_unpack(const unsigned long long *packed, float *dist, in
                                genpc_stream_t stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     if (count == 0) return GENPC_OK;
-    nn_unpack_kernel<<<(unsigned)((count + 255) / 256), 256, 0, stream>>>(packed, dist, idx, count, nullptr, nullptr, 0);
+    nn_unpack_kernel<<<(unsigned)((count + 255) / 256), 256, 0, stream>>>(const_cast<unsigned long long *>(packed), dist, idx,
+                                                                          count, nullptr, nullptr, 0, 0);
     GENPC_CHECK_LAUNCH();
     return GENPC_OK;
 }

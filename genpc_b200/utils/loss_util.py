@@ -200,6 +200,10 @@ class GraphedLossStep:
     `loss`, `ggen`, `ggt` are the SAME tensors on every call (overwritten by the next replay).  Passing no arguments replays on
     the current contents of `step.gen` / `step.gt` (write into them in place to avoid the copy).
 
+    The graph owns the Chamfer workspace it was captured on (`step.workspace`, the cached scratch of this shape on
+    `step.stream`): its pointers are baked into the graph, so the step keeps it alive after the process-wide cache drops it
+    (more shapes than the cache holds, or a knob that changes the workspace size).
+
     Ragged batch: gen_lengths / gt_lengths (as for get_loss) are copied into device tensors `step.gen_lengths` /
     `step.gt_lengths` that the graph reads, so a replay takes new lengths as well as new clouds:
     step(gen_new, gt_new, gen_lengths_new, gt_lengths_new), or write into those tensors in place."""
@@ -226,6 +230,8 @@ class GraphedLossStep:
         with torch.cuda.graph(self.graph, stream=self.stream):
             loss = loss_obj.get_loss(self.gen, self.gt, self.gen_lengths, self.gt_lengths)
             loss.backward()
+        with torch.cuda.stream(self.stream):   # (None for EMD: no Chamfer workspace)
+            self.workspace = chamfer_3D.cached_step_workspace(dev, self.gen.shape[0], self.gen.shape[1], self.gt.shape[1])
         self.loss = loss.detach()
         self.grad_gen, self.grad_gt = self.gen.grad, self.gt.grad
 

@@ -104,7 +104,9 @@ int genpc_chamfer_forward_host(genpc_host_feed_t *feed, const float *h_xyz1, con
  * A loss step is then 3 launches (scan, epilogue, gradient) instead of 7.  dist/idx outputs are unchanged, bit for bit.
  * loss_workspace: genpc_chamfer_fuse_workspace_bytes(B,N,M) bytes, zeroed ONCE by the caller (only read when loss_out
  * is not NULL).  fuse == NULL makes both calls identical to the plain entries.  Shapes that do not take the symmetric
- * path (tiny or empty clouds) run the same duties as separate launches. */
+ * path (tiny or empty clouds, GENPC_CHAMFER_MODE=scan) run the same duties as separate launches, re-arming included: after
+ * any successful fused call with N > 0 and M > 0 the packed words are all-ones, whichever scan ran, and one loss workspace
+ * serves calls of either path in any order. */
 typedef struct genpc_chamfer_fuse {
     int workspace_armed;         /* in: the packed words of `workspace` are all-ones (left so by a previous fused call) */
     int use_sqrt;                /* loss: f = sqrt (chamfer_l1 forms) or identity (chamfer_l2 forms) */
