@@ -12,7 +12,9 @@
 //     Kabsch/SVD with the reflection fix gives, without an SVD;  t = mu_t - R mu_s
 //   T <- [R|t] T for candidates that are active and have >= 3 inliers
 // -- one CTA per candidate, no host synchronisation anywhere in the loop (the torch formulation it replaces needed ~25
-// tiny launches, a batched float64 SVD and one host sync per iteration).
+// tiny launches, a batched float64 SVD and one host sync per iteration).  The ragged form (genpc_icp_step_ragged) gives every
+// candidate its own source / target point counts and also applies T to the untransformed source, so that a batch of
+// differently-sized objects runs one loop.
 #include "common.cuh"
 
 namespace genpc {
@@ -80,41 +82,30 @@ __device__ __forceinline__ void sym4_top_eigenvector(double (&A)[4][4], double (
     for (int k = 0; k < 4; ++k) q[k] /= nrm;
 }
 
-__global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(const float *__restrict__ cur, const float *__restrict__ target,
-                                                               const float *__restrict__ dist, const int *__restrict__ idx,
-                                                               float *T, float *state, int Ns, int Kt, int Nt, float max_dist2,
-                                                               float rel_fitness, float rel_rmse, int update) {
-    __shared__ double sh[ICP_THREADS / 32][ICP_NACC];
-    const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const float *cp = cur + (size_t)k * Ns * 3;
-    const float *tp = target + (size_t)(Kt == 1 ? 0 : k) * Nt * 3;
-    const float *dp = dist + (size_t)k * Ns;
-    const int *ip = idx + (size_t)k * Ns;
-    double acc[ICP_NACC];
+// cur[j] = T source[j] for j < n, one row per thread in turn: c_r = fma(T[r][2], z, fma(T[r][1], y, fma(T[r][0], x, T[r][3])))
+// (DESIGN § 3 item 12), so a candidate's points do not depend on the batch it sits in.  T is read with plain loads: thread 0
+// of the CTA may have just written it.
+__device__ __forceinline__ void icp_transform_rows(const float *Tk, const float *__restrict__ sp, float *cp, int n) {
+    float M[12];
 #pragma unroll
-    for (int i = 0; i < ICP_NACC; ++i) acc[i] = 0.0;
-    for (int j = tid; j < Ns; j += ICP_THREADS) {
-        const float d = __ldg(dp + j);
-        if (!(d < max_dist2)) continue;
-        const int t = __ldg(ip + j);
-        const double sx = __ldg(cp + j * 3), sy = __ldg(cp + j * 3 + 1), sz = __ldg(cp + j * 3 + 2);
-        const double qx = __ldg(tp + (size_t)t * 3), qy = __ldg(tp + (size_t)t * 3 + 1), qz = __ldg(tp + (size_t)t * 3 + 2);
-        acc[0] += 1.0;
-        acc[1] += sx, acc[2] += sy, acc[3] += sz;
-        acc[4] += qx, acc[5] += qy, acc[6] += qz;
-        acc[7] += sx * qx, acc[8] += sx * qy, acc[9] += sx * qz;
-        acc[10] += sy * qx, acc[11] += sy * qy, acc[12] += sy * qz;
-        acc[13] += sz * qx, acc[14] += sz * qy, acc[15] += sz * qz;
-        acc[16] += (double)d;
+    for (int i = 0; i < 12; ++i) M[i] = Tk[i];
+    for (int j = threadIdx.x; j < n; j += ICP_THREADS) {
+        const float x = __ldg(sp + j * 3), y = __ldg(sp + j * 3 + 1), z = __ldg(sp + j * 3 + 2);
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+            cp[j * 3 + r] = fmaf(M[r * 4 + 2], z, fmaf(M[r * 4 + 1], y, fmaf(M[r * 4], x, M[r * 4 + 3])));
     }
-#pragma unroll
-    for (int i = 0; i < ICP_NACC; ++i) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc[i] += __shfl_xor_sync(0xffffffffu, acc[i], o);
-        if (lane == 0) sh[warp][i] = acc[i];
+}
+
+// thread 0: statistics, convergence test and T update of candidate k from the warp partials.  frozen: the candidate entered
+// the call converged (ragged form), read nothing and keeps T, fitness and rmse; only its call counter moves.
+__device__ __forceinline__ void icp_finish(const double (&sh)[ICP_THREADS / 32][ICP_NACC], float *Tk, float *st, int *scan_len,
+                                           int ns, bool frozen, float rel_fitness, float rel_rmse, int update) {
+    if (frozen) {
+        st[3] = st[3] + 1.f;
+        *scan_len = 0;
+        return;
     }
-    __syncthreads();
-    if (tid != 0) return;
     double a[ICP_NACC];
 #pragma unroll
     for (int i = 0; i < ICP_NACC; ++i) {
@@ -123,14 +114,14 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(const float *__re
         for (int w = 0; w < ICP_THREADS / 32; ++w) r += sh[w][i];  // fixed order
         a[i] = r;
     }
-    float *st = state + (size_t)k * 4;  // fitness, rmse, converged, calls
     const double cnt = a[0];
-    const float fitness = (float)(cnt / (double)Ns);
+    const float fitness = (float)(cnt / (double)(ns > 0 ? ns : 1));
     const float rmse = (float)sqrt(a[16] / (cnt > 0.0 ? cnt : 1.0));
     const bool was_converged = st[2] != 0.f;
     bool converged = was_converged;
     if (!was_converged && st[3] > 0.f && fabsf(fitness - st[0]) < rel_fitness && fabsf(rmse - st[1]) < rel_rmse) converged = true;
     st[0] = fitness, st[1] = rmse, st[2] = converged ? 1.f : 0.f, st[3] = st[3] + 1.f;
+    if (scan_len) *scan_len = converged ? 0 : ns;
     if (!update || converged || cnt < 3.0) return;
     // ---- Horn: R from the cross-covariance of the centred inlier pairs ----
     const double ms[3] = {a[1] / cnt, a[2] / cnt, a[3] / cnt}, mq[3] = {a[4] / cnt, a[5] / cnt, a[6] / cnt};
@@ -162,7 +153,6 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(const float *__re
 #pragma unroll
     for (int r = 0; r < 3; ++r) t[r] = mq[r] - (R[r][0] * ms[0] + R[r][1] * ms[1] + R[r][2] * ms[2]);
     // ---- T <- [R|t] T ----
-    float *Tk = T + (size_t)k * 16;
     double Told[4][4], Tnew[3][4];
 #pragma unroll
     for (int r = 0; r < 4; ++r)
@@ -179,6 +169,68 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(const float *__re
         for (int c = 0; c < 4; ++c) Tk[r * 4 + c] = (float)Tnew[r][c];
 }
 
+// One ICP iteration, one CTA per candidate.  Equal-size form (src_len == nullptr, genpc_icp_step): Ns source and Nt target
+// points per candidate, source / tgt_len / scan_len unused.  Ragged form (genpc_icp_step_ragged, DESIGN § 3 item 12):
+// candidate k has ns = clamp(src_len[k], 0, Ns) source and nt = clamp(tgt_len[Kt == 1 ? 0 : k], 0, Nt) target points; the
+// statistics run over j < ns (fitness = inliers / ns), an idx outside [0, nt) is no inlier, a candidate that enters converged
+// reads no dist / idx, and once T is final the CTA writes the next iteration's cur = T source for j < ns.  The write is in
+// place: only this CTA reads these rows, and all of its reads come before the barrier the write follows.  dist == nullptr:
+// transform only (cur and scan_len, state untouched).  A candidate with no points on a side gets no cur row written.
+__global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(float *cur, const float *__restrict__ source,
+                                                               const float *__restrict__ target, const float *__restrict__ dist,
+                                                               const int *__restrict__ idx, const int *__restrict__ src_len,
+                                                               const int *__restrict__ tgt_len, int *scan_len, float *T,
+                                                               float *state, int Ns, int Kt, int Nt, float max_dist2,
+                                                               float rel_fitness, float rel_rmse, int update) {
+    __shared__ double sh[ICP_THREADS / 32][ICP_NACC];
+    const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const bool ragged = src_len != nullptr;
+    const int ns = ragged ? min(max(__ldg(src_len + k), 0), Ns) : Ns;
+    const int nt = ragged ? min(max(__ldg(tgt_len + (Kt == 1 ? 0 : k)), 0), Nt) : Nt;
+    float *st = state + (size_t)k * 4;  // fitness, rmse, converged, calls
+    float *Tk = T + (size_t)k * 16;
+    if (dist == nullptr) {
+        if (tid == 0) scan_len[k] = st[2] != 0.f ? 0 : ns;
+        if (nt > 0) icp_transform_rows(Tk, source + (size_t)k * Ns * 3, cur + (size_t)k * Ns * 3, ns);
+        return;
+    }
+    const bool frozen = ragged && st[2] != 0.f;
+    const int n = (frozen || nt == 0) ? 0 : ns;
+    const float *cp = cur + (size_t)k * Ns * 3;
+    const float *tp = target + (size_t)(Kt == 1 ? 0 : k) * Nt * 3;
+    const float *dp = dist + (size_t)k * Ns;
+    const int *ip = idx + (size_t)k * Ns;
+    double acc[ICP_NACC];
+#pragma unroll
+    for (int i = 0; i < ICP_NACC; ++i) acc[i] = 0.0;
+    for (int j = tid; j < n; j += ICP_THREADS) {
+        const float d = __ldg(dp + j);
+        if (!(d < max_dist2)) continue;
+        const int t = __ldg(ip + j);
+        if ((unsigned)t >= (unsigned)nt) continue;
+        const double sx = __ldg(cp + j * 3), sy = __ldg(cp + j * 3 + 1), sz = __ldg(cp + j * 3 + 2);
+        const double qx = __ldg(tp + (size_t)t * 3), qy = __ldg(tp + (size_t)t * 3 + 1), qz = __ldg(tp + (size_t)t * 3 + 2);
+        acc[0] += 1.0;
+        acc[1] += sx, acc[2] += sy, acc[3] += sz;
+        acc[4] += qx, acc[5] += qy, acc[6] += qz;
+        acc[7] += sx * qx, acc[8] += sx * qy, acc[9] += sx * qz;
+        acc[10] += sy * qx, acc[11] += sy * qy, acc[12] += sy * qz;
+        acc[13] += sz * qx, acc[14] += sz * qy, acc[15] += sz * qz;
+        acc[16] += (double)d;
+    }
+#pragma unroll
+    for (int i = 0; i < ICP_NACC; ++i) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[i] += __shfl_xor_sync(0xffffffffu, acc[i], o);
+        if (lane == 0) sh[warp][i] = acc[i];
+    }
+    __syncthreads();
+    if (tid == 0) icp_finish(sh, Tk, st, ragged ? scan_len + k : nullptr, ns, frozen, rel_fitness, rel_rmse, update);
+    if (!ragged || frozen || ns == 0 || nt == 0) return;
+    __syncthreads();  // T is final
+    icp_transform_rows(Tk, source + (size_t)k * Ns * 3, cur + (size_t)k * Ns * 3, ns);
+}
+
 }  // namespace genpc
 
 using namespace genpc;
@@ -189,8 +241,22 @@ extern "C" int genpc_icp_step(const float *cur, const float *target, const float
     cudaStream_t stream = (cudaStream_t)stream_;
     if (K < 0 || Ns <= 0 || Nt <= 0 || (Kt != 1 && Kt != K)) return GENPC_ERR_SHAPE;
     if (K == 0) return GENPC_OK;
-    icp_step_kernel<<<(unsigned)K, ICP_THREADS, 0, stream>>>(cur, target, dist, idx, T, state, Ns, Kt, Nt, max_dist2, rel_fitness,
-                                                            rel_rmse, update);
+    icp_step_kernel<<<(unsigned)K, ICP_THREADS, 0, stream>>>(const_cast<float *>(cur), nullptr, target, dist, idx, nullptr, nullptr,
+                                                            nullptr, T, state, Ns, Kt, Nt, max_dist2, rel_fitness, rel_rmse,
+                                                            update);
+    GENPC_CHECK_LAUNCH();
+    return GENPC_OK;
+}
+
+extern "C" int genpc_icp_step_ragged(const float *source, float *cur, const float *target, const float *dist, const int *idx,
+                                     const int *src_len, const int *tgt_len, int *scan_len, float *T, float *state, int K,
+                                     int Ns, int Kt, int Nt, float max_dist2, float rel_fitness, float rel_rmse, int update,
+                                     genpc_stream_t stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (!source || !src_len || !tgt_len || !scan_len || (dist == nullptr) != (idx == nullptr)) return GENPC_ERR_SHAPE;
+    if (K <= 0 || Ns <= 0 || Nt <= 0 || (Kt != 1 && Kt != K)) return GENPC_ERR_SHAPE;
+    icp_step_kernel<<<(unsigned)K, ICP_THREADS, 0, stream>>>(cur, source, target, dist, idx, src_len, tgt_len, scan_len, T, state,
+                                                            Ns, Kt, Nt, max_dist2, rel_fitness, rel_rmse, update);
     GENPC_CHECK_LAUNCH();
     return GENPC_OK;
 }

@@ -15,10 +15,10 @@ import os
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, chamfer_3D
 from .fps import furthest_point_sample
 from .loss_functions import chamfer_3DDist
-from .optim_registration.diff_obj_pose import object_pose_optimization_points
+from .optim_registration.diff_obj_pose import object_pose_optimization_points, pad_clouds
 from .utils.dataUtils import normalize_numpy, voxel_down_sample  # noqa: F401
 
 _cd = chamfer_3DDist()
@@ -29,21 +29,47 @@ def _apply(T, pts):
     return pts @ T[:, :3, :3].transpose(1, 2) + T[:, None, :3, 3]
 
 
-def chamfer_partial_l1_batched(src, tgt, cd_inv_weight=0.0):
+def chamfer_partial_l1_batched(src, tgt, cd_inv_weight=0.0, src_lengths=None, tgt_lengths=None):
     """Per-candidate score of the reference's sweep (reg_xyz.py:81-84, 167-170):
-    CDp-L1(src->tgt) + cd_inv_weight * CDp-L1(tgt->src), src [K,Ns,3], tgt [K,Nt,3] -> [K]."""
-    d1, d2, _, _ = _cd(src.contiguous(), tgt.contiguous())
-    return torch.sqrt(d1).mean(1) + cd_inv_weight * torch.sqrt(d2).mean(1)
+    CDp-L1(src->tgt) + cd_inv_weight * CDp-L1(tgt->src), src [K,Ns,3], tgt [K,Nt,3] -> [K].
+    src_lengths / tgt_lengths (integer tensors [K], either may be omitted = full stride): ragged batch, each candidate's
+    means taken over its own points (a side with no points contributes 0)."""
+    src, tgt = src.contiguous(), tgt.contiguous()
+    lens = chamfer_3D.lengths(src, tgt, src_lengths, tgt_lengths)
+    if lens is None:
+        d1, d2, _, _ = _cd(src, tgt)
+        return torch.sqrt(d1).mean(1) + cd_inv_weight * torch.sqrt(d2).mean(1)
+    d1, d2, _, _ = _cd(src, tgt, *lens)   # rows past a length come back as dist 0
+    n1, n2 = (ln.clamp(min=1).float() for ln in lens)
+    return torch.sqrt(d1).sum(1) / n1 + cd_inv_weight * (torch.sqrt(d2).sum(1) / n2)
+
+
+def _candidate_lengths(source, target, source_lengths, target_lengths):
+    """Lengths of a ragged ICP batch -> int32 [K] pair, checked as chamfer_3D.lengths does; a [1] target length of a shared
+    [1,Nt,3] target is expanded with it."""
+    K = source.shape[0]
+    if isinstance(target_lengths, torch.Tensor) and tuple(target_lengths.shape) == (1,) and target.shape[0] == 1 and K > 1:
+        target_lengths = target_lengths.expand(K)
+    return chamfer_3D.lengths(source, target.expand(K, -1, -1), source_lengths, target_lengths)
 
 
 def icp_point_to_point(source, target, max_correspondence_distance=0.05, init_transform=None, max_iteration=30,
-                       relative_fitness=1e-6, relative_rmse=1e-6):
+                       relative_fitness=1e-6, relative_rmse=1e-6, source_lengths=None, target_lengths=None):
     """Batched Open3D-style registration_icp (TransformationEstimationPointToPoint, no scaling), reg_xyz.py:9-38.
     source [K,Ns,3], target [K,Nt,3] (or [1,Nt,3]) -> (T [K,4,4], fitness [K], inlier_rmse [K]).
     Per iteration: transform (one bmm), nearest neighbours of all candidates (one Chamfer launch pair) and ONE
     genpc_icp_step launch (inliers, fitness / rmse / convergence, covariance, Horn rotation, T update) -- no host
     synchronisation except a convergence poll every 4 iterations.  GENPC_ICP_TORCH=1 selects the torch formulation
-    (batched float64 SVD, ~25 launches and a host sync per iteration) the kernel replaced; both agree to rounding."""
+    (batched float64 SVD, ~25 launches and a host sync per iteration) the kernel replaced; both agree to rounding.
+    source_lengths [K] / target_lengths [K] (or [1] with a shared target; integer tensors on the clouds' device, either may be
+    omitted = full stride): ragged batch, candidate k has its first source_lengths[k] / target_lengths[k] points and the rest
+    is padding that is never read.  Its results are bit for bit what it gets alone; see _icp_point_to_point_ragged."""
+    if source_lengths is not None or target_lengths is not None:
+        if os.environ.get("GENPC_ICP_TORCH") == "1":
+            raise _lib.GenpcError("GENPC_ICP_TORCH=1 has no ragged form: drop the lengths or the knob")
+        T, state = _icp_point_to_point_ragged(source, target, max_correspondence_distance, init_transform, max_iteration,
+                                              relative_fitness, relative_rmse, source_lengths, target_lengths)
+        return T, state[:, 0].clone(), state[:, 1].clone()
     if os.environ.get("GENPC_ICP_TORCH") == "1":
         return _icp_point_to_point_torch(source, target, max_correspondence_distance, init_transform, max_iteration,
                                          relative_fitness, relative_rmse)
@@ -73,6 +99,49 @@ def icp_point_to_point(source, target, max_correspondence_distance=0.05, init_tr
             if it % 4 == 3 and bool(state[:, 2].all()):   # every candidate converged: the remaining iterations are no-ops
                 break
     return T, state[:, 0].clone(), state[:, 1].clone()
+
+
+def _icp_point_to_point_ragged(source, target, max_correspondence_distance, init_transform, max_iteration, relative_fitness,
+                               relative_rmse, source_lengths, target_lengths):
+    """icp_point_to_point for a ragged batch: a transform-only genpc_icp_step_ragged call writes cur = T source, then per
+    iteration one ragged Chamfer call over the candidates that have not converged (scan_len) and one genpc_icp_step_ragged
+    launch, which also writes the next cur.  Same convergence poll as the equal-size loop.  A candidate's arithmetic does not
+    depend on its batch, so the batch runs until its slowest candidate converges and each one ends as it would alone.
+    -> (T [K,4,4], state [K,4] = fitness, inlier_rmse, converged, calls)."""
+    src_len, tgt_len = _candidate_lengths(source, target, source_lengths, target_lengths)
+    _lib.require_cuda(source, target)
+    K, Ns, _ = source.shape
+    dev = source.device
+    source = source.contiguous().float()
+    tgt = target.float()
+    if tgt.shape[0] == 1 and K > 1:
+        tgt = tgt.expand(K, -1, -1)   # the ragged Chamfer takes one target per pair
+    tgt = tgt.contiguous()
+    Nt = tgt.shape[1]
+    T = torch.eye(4, device=dev).repeat(K, 1, 1) if init_transform is None else \
+        torch.as_tensor(init_transform, dtype=torch.float32, device=dev).expand(K, 4, 4).clone()
+    T = T.contiguous()
+    state = torch.zeros(K, 4, device=dev)
+    cur = torch.zeros_like(source)
+    scan_len = torch.empty(K, dtype=torch.int32, device=dev)
+    thr2 = float(max_correspondence_distance) ** 2
+    L = _lib.lib()
+
+    def step(d1, i1, update):
+        rc = L.genpc_icp_step_ragged(_lib.ptr(source), _lib.ptr(cur), _lib.ptr(tgt), _lib.ptr(d1), _lib.ptr(i1),
+                                     _lib.ptr(src_len), _lib.ptr(tgt_len), _lib.ptr(scan_len), _lib.ptr(T), _lib.ptr(state),
+                                     K, Ns, K, Nt, thr2, float(relative_fitness), float(relative_rmse), int(update),
+                                     _lib.current_stream(dev))
+        _lib.check(rc, "genpc_icp_step_ragged")
+
+    with torch.no_grad(), torch.cuda.device(dev):
+        step(None, None, 0)
+        for it in range(max_iteration + 1):
+            d1, _, i1, _ = _cd(cur, tgt, scan_len, tgt_len)
+            step(d1, i1, it < max_iteration)
+            if it % 4 == 3 and bool(state[:, 2].all()):
+                break
+    return T, state
 
 
 def _icp_point_to_point_torch(source, target, max_correspondence_distance=0.05, init_transform=None, max_iteration=30,
@@ -142,6 +211,53 @@ def icp_with_scaling(source, target, scale, max_correspondence_distance=0.05, in
     S = torch.eye(4, device=source.device).repeat(K, 1, 1)
     S[:, 0, 0] = S[:, 1, 1] = S[:, 2, 2] = scale
     return icp_point_to_point(src, tgt, max_correspondence_distance, T0 @ S)
+
+
+def coarse_scale_sweep(s_down, t_down, scales, max_correspondence_distance=0.075, cd_inv_weight=0.5):
+    """The coarse sweep of reg() for one object (reg_xyz.py:146-173): icp_with_scaling over `scales`, then every candidate
+    scored by partial CD-L1 of the scan against the target moved by the inverse transform; the first minimum wins.
+    s_down [Ns,3] / t_down [Nt,3]: the voxel down-sampled scan and generated shape.
+    -> {"best_scale": float, "coarse_loss": float, "coarse_transformation": [4,4] tensor}."""
+    Ts, _, _ = icp_with_scaling(s_down, t_down, scales, max_correspondence_distance)
+    inv = torch.linalg.inv(Ts.double()).float()
+    t_moved = _apply(inv, t_down[None].expand(len(scales), -1, -1))
+    cd = chamfer_partial_l1_batched(s_down[None].expand(len(scales), -1, -1), t_moved, cd_inv_weight)
+    k = int(torch.argmin(cd))
+    return {"best_scale": float(scales[k]), "coarse_loss": float(cd[k]), "coarse_transformation": Ts[k]}
+
+
+def coarse_scale_sweep_batch(sources, targets, scales=np.linspace(1.5, 0.8, 11), max_correspondence_distance=0.075,
+                             cd_inv_weight=0.5):
+    """coarse_scale_sweep for a dataset of objects of different sizes in one ragged batch.  sources / targets: lists of
+    [n_i,3] CUDA tensors, already down-sampled (object i = (sources[i], targets[i])).  -> one dict per object, with the keys
+    of coarse_scale_sweep.
+
+    The first ICP pass of icp_with_scaling starts from the identity whatever the scale, so it runs once per object (O
+    candidates, not len(scales)·O); the second pass runs from T0 @ diag(s) over the len(scales)·O (object, scale) candidates
+    (object-major).  Each object's transforms are bit for bit those it gets alone in this function; against
+    coarse_scale_sweep they differ by rounding only (the ragged loop transforms the clouds with its own fma order, not a
+    bmm), and the losses are per-candidate means over the object's own points."""
+    if len(sources) != len(targets):
+        raise ValueError(f"coarse_scale_sweep_batch: {len(sources)} sources but {len(targets)} targets")
+    src, src_len = pad_clouds(sources)
+    tgt, tgt_len = pad_clouds(targets)
+    O, S = src.shape[0], len(scales)
+    dev = src.device
+    T0, _, _ = icp_point_to_point(src, tgt, max_correspondence_distance, source_lengths=src_len, target_lengths=tgt_len)
+    sc = torch.as_tensor(np.asarray(scales), dtype=torch.float32, device=dev)
+    D = torch.eye(4, device=dev).repeat(S, 1, 1)
+    D[:, 0, 0] = D[:, 1, 1] = D[:, 2, 2] = sc
+    init = T0.repeat_interleave(S, 0) @ D.repeat(O, 1, 1)
+    src2, tgt2 = src.repeat_interleave(S, 0), tgt.repeat_interleave(S, 0)
+    sl2, tl2 = src_len.repeat_interleave(S), tgt_len.repeat_interleave(S)
+    Ts, _, _ = icp_point_to_point(src2, tgt2, max_correspondence_distance, init, source_lengths=sl2, target_lengths=tl2)
+    inv = torch.linalg.inv(Ts.double()).float()
+    cd = chamfer_partial_l1_batched(src2, _apply(inv, tgt2), cd_inv_weight, sl2, tl2).view(O, S)
+    k = torch.argmin(cd, 1)   # first minimum per object, as coarse_scale_sweep
+    loss = cd.gather(1, k[:, None])[:, 0].cpu().tolist()
+    k = k.cpu().tolist()
+    return [{"best_scale": float(scales[k[o]]), "coarse_loss": float(loss[o]), "coarse_transformation": Ts[o * S + k[o]]}
+            for o in range(O)]
 
 
 def iterative_scale_search(source_xyz, target_xyz, scale_ranges, scale_steps, init_transform=None, cd_inv_weight=0.0,
@@ -256,14 +372,9 @@ def reg_points(partial_xyz, complete_xyz, cd_inv_weight=0.5, diff_init=True, reg
     # coarse sweep (:146-173), all 11 scales at once
     scales = np.linspace(1.5, 0.8, 11)
     s_down, t_down = voxel_down_sample(source, 0.03), voxel_down_sample(target, 0.03)
-    Ts, _, _ = icp_with_scaling(s_down, t_down, scales, 0.075)
-    inv = torch.linalg.inv(Ts.double()).float()
-    t_moved = _apply(inv, t_down[None].expand(len(scales), -1, -1))
-    cd = chamfer_partial_l1_batched(s_down[None].expand(len(scales), -1, -1), t_moved, cd_inv_weight)
-    k = int(torch.argmin(cd))
-    coarse = Ts[k]
-    out = {"best_scale": float(scales[k]), "coarse_loss": float(cd[k]), "coarse_transformation": coarse,
-           "diff_transform": diff_T}
+    out = coarse_scale_sweep(s_down, t_down, scales, 0.075, cd_inv_weight)
+    out["diff_transform"] = diff_T
+    coarse = out["coarse_transformation"]
     tgt_full = target
     if reg_fine_xyz:
         source = source @ coarse[:3, :3].T + coarse[:3, 3]          # :176

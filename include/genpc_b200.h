@@ -236,6 +236,25 @@ int genpc_mesh_sample(const float *verts, const int *faces, const float *vertex_
 int genpc_icp_step(const float *cur, const float *target, const float *dist, const int *idx, float *T, float *state, int K,
                    int Ns, int Kt, int Nt, float max_dist2, float rel_fitness, float rel_rmse, int update,
                    genpc_stream_t stream);
+/* Ragged batch: the same step for candidates of different sizes in one call.  src_len [K] / tgt_len [Kt] are device int32
+ * arrays, never NULL: candidate k has src_len[k] points at the start of its Ns stride in source / cur and its target
+ * tgt_len[k] (Kt = 1: tgt_len[0]) at the start of its Nt stride; the device clamps them to [0, Ns] / [0, Nt].  Rows past a
+ * length are never read (any value, NaN included).  Inliers, fitness and rmse are taken over j < src_len[k] (fitness =
+ * inliers / src_len[k]); an idx outside [0, tgt_len) is no inlier.  A candidate with 0 source or 0 target points has fitness 0
+ * and rmse 0, never updates and gets no cur row written.
+ *   source [K][Ns][3]  the untransformed clouds; after the step, cur[k][j] = T_k source[k][j] for j < src_len[k] (in place,
+ *                      c_r = fma(T[r][2], z, fma(T[r][1], y, fma(T[r][0], x, T[r][3]))) in fp32): the next iteration's cur
+ *   scan_len [K]       out: converged ? 0 : src_len[k] -- len1 of the next genpc_chamfer_forward_ragged, so that converged
+ *                      candidates cost no scan work while the rest of the batch iterates
+ * A candidate that enters a call converged reads no dist / idx (they are padding after scan_len = 0) and keeps T, fitness and
+ * rmse; its calls counter still increments.  dist = idx = NULL: transform only (writes cur and scan_len, leaves T and state),
+ * the call before a loop's first iteration.  Every candidate's T and state are bit for bit what it gets alone on its sliced
+ * clouds.  GENPC_ERR_SHAPE, before anything is queued, for a NULL source or length pointer, only one of dist / idx NULL,
+ * Kt not in {1, K} and sizes <= 0. */
+int genpc_icp_step_ragged(const float *source, float *cur, const float *target, const float *dist, const int *idx,
+                          const int *src_len, const int *tgt_len, int *scan_len, float *T, float *state, int K, int Ns,
+                          int Kt, int Nt, float max_dist2, float rel_fitness, float rel_rmse, int update,
+                          genpc_stream_t stream);
 
 /* ---- Farthest point sampling -------------------------------------------------------------------
  * Replaces the reference's CPU call fpsample.fps_sampling(xyz, K) (main.py:21-22, reg_xyz.py:215,
