@@ -7,6 +7,7 @@
 //   inliers (dist < max_dist^2), fitness = inliers / Ns, inlier_rmse = sqrt(sum dist / inliers)   (Open3D's definitions)
 //   convergence: |fitness - previous| < rel_fitness and |rmse - previous| < rel_rmse             (ICPConvergenceCriteria)
 //   centroids and the 3x3 cross-covariance of the inlier pairs, accumulated in double with a fixed tree (deterministic)
+//     about an anchor in the cloud (target row 0), so that clouds far from the origin keep their precision
 //   optimal rotation by Horn's closed form: the eigenvector of the largest eigenvalue of the 4x4 matrix N(H) (cyclic
 //     Jacobi in double) is the unit quaternion of the rotation that minimises sum |R s + t - q|^2 -- the same optimum
 //     Kabsch/SVD with the reflection fix gives, without an SVD;  t = mu_t - R mu_s
@@ -99,8 +100,10 @@ __device__ __forceinline__ void icp_transform_rows(const float *Tk, const float 
 
 // thread 0: statistics, convergence test and T update of candidate k from the warp partials.  frozen: the candidate entered
 // the call converged (ragged form), read nothing and keeps T, fitness and rmse; only its call counter moves.
-__device__ __forceinline__ void icp_finish(const double (&sh)[ICP_THREADS / 32][ICP_NACC], float *Tk, float *st, int *scan_len,
-                                           int ns, bool frozen, float rel_fitness, float rel_rmse, int update) {
+// The sums are taken about the anchor o (they hold s - o and q - o), so ms / mq below are centroids relative to o.
+__device__ __forceinline__ void icp_finish(const double (&sh)[ICP_THREADS / 32][ICP_NACC], const double (&o)[3], float *Tk,
+                                           float *st, int *scan_len, int ns, bool frozen, float rel_fitness, float rel_rmse,
+                                           int update) {
     if (frozen) {
         st[3] = st[3] + 1.f;
         *scan_len = 0;
@@ -151,7 +154,8 @@ __device__ __forceinline__ void icp_finish(const double (&sh)[ICP_THREADS / 32][
                             {2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)}};
     double t[3];
 #pragma unroll
-    for (int r = 0; r < 3; ++r) t[r] = mq[r] - (R[r][0] * ms[0] + R[r][1] * ms[1] + R[r][2] * ms[2]);
+    for (int r = 0; r < 3; ++r)
+        t[r] = (mq[r] + o[r]) - (R[r][0] * (ms[0] + o[0]) + R[r][1] * (ms[1] + o[1]) + R[r][2] * (ms[2] + o[2]));
     // ---- T <- [R|t] T ----
     double Told[4][4], Tnew[3][4];
 #pragma unroll
@@ -200,6 +204,14 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(float *cur, const
     const float *tp = target + (size_t)(Kt == 1 ? 0 : k) * Nt * 3;
     const float *dp = dist + (size_t)k * Ns;
     const int *ip = idx + (size_t)k * Ns;
+    // anchor o = target row 0 (0 if it is not finite): raw moments about the origin cancel in H = sum s q^T - cnt ms mq^T
+    // when the clouds sit far from it (an offset of 1000 at an extent of 0.1 cost 3 fp32 ulps of t), moments about a point
+    // of the cloud do not.  It depends on the candidate only, so a candidate's result still does not depend on its batch.
+    double o[3] = {0.0, 0.0, 0.0};
+    if (n > 0) {
+        const float ox = __ldg(tp), oy = __ldg(tp + 1), oz = __ldg(tp + 2);
+        if (isfinite(ox) && isfinite(oy) && isfinite(oz)) o[0] = ox, o[1] = oy, o[2] = oz;
+    }
     double acc[ICP_NACC];
 #pragma unroll
     for (int i = 0; i < ICP_NACC; ++i) acc[i] = 0.0;
@@ -208,8 +220,9 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(float *cur, const
         if (!(d < max_dist2)) continue;
         const int t = __ldg(ip + j);
         if ((unsigned)t >= (unsigned)nt) continue;
-        const double sx = __ldg(cp + j * 3), sy = __ldg(cp + j * 3 + 1), sz = __ldg(cp + j * 3 + 2);
-        const double qx = __ldg(tp + (size_t)t * 3), qy = __ldg(tp + (size_t)t * 3 + 1), qz = __ldg(tp + (size_t)t * 3 + 2);
+        const double sx = __ldg(cp + j * 3) - o[0], sy = __ldg(cp + j * 3 + 1) - o[1], sz = __ldg(cp + j * 3 + 2) - o[2];
+        const double qx = __ldg(tp + (size_t)t * 3) - o[0], qy = __ldg(tp + (size_t)t * 3 + 1) - o[1],
+                     qz = __ldg(tp + (size_t)t * 3 + 2) - o[2];
         acc[0] += 1.0;
         acc[1] += sx, acc[2] += sy, acc[3] += sz;
         acc[4] += qx, acc[5] += qy, acc[6] += qz;
@@ -225,7 +238,7 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_step_kernel(float *cur, const
         if (lane == 0) sh[warp][i] = acc[i];
     }
     __syncthreads();
-    if (tid == 0) icp_finish(sh, Tk, st, ragged ? scan_len + k : nullptr, ns, frozen, rel_fitness, rel_rmse, update);
+    if (tid == 0) icp_finish(sh, o, Tk, st, ragged ? scan_len + k : nullptr, ns, frozen, rel_fitness, rel_rmse, update);
     if (!ragged || frozen || ns == 0 || nt == 0) return;
     __syncthreads();  // T is final
     icp_transform_rows(Tk, source + (size_t)k * Ns * 3, cur + (size_t)k * Ns * 3, ns);

@@ -227,7 +227,9 @@ int genpc_mesh_sample(const float *verts, const int *faces, const float *vertex_
  *   cur [K][Ns][3]    the candidates' source clouds under their current transforms
  *   target [Kt][Nt][3], Kt = K or 1 (one target shared by all candidates)
  *   T [K][16]         row-major 4x4 transforms, updated in place: T <- [R|t] T, (R, t) = the least-squares rigid motion of
- *                     the inlier pairs (dist < max_dist2) -- Horn's closed form, identical optimum to Kabsch/SVD
+ *                     the inlier pairs (dist < max_dist2, NaN never, idx in [0, Nt)) -- Horn's closed form, identical
+ *                     optimum to Kabsch/SVD; the sums are taken about the candidate's target row 0 (about the origin if
+ *                     that row is not finite), so clouds far from the origin keep their precision
  *   state [K][4]      fitness, inlier_rmse, converged (0/1), calls -- zeroed by the caller before the first call; a
  *                     candidate converges when both |fitness - previous| < rel_fitness and |rmse - previous| < rel_rmse
  *                     (Open3D ICPConvergenceCriteria) and is left unchanged from then on, like one with < 3 inliers

@@ -49,6 +49,7 @@ def lib():
                                        _i32p]
         L.oracle_pose_matrix.argtypes = [_f32p, _f32p]
         L.oracle_transform.argtypes = [_int, _f32p, _f32p, _f32p, _f32p]
+        L.oracle_fmaf.argtypes = [_int, _f32p, _f32p, _f32p, _f32p]
         _lib = L
     return _lib
 
@@ -224,6 +225,14 @@ def transform(V, center, params):
     V = _c(V, np.float32)
     out = np.zeros_like(V)
     lib().oracle_transform(V.shape[0], V, _c(center, np.float32), _c(params, np.float32), out)
+    return out
+
+
+def fmaf(a, b, c):
+    """fp32 a * b + c with one rounding (C fmaf), elementwise with numpy broadcasting -> float32 array."""
+    a, b, c = (_c(x, np.float32) for x in np.broadcast_arrays(*(np.asarray(x, np.float32) for x in (a, b, c))))
+    out = np.zeros(a.shape, np.float32)
+    lib().oracle_fmaf(a.size, a, b, c, out)
     return out
 
 

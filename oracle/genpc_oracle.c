@@ -573,3 +573,9 @@ void oracle_transform(int N, const float *V, const float *c, const float *par, f
         out[i * 3 + 2] = (rz + c[2]) + par[8];
     }
 }
+
+/* fp32 fused multiply-add, one rounding (C99 fmaf), elementwise over n values: out = a * b + c.  numpy has no fp32 fma and
+ * float64 a * b + c rounds twice on the way to fp32, so tests that state a kernel's explicit fmaf order use this. */
+void oracle_fmaf(int n, const float *a, const float *b, const float *c, float *out) {
+    for (int i = 0; i < n; i++) out[i] = fmaf(a[i], b[i], c[i]);
+}

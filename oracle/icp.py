@@ -24,10 +24,10 @@ def kabsch(src, dst):
 def icp_step(cur, target, dist, idx, T, state, max_dist2, rel_fitness, rel_rmse, update=True):
     """One call of genpc_icp_step for ONE candidate.  cur [Ns,3] (source under T), target [Nt,3], dist/idx = squared NN
     distance / index of every cur point, T [4,4] float32, state = [fitness, rmse, converged, calls] float32.
-    -> (T', state')."""
+    An inlier has dist < max_dist2 (NaN is none) and an idx in [0, Nt).  -> (T', state')."""
     cur, target = np.asarray(cur, np.float32), np.asarray(target, np.float32)
-    dist = np.asarray(dist, np.float32)
-    inl = dist < np.float32(max_dist2)
+    dist, idx = np.asarray(dist, np.float32), np.asarray(idx)
+    inl = (dist < np.float32(max_dist2)) & (idx >= 0) & (idx < target.shape[0])
     cnt = int(inl.sum())
     fitness = np.float32(cnt / cur.shape[0])
     rmse = np.float32(np.sqrt(dist[inl].astype(np.float64).sum() / (cnt if cnt > 0 else 1)))
@@ -40,7 +40,7 @@ def icp_step(cur, target, dist, idx, T, state, max_dist2, rel_fitness, rel_rmse,
     T = np.array(T, np.float32)
     if not update or converged or cnt < 3:
         return T, new_state
-    R, t = kabsch(cur[inl], target[np.asarray(idx)[inl]])
+    R, t = kabsch(cur[inl], target[idx[inl]])
     M = np.eye(4)
     M[:3, :3], M[:3, 3] = R, t
     Tn = T.copy()

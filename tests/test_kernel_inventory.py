@@ -165,7 +165,7 @@ KERNELS = {
     "genpc::register_finish_kernel<256>": DSP + "test_registration_8_scans_exhaustive_sym_finish256_vs_oracle",
     "genpc::register_finish_kernel<512>": DSP + "test_registration_c3_pruned_sym_finish512_vs_oracle",
     "genpc::register_sims_kernel": DSP + "test_registration_c3_pruned_sym_finish512_vs_oracle",
-    "genpc::icp_step_kernel": "tests/test_reg_xyz.py::test_icp_step_kernel_matches_the_torch_formulation",
+    "genpc::icp_step_kernel": "tests/test_icp_geometry.py::test_unique_optimum_within_two_ulps_of_kabsch",
     "genpc::knn_mean_kernel<1>": DSP + "test_knn_mean_distance_every_list_size",
     # mesh sampling, depth rendering
     "genpc::mesh_face_area_kernel": "tests/test_mesh_glb.py::test_sampler_kernel_bit_exact_vs_oracle",
