@@ -64,6 +64,7 @@ _SIGNATURES = {
     "genpc_icp_step_ragged": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _flt, _flt,
                                      _flt, _int, _vp]),
     "genpc_knn_mean_distance": (_int, [_vp, _int, _int, _int, _vp, _vp]),
+    "genpc_knn_mean_distance_ragged": (_int, [_vp, _vp, _int, _int, _int, _int, _vp, _vp]),
     "genpc_mesh_face_areas": (_int, [_vp, _vp, _int, _int, _vp, _vp]),
     "genpc_mesh_sample": (_int, [_vp, _vp, _vp, _vp, _int, _int, ctypes.c_ulonglong, _vp, _vp, _vp, _vp]),
     "genpc_fps_workspace_bytes": (_sz, [_int, _int, _int]),

@@ -28,21 +28,24 @@ def lengths(xyz1, xyz2, len1=None, len2=None):
     if len1 is None and len2 is None:
         return None
     B = xyz1.shape[0]
-    out = []
-    for ln, xyz, name in ((len1, xyz1, "len1"), (len2, xyz2, "len2")):
-        if ln is None:
-            out.append(torch.full((B,), xyz.shape[1], dtype=torch.int32, device=xyz.device))
-            continue
-        if not isinstance(ln, torch.Tensor):
-            raise _lib.GenpcError(f"{name} must be a tensor")
-        if ln.dtype.is_floating_point or ln.dtype.is_complex or ln.dtype == torch.bool:
-            raise _lib.GenpcError(f"{name} must be an integer tensor, got {ln.dtype}")
-        if tuple(ln.shape) != (B,):
-            raise _lib.GenpcError(f"{name} must have shape ({B},), got {tuple(ln.shape)}")
-        if ln.device != xyz.device:
-            raise _lib.GenpcError(f"{name} is on {ln.device}, the clouds on {xyz.device}")
-        out.append(ln.to(torch.int32).contiguous())
-    return tuple(out)
+    return cloud_lengths(xyz1, len1, B, "len1"), cloud_lengths(xyz2, len2, B, "len2")
+
+
+def cloud_lengths(xyz, ln, B, name):
+    """One side of `lengths`: the point counts `ln` of the B clouds of xyz [B,stride,3] -> contiguous int32 [B] on xyz's device
+    (None: every cloud fills its stride).  Raises GenpcError for a non-tensor, a non-integer dtype, a shape other than (B,) or
+    another device."""
+    if ln is None:
+        return torch.full((B,), xyz.shape[1], dtype=torch.int32, device=xyz.device)
+    if not isinstance(ln, torch.Tensor):
+        raise _lib.GenpcError(f"{name} must be a tensor")
+    if ln.dtype.is_floating_point or ln.dtype.is_complex or ln.dtype == torch.bool:
+        raise _lib.GenpcError(f"{name} must be an integer tensor, got {ln.dtype}")
+    if tuple(ln.shape) != (B,):
+        raise _lib.GenpcError(f"{name} must have shape ({B},), got {tuple(ln.shape)}")
+    if ln.device != xyz.device:
+        raise _lib.GenpcError(f"{name} is on {ln.device}, the clouds on {xyz.device}")
+    return ln.to(torch.int32).contiguous()
 
 
 def forward(xyz1, xyz2, dist1, dist2, idx1, idx2):

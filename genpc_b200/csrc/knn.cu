@@ -1,4 +1,5 @@
-// knn.cu -- mean distance to the k nearest neighbours of every point of one cloud (k <= 32), for sm_100a.
+// knn.cu -- mean distance to the k nearest neighbours of every point of a cloud, or of each cloud of a batch (k <= 32),
+// for sm_100a.
 //
 // The fusion tail of reg() ends with Open3D's remove_statistical_outlier(nb_neighbors=20, std_ratio) on the fused cloud
 // (reg_xyz.py:219, utils/dataUtils.py:652-666; third-party CPU KD-tree code, not vendored): per point the mean distance
@@ -12,6 +13,8 @@
 //   * mean = (sum of sqrt of the k values, added in ascending order in fp32) / k  -- order fixed => bit-reproducible,
 //     mirrored by oracle_knn_mean_distance.
 // include_self != 0 counts the point itself (distance 0) among the k, as Open3D's KD-tree query of a cloud point does.
+// A batch of clouds is one launch: cloud b is blockIdx.y, its first len[b] rows of a common stride are its points.  A cloud's
+// CTAs, tiles and lane clamps are those of a solo call on its points alone, so every cloud gets the solo call's bits.
 #include "common.cuh"
 
 namespace genpc {
@@ -31,12 +34,23 @@ __device__ __forceinline__ void knn_insert(float (&best)[K], float v) {
     }
 }
 
+// xyz [B][stride][3], mean_out [B][stride]; len [B] (NULL: every cloud fills the stride) is clamped to [0, stride] here.
+// Rows past a cloud's length are never read and get -1 (Open3D's "the query found nothing").
 template <int K>
-__global__ void __launch_bounds__(KNN_THREADS) knn_mean_kernel(const float *__restrict__ xyz, int n, int include_self,
+__global__ void __launch_bounds__(KNN_THREADS) knn_mean_kernel(const float *__restrict__ xyz, int stride,
+                                                               const int *__restrict__ len, int include_self,
                                                                float *__restrict__ mean_out) {
     __shared__ __align__(16) float s[3][KNN_TILE];
+    xyz += (size_t)blockIdx.y * stride * 3;
+    mean_out += (size_t)blockIdx.y * stride;
+    const int n = len ? min(max(__ldg(len + blockIdx.y), 0), stride) : stride;
     // KNN_SPLIT adjacent lanes share one query (a thread per query leaves one warp per scheduler on a 20 000-point cloud:
     // latency bound); out-of-range queries are clamped so that whole lane groups stay converged for the shuffles
+    const int q0 = blockIdx.x * (KNN_THREADS / KNN_SPLIT);
+    if (q0 >= n) {  // the whole CTA lies in the padding: its rows get -1 and it leaves before the first barrier
+        if (threadIdx.x < KNN_THREADS / KNN_SPLIT && q0 + threadIdx.x < stride) mean_out[q0 + threadIdx.x] = -1.0f;
+        return;
+    }
     const int q = (blockIdx.x * KNN_THREADS + threadIdx.x) / KNN_SPLIT, sub = threadIdx.x & (KNN_SPLIT - 1);
     const bool valid = q < n;
     const int i = valid ? q : n - 1;
@@ -86,7 +100,11 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_mean_kernel(const float *__re
         for (int c = 0; c < K; ++c)
             if (other[c] < best[K - 1]) knn_insert<K>(best, other[c]);
     }
-    if (!valid || sub != 0) return;
+    if (sub != 0 || q >= stride) return;
+    if (!valid) {
+        mean_out[q] = -1.0f;
+        return;
+    }
     float sum = 0.f;
     int m = 0;
 #pragma unroll
@@ -103,14 +121,13 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_mean_kernel(const float *__re
 
 using namespace genpc;
 
-extern "C" int genpc_knn_mean_distance(const float *xyz, int n, int k, int include_self, float *mean_dist,
-                                       genpc_stream_t stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
-    if (n < 0 || k < 1 || k > 32) return GENPC_ERR_SHAPE;
+// One cloud per grid row; genpc_knn_mean_distance is the B = 1, len = NULL case (a 1-D grid).
+static int knn_launch(const float *xyz, const int *len, int B, int n, int k, int include_self, float *mean_dist,
+                      cudaStream_t stream) {
     if (n == 0) return GENPC_OK;
-    const unsigned grid = (unsigned)(((size_t)n * KNN_SPLIT + KNN_THREADS - 1) / KNN_THREADS);
+    const dim3 grid((unsigned)(((size_t)n * KNN_SPLIT + KNN_THREADS - 1) / KNN_THREADS), (unsigned)B);
 #define KNN_CASE(KK) \
-    if (k <= KK) { knn_mean_kernel<KK><<<grid, KNN_THREADS, 0, stream>>>(xyz, n, include_self, mean_dist); GENPC_CHECK_LAUNCH(); return GENPC_OK; }
+    if (k <= KK) { knn_mean_kernel<KK><<<grid, KNN_THREADS, 0, stream>>>(xyz, n, len, include_self, mean_dist); GENPC_CHECK_LAUNCH(); return GENPC_OK; }
     // a list longer than k is NOT equivalent (the mean runs over the whole list), so every k has its own size
     switch (k) {
         case 1: KNN_CASE(1) case 2: KNN_CASE(2) case 3: KNN_CASE(3) case 4: KNN_CASE(4) case 5: KNN_CASE(5)
@@ -123,4 +140,16 @@ extern "C" int genpc_knn_mean_distance(const float *xyz, int n, int k, int inclu
     }
 #undef KNN_CASE
     return GENPC_ERR_SHAPE;
+}
+
+extern "C" int genpc_knn_mean_distance(const float *xyz, int n, int k, int include_self, float *mean_dist,
+                                       genpc_stream_t stream) {
+    if (n < 0 || k < 1 || k > 32) return GENPC_ERR_SHAPE;
+    return knn_launch(xyz, nullptr, 1, n, k, include_self, mean_dist, (cudaStream_t)stream);
+}
+
+extern "C" int genpc_knn_mean_distance_ragged(const float *xyz, const int *len, int B, int n, int k, int include_self,
+                                              float *mean_dist, genpc_stream_t stream) {
+    if (!xyz || !len || !mean_dist || B < 1 || B > 65535 || n < 0 || k < 1 || k > 32) return GENPC_ERR_SHAPE;
+    return knn_launch(xyz, len, B, n, k, include_self, mean_dist, (cudaStream_t)stream);
 }

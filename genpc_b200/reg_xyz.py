@@ -292,33 +292,56 @@ def remove_close_points(source_xyz, target_xyz, distance_threshold=0.0001):
     return d1[0] >= distance_threshold
 
 
-def knn_mean_distance(xyz, k, include_self=True):
+def knn_mean_distance(xyz, k, include_self=True, lengths=None):
     """Mean distance from each point of xyz [N,3] (CUDA) to its k nearest points of the same cloud
-    (genpc_knn_mean_distance; include_self counts the point itself, as a KD-tree query of a cloud point does)."""
+    (genpc_knn_mean_distance; include_self counts the point itself, as a KD-tree query of a cloud point does).
+    A batch xyz [B,N,3] -> [B,N] in one launch (genpc_knn_mean_distance_ragged): lengths (integer tensor [B] on the clouds'
+    device, None = every cloud fills the stride) gives each cloud's point count, its points being the first rows of its stride.
+    Each cloud's rows are bit for bit its solo call on its own points; rows past a length are never read and come back -1.
+    The lengths are clamped to [0, N] on the device, so the call does not synchronise with the host."""
+    if xyz.dim() == 2 and lengths is not None:
+        raise _lib.GenpcError("lengths need a batch of clouds [B,N,3], got one cloud [N,3]")
+    if xyz.dim() not in (2, 3) or xyz.shape[-1] != 3:
+        raise _lib.GenpcError(f"knn_mean_distance takes [N,3] or [B,N,3] clouds, got {tuple(xyz.shape)}")
+    if xyz.dim() == 3:
+        ln = chamfer_3D.cloud_lengths(xyz, lengths, xyz.shape[0], "lengths")
     _lib.require_cuda(xyz)
     x = xyz.contiguous().float()
-    out = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
+    out = torch.empty(x.shape[:-1], dtype=torch.float32, device=x.device)
     with torch.cuda.device(x.device):
-        rc = _lib.lib().genpc_knn_mean_distance(_lib.ptr(x), x.shape[0], int(k), int(bool(include_self)), _lib.ptr(out),
-                                                _lib.current_stream(x.device))
-    _lib.check(rc, "genpc_knn_mean_distance")
+        if x.dim() == 2:
+            rc = _lib.lib().genpc_knn_mean_distance(_lib.ptr(x), x.shape[0], int(k), int(bool(include_self)), _lib.ptr(out),
+                                                    _lib.current_stream(x.device))
+        else:
+            rc = _lib.lib().genpc_knn_mean_distance_ragged(_lib.ptr(x), _lib.ptr(ln), x.shape[0], x.shape[1], int(k),
+                                                           int(bool(include_self)), _lib.ptr(out), _lib.current_stream(x.device))
+    _lib.check(rc, "genpc_knn_mean_distance" if x.dim() == 2 else "genpc_knn_mean_distance_ragged")
     return out
 
 
-def remove_statistical_outlier(xyz, nb_neighbors=20, std_ratio=2.5):
+def statistical_outlier_mask(mean_dist, std_ratio):
+    """Open3D's threshold over per-point k-NN means [..., N] (the last axis is one cloud) -> bool keep mask of the same shape:
+    keep 0 < mean < cloud_mean + std_ratio * std_dev, in float64.  Only means > 0 enter the sums (a mean of exactly 0 comes from
+    duplicated points); the divisors count every answered query (mean >= 0, so -1 rows -- padding, or a query that found
+    nothing -- count nowhere); std_dev divides by n_valid - 1 and is 0 below two answered queries.  Masked reductions, no
+    boolean indexing: no host synchronisation, and a cloud with nothing answered keeps nothing."""
+    md = mean_dist.double()
+    pos = md > 0
+    nv = (md >= 0).sum(-1, keepdim=True)
+    mu = torch.where(pos, md, 0.0).sum(-1, keepdim=True) / nv.clamp(min=1)
+    ss = torch.where(pos, (md - mu) ** 2, 0.0).sum(-1, keepdim=True)
+    sd = torch.where(nv > 1, torch.sqrt(ss / (nv - 1).clamp(min=1)), 0.0)
+    return pos & (md < mu + std_ratio * sd)
+
+
+def remove_statistical_outlier(xyz, nb_neighbors=20, std_ratio=2.5, lengths=None):
     """Open3D remove_statistical_outlier as the reference uses it (reg_xyz.py:219, utils/dataUtils.py:652-666),
     restated on the k-NN kernel: per point the mean distance to its nb_neighbors nearest points -- the KD-tree query of
-    a cloud point returns the point itself first, so it is one of them -- then keep 0 < mean < cloud_mean + std_ratio *
-    std_dev (float64 statistics; means of exactly 0 -- duplicated points -- stay out of both sums, as in Open3D).  Returns the boolean keep mask.  (Open3D is not vendored: semantics from its
-    documented behaviour, parity unpinned; the oracle defines them.)"""
-    md = knn_mean_distance(xyz, nb_neighbors, include_self=True).double()
-    nv = int((md >= 0).sum())
-    if nv == 0:
-        return torch.zeros_like(md, dtype=torch.bool)
-    pos = md > 0            # Open3D: only positive means enter the sums, the divisors count every answered query
-    mu = md[pos].sum() / nv
-    sd = torch.sqrt(((md[pos] - mu) ** 2).sum() / (nv - 1)) if nv > 1 else torch.zeros((), dtype=torch.float64, device=md.device)
-    return pos & (md < mu + std_ratio * sd)
+    a cloud point returns the point itself first, so it is one of them -- then statistical_outlier_mask's threshold.
+    xyz [N,3] -> bool keep mask [N]; a batch xyz [B,N,3] with lengths as knn_mean_distance -> [B,N], every cloud thresholded
+    over its own points and padding rows False.  No host synchronisation in either form.  (Open3D is not vendored: semantics
+    from its documented behaviour, parity unpinned; the oracle defines them.)"""
+    return statistical_outlier_mask(knn_mean_distance(xyz, nb_neighbors, True, lengths), std_ratio)
 
 
 def get_rotate_matrix(axis, angle):

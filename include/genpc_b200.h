@@ -202,6 +202,15 @@ int genpc_chamfer_sym_fixup(const float *rows_full, const float *cols, const uns
  * Squared distances with the Chamfer rounding order, square roots added in ascending order in fp32: reproducible
  * bit for bit (oracle_knn_mean_distance).  A cloud with fewer than k candidates averages what it has; none: -1. */
 int genpc_knn_mean_distance(const float *xyz, int n, int k, int include_self, float *mean_dist, genpc_stream_t stream);
+/* Ragged batch: the same statistic for B clouds of different sizes in one launch.  xyz [B][n][3], mean_dist [B][n]; len is a
+ * device int32 [B] array, never NULL: cloud b has len[b] points at the start of its n-stride, and the device clamps len[b] to
+ * [0, n].  Rows past a length are never read (any value, NaN included).  For j < len[b], mean_dist[b][j] is bit for bit what
+ * genpc_knn_mean_distance returns for that cloud alone on its len[b] points (include_self = 0 leaves out the query's own row of
+ * its cloud); every row j in [len[b], n) gets -1, Open3D's marker of a query that found nothing.  n = 0 queues nothing.
+ * GENPC_ERR_SHAPE, before anything is queued, for a NULL xyz, len or mean_dist, B outside [1, 65535] (the grid's y extent),
+ * n < 0 and k outside [1, 32]. */
+int genpc_knn_mean_distance_ragged(const float *xyz, const int *len, int B, int n, int k, int include_self,
+                                   float *mean_dist, genpc_stream_t stream);
 
 /* ---- surface sampling of the generated mesh -------------------------------------------------------
  * Replaces the sampling step of glb2point (utils/dataUtils.py:217-250: trimesh mesh.sample(num_points, return_index=True)
